@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N ...            # reference algorithm on the host CPUs
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one forward + one backward of the operator core (model/advection.py:129-169) over
 one batch of synthetic fields.  Workload at N=1: the configuration BASELINE.json's metric is
@@ -36,6 +37,8 @@ BYTES_FWD, BYTES_BWD = 16, 28                                   # algorithmic B 
 BYTES_STEP = 44
 CFL_CELLS = 6.0        # the benchmark clips |u|, |v| at 4 cells: great-circle step <= 4*sqrt(2) < 6 cells
 CPU_SAMPLE_V = 8                                                # channels of the bounded CPU sample
+DUMP_SAMPLES = 1 << 21      # per output: four float32 outputs of 8 MB each stay under 64 MB
+OUTPUT_NAMES = ("out", "grad_field", "grad_u", "grad_v")
 
 
 def parse():
@@ -59,7 +62,35 @@ def parse():
     ap.add_argument("--no-graph", action="store_true", help="latband: eager autograd step instead of a CUDA graph")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write out / grad_field / grad_u / grad_v of the last step as "
+                         "DIR/<name>.npy (float32); outputs of more than DUMP_SAMPLES elements are reduced to the "
+                         "flat-index sample of sample_index().  --impl reference writes its [1, CPU_SAMPLE_V, H, W] "
+                         "CPU sample, so its files compare with those of other reference runs, not with the b200 arm's")
     return ap.parse_args()
+
+
+def sample_index(numel):
+    """The fixed, seeded sample of flat indices that --dump-outputs writes of a large output (sorted, unique)."""
+    import numpy as np
+    return np.unique(np.random.default_rng(0).integers(0, numel, DUMP_SAMPLES))
+
+
+def dump_outputs(path, outputs):
+    """Write each tensor of `outputs` (name -> tensor, all of one shape) as <path>/<name>.npy in float32: whole when
+    it has at most DUMP_SAMPLES elements, else the elements at sample_index(numel) of its flattened form."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    idx = None
+    numel = next(iter(outputs.values())).numel()
+    if numel > DUMP_SAMPLES:
+        idx = torch.from_numpy(sample_index(numel))
+    for name, t in outputs.items():
+        t = t.detach()
+        if idx is not None:
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
 
 
 def measured_peak():
@@ -189,7 +220,7 @@ def run_reference(args):
     if rank != 0:
         return
     H, W, V, Bg, poles = WORKLOADS[args.workload]
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     warm = max(1, min(args.warmup, 1))
     import torch
     from oracle import sl_oracle as O
@@ -201,8 +232,10 @@ def run_reference(args):
         O.sl_advect_fwd_bwd(field, u, v, lat, lon, S.DT_DEFAULT, go, args.interp)
     t0 = time.perf_counter()
     for _ in range(steps):
-        O.sl_advect_fwd_bwd(field, u, v, lat, lon, S.DT_DEFAULT, go, args.interp)
+        res = O.sl_advect_fwd_bwd(field, u, v, lat, lon, S.DT_DEFAULT, go, args.interp)
     sec = (time.perf_counter() - t0) / steps
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(OUTPUT_NAMES, res)))
     pts = CPU_SAMPLE_V * H * W
     val = pts / sec
     sample = f"[1,{CPU_SAMPLE_V},{H},{W}] slice of the workload per step ({steps} steps, {warm} warm-up)"
@@ -238,6 +271,8 @@ def run_b200(args):
     if decomp == "auto":      # BASELINE.json configs[2]: "0.25 deg ... 1/2/4/8 B200 with latitude-band halo exchange"
         decomp = "latband" if (world > 1 and args.workload == "c3") else "batch"
     if decomp == "latband" and world > 1:
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs needs one whole output per process: use --decomp batch")
         from paradis_model_b200 import halo
         return halo.bench_latband(args, WORKLOADS[args.workload], rank, world, dev)
 
@@ -276,6 +311,8 @@ def run_b200(args):
     if world > 1:
         dist.barrier()
     P.check_status(dev)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dict(zip(OUTPUT_NAMES, (R.out, R.gfield, R.gu, R.gv))))
     total_ms = ev[0][0].elapsed_time(ev[-1][2])
     phase = [sum(e[i].elapsed_time(e[i + 1]) for e in ev) / args.steps for i in range(2)]
     t = torch.tensor([total_ms], device=dev)

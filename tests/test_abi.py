@@ -1,5 +1,6 @@
 """CPU tests of the boundary: the library builds/loads, exports every symbol the header
-declares, and rejects bad arguments with the documented codes before touching a GPU."""
+declares, and rejects bad arguments with the documented codes before touching a GPU; bench.py's output line and
+output dumps (the b200 arm's on the GPU)."""
 import ctypes as C
 import os
 import re
@@ -73,13 +74,15 @@ def test_ops_fail_loudly_on_cpu():
         P.geocyclic_pad(x, 1)
 
 
-def test_bench_reference_arm_prints_the_contract_line():
-    """`bench.py --impl reference` (the CPU arm the driver runs beside the GPU arm) needs no GPU: one JSON line
-    with the same metric / unit / config as the product arm plus impl, cpu_baseline and a zero-copy e2e object."""
+def test_bench_reference_arm_prints_the_contract_line(tmp_path):
+    """`bench.py --impl reference` (the CPU arm run beside the GPU arm) needs no GPU: one JSON line
+    with the same metric / unit / config as the product arm plus impl, cpu_baseline and a zero-copy e2e object;
+    --dump-outputs writes the four arrays of the last timed step."""
     import json, os, subprocess, sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--steps", "1",
-                          "--warmup", "0", "--workload", "c2"], capture_output=True, text=True, timeout=600, cwd=root)
+                          "--warmup", "0", "--workload", "c2", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=root)
     assert res.returncode == 0, res.stderr[-2000:]
     line = json.loads(res.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "grid-pt*ch/s" and line["higher_is_better"] is True
@@ -89,3 +92,57 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert line["e2e"] == {"value": line["value"], "unit": line["unit"], "h2d_bytes_per_step": 0,
                            "d2h_bytes_per_step": 0}
     assert "workload" in line["config"] and line["n_gpus"] == 1 and line["vs_baseline"] is None
+    # c2 mesh (128 x 256, no pole rows), the 8-channel CPU sample, seed 0: small enough to be written whole
+    import numpy as np
+    import torch
+    from conftest import relmax
+    from oracle import sl_oracle as O
+    from paradis_model_b200 import synthetic as S
+    field, u, v, go = S.white_noise_inputs(128, 256, 1, 8)
+    lat, lon = O.make_grids(128, 256, False)
+    ref = O.sl_advect_fwd_bwd(field, u, v, lat, lon, S.DT_DEFAULT, go, "bilinear")
+    assert sorted(os.listdir(tmp_path)) == ["grad_field.npy", "grad_u.npy", "grad_v.npy", "out.npy"]
+    for name, r in zip(("out", "grad_field", "grad_u", "grad_v"), ref):
+        a = np.load(tmp_path / f"{name}.npy")
+        assert a.dtype == np.float32 and a.shape == tuple(r.shape), name
+        assert relmax(torch.from_numpy(a), r) < 1e-5, name
+
+
+@pytest.mark.gpu
+def test_bench_b200_arm_dumps_a_sample_of_the_last_step(tmp_path):
+    """`bench.py --dump-outputs` on c2 ([8, 64, 128, 256]: more elements than DUMP_SAMPLES): four float32 files holding
+    the timed path's outputs at sample_index(numel), bit for bit what RawAdvection computes from the same seeded inputs
+    in this process, and within the white-noise tolerances of the oracle run by torch on the same GPU."""
+    import importlib.util, subprocess, sys
+    import numpy as np
+    import torch
+    import paradis_model_b200 as P
+    from conftest import bad_fraction
+    from oracle import sl_oracle as O
+    from paradis_model_b200 import synthetic as S
+    from paradis_model_b200.ops import RawAdvection
+    res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--workload",
+                          "c2", "--no-cpu", "--no-e2e", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert res.returncode == 0, res.stderr[-2000:]
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    H, W, V, B, poles = bench.WORKLOADS["c2"]
+    idx = torch.from_numpy(bench.sample_index(B * V * H * W)).cuda()
+    assert 0 < idx.numel() <= bench.DUMP_SAMPLES < B * V * H * W
+    field, u, v, go = [t.cuda() for t in S.white_noise_inputs(H, W, B, V)]
+    lat, lon = [t.cuda() for t in S.make_grids(H, W, poles)]
+    R = RawAdvection(P.SLGeometry.from_grids(lat, lon), B, V, "bilinear", True, "fast", bench.CFL_CELLS)
+    R.forward(field, u, v, S.DT_DEFAULT)
+    R.backward(go, field, u, v, S.DT_DEFAULT, 3)
+    P.check_status()
+    ref = O.sl_advect_fwd_bwd(field, u, v, lat, lon, S.DT_DEFAULT, go, "bilinear")
+    assert sorted(os.listdir(tmp_path)) == ["grad_field.npy", "grad_u.npy", "grad_v.npy", "out.npy"]
+    for k, (name, mine) in enumerate(zip(bench.OUTPUT_NAMES, (R.out, R.gfield, R.gu, R.gv))):
+        a = np.load(tmp_path / f"{name}.npy")
+        assert a.dtype == np.float32 and a.shape == tuple(idx.shape), name
+        a = torch.from_numpy(a)
+        assert torch.equal(a, mine.reshape(-1)[idx].cpu()), name
+        if k < 3:      # the tolerances of test_fast_mode_white_noise_statistics
+            assert bad_fraction(a, ref[k].reshape(-1)[idx].cpu(), 1e-3 if k == 2 else 1e-4) < (2e-3 if k == 2 else 1e-3), name
