@@ -8,7 +8,8 @@
  *
  * Conventions
  *   - All tensors are fp32, NCHW, W innermost, device pointers unless the
- *     function name ends in _host.
+ *     function name ends in _host.  bf16 storage of the advection core's field, u, v
+ *     and their gradients: include/paradis_sl_bf16.h (same struct and status codes).
  *   - The caller owns every buffer (inputs, outputs, workspace).  The library
  *     never allocates or frees device memory and keeps no pointer after return.
  *   - Calls are asynchronous on `stream` (a cudaStream_t passed as void*), never

@@ -1,4 +1,5 @@
-"""ctypes binding of the C ABI declared in include/paradis_sl.h.
+"""ctypes binding of the C ABI declared in include/paradis_sl.h (and the bf16 entry points of
+include/paradis_sl_bf16.h, in a table of their own).
 
 The product has no CPU fallback: if the shared library is missing this module
 raises, it never substitutes another implementation.
@@ -62,8 +63,25 @@ _PROTOS = {
 }
 
 
+# include/paradis_sl_bf16.h: bf16 storage of field, u, v and their gradients (same ABI version: entry points added)
+_PROTOS_BF16 = {
+    "paradis_sl_advect_fwd_bf16": (C.c_int, [C.POINTER(Geom), _P, _P, _P, _P, C.c_int, C.c_int, C.c_int64, C.c_int64,
+                                             C.c_int64, C.c_float, C.c_int, C.c_int, C.c_int, _P, C.c_size_t, _P, _P]),
+    "paradis_sl_advect_bwd_bf16_workspace": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "paradis_sl_advect_bwd_bf16": (C.c_int, [C.POINTER(Geom), _P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int64,
+                                             C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_int, C.c_int, C.c_int,
+                                             C.c_int, C.c_float, _P, C.c_size_t, _P, _P]),
+}
+
+
 def exported_symbols():
+    """The functions of include/paradis_sl.h."""
     return list(_PROTOS)
+
+
+def exported_symbols_bf16():
+    """The functions of include/paradis_sl_bf16.h."""
+    return list(_PROTOS_BF16)
 
 
 def lib():
@@ -92,7 +110,7 @@ def lib():
             except Exception:
                 pass
         handle = C.CDLL(path)
-        for name, (res, args) in _PROTOS.items():
+        for name, (res, args) in list(_PROTOS.items()) + list(_PROTOS_BF16.items()):
             fn = getattr(handle, name)
             fn.restype, fn.argtypes = res, args
         if handle.paradis_sl_abi_version() != 2 and not os.environ.get("PARADIS_SL_SKIP_ABI_CHECK"):

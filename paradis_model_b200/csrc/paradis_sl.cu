@@ -23,6 +23,7 @@
 #include <vector>
 
 #include "../../include/paradis_sl.h"
+#include "../../include/paradis_sl_bf16.h"
 #include "sl_device.cuh"
 
 using namespace psl;
@@ -54,13 +55,14 @@ extern "C" const char* paradis_last_error(void) { return g_err; }
 // ---------------------------------------------------------------------------------------------
 // small helpers
 // ---------------------------------------------------------------------------------------------
-__device__ __forceinline__ const float* plane_ptr(const float* base, long long sB, int V, int rows,
-                                                  int W, int pl) {
+template <typename T>
+__device__ __forceinline__ const T* plane_ptr(const T* base, long long sB, int V, int rows, int W, int pl) {
   const int b = pl / V, c = pl - b * V;
   return base + (long long)b * sB + (long long)c * rows * W;
 }
 // same, for kernels launched on a (blocks, V, B) grid: no integer division
-__device__ __forceinline__ const float* plane_ptr_bc(const float* base, long long sB, int b, int c, int rows, int W) {
+template <typename T>
+__device__ __forceinline__ const T* plane_ptr_bc(const T* base, long long sB, int b, int c, int rows, int W) {
   return base + (long long)b * sB + (long long)c * rows * W;
 }
 
@@ -76,10 +78,11 @@ __device__ __forceinline__ float warp_row_sum(const float* row, int W, int lane)
 // deterministic zonal sum of one row by one 128-thread CTA: fixed per-thread order, shuffle tree, the four warp
 // partials added in warp order (one warp walking a 1440-element row took 8.5 us per launch, five launches per step)
 constexpr int kPoleThreads = 128;
-__device__ __forceinline__ float block_row_sum(const float* row, int W) {
+template <typename T>
+__device__ __forceinline__ float block_row_sum(const T* row, int W) {
   __shared__ float part[kPoleThreads / 32];
   float s = 0.0f;
-  for (int x = threadIdx.x; x < W; x += kPoleThreads) s += row[x];
+  for (int x = threadIdx.x; x < W; x += kPoleThreads) s += ld_f(row + x);
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
   if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = s;
@@ -93,22 +96,36 @@ __device__ __forceinline__ float block_row_sum(const float* row, int W) {
 
 // means[pl][k], k = 0: global row 0, k = 1: global row H-1 of tensor `t` whose window is (row0, rows); one CTA per
 // (plane, pole).  A second tensor (t2 -> means2, its own window) rides in the same launch (backward: field, grad_out).
-__global__ void __launch_bounds__(kPoleThreads) pole_means_kernel(const float* __restrict__ t, long long sB, int V, int rows, int row0,
+// T = storage type of `t` (field); t2 (grad_out) is fp32.
+template <typename T>
+__device__ __forceinline__ float pole_row_mean(const T* t, long long sB, int V, int rows, int row0, int H, int W, int job) {
+  const int pl = job >> 1, k = job & 1;
+  const int gr = k ? H - 1 : 0, lr = gr - row0;
+  float m = 0.0f;
+  if (lr >= 0 && lr < rows) {
+    const T* row = plane_ptr(t, sB, V, rows, W, pl) + (long long)lr * W;
+    m = block_row_sum(row, W) / (float)W;
+  }
+  return m;
+}
+template <typename T>
+__global__ void __launch_bounds__(kPoleThreads) pole_means_kernel(const T* __restrict__ t, long long sB, int V, int rows, int row0,
                                                                   int H, int W, int planes, float* __restrict__ means,
                                                                   const float* __restrict__ t2, long long sB2, int rows2,
                                                                   int row02, float* __restrict__ means2) {
   int job = blockIdx.x;
   if (job >= planes * 2) {
     if (!t2) return;
-    job -= planes * 2; t = t2; sB = sB2; rows = rows2; row0 = row02; means = means2;
+    job -= planes * 2;
+    if constexpr (kIsF32<T>) {
+      t = t2; sB = sB2; rows = rows2; row0 = row02; means = means2;
+    } else {                                   // fp32 grad_out beside a bf16 field
+      const float m = pole_row_mean(t2, sB2, V, rows2, row02, H, W, job);
+      if (threadIdx.x == 0) means2[job] = m;
+      return;
+    }
   }
-  const int pl = job >> 1, k = job & 1;
-  const int gr = k ? H - 1 : 0, lr = gr - row0;
-  float m = 0.0f;
-  if (lr >= 0 && lr < rows) {
-    const float* row = plane_ptr(t, sB, V, rows, W, pl) + (long long)lr * W;
-    m = block_row_sum(row, W) / (float)W;
-  }
+  const float m = pole_row_mean(t, sB, V, rows, row0, H, W, job);
   if (threadIdx.x == 0) means[job] = m;
 }
 
@@ -126,7 +143,7 @@ __global__ void __launch_bounds__(kPoleThreads) pole_rows_fix_kernel(float* __re
 // ---------------------------------------------------------------------------------------------
 // forward
 // ---------------------------------------------------------------------------------------------
-template <bool EXACT, int INTERP, int VEC, bool PEER>
+template <bool EXACT, int INTERP, int VEC, bool PEER, typename T>
 __global__ void __launch_bounds__(256) sl_fwd_kernel(const Params P) {
   const int c = blockIdx.y, b = blockIdx.z, pl = b * P.V + c;
   const unsigned unit = blockIdx.x * blockDim.x + threadIdx.x;
@@ -135,20 +152,20 @@ __global__ void __launch_bounds__(256) sl_fwd_kernel(const Params P) {
   const int x = (unit - r * P.upr) * VEC;
   const int y = P.own0 + (int)r;  // global arrival row
   const float sp = __ldg(P.sin_lat + y), cp = __ldg(P.cos_lat + y);
-  const float* f = plane_ptr_bc(P.field, P.field_sB, b, c, P.fldN, P.W);
+  const T* f = plane_ptr_bc(as<T>(P.field), P.field_sB, b, c, P.fldN, P.W);
   const int aoff = (y - P.uvg0) * P.W + x;
-  const float* up = plane_ptr_bc(P.u, P.u_sB, b, c, P.uvgN, P.W) + aoff;
-  const float* vp = plane_ptr_bc(P.v, P.v_sB, b, c, P.uvgN, P.W) + aoff;
+  const T* up = plane_ptr_bc(as<T>(P.u), P.u_sB, b, c, P.uvgN, P.W) + aoff;
+  const T* vp = plane_ptr_bc(as<T>(P.v), P.v_sB, b, c, P.uvgN, P.W) + aoff;
   float mean0 = 0.0f, mean1 = 0.0f;
   if (P.pole_fix) { mean0 = __ldg(P.fmean + 2 * pl); mean1 = __ldg(P.fmean + 2 * pl + 1); }
   float uu[VEC], vv[VEC], ll[VEC], oo[VEC];
   if (VEC == 4) {
-    *reinterpret_cast<float4*>(uu) = __ldcs(reinterpret_cast<const float4*>(up));
-    *reinterpret_cast<float4*>(vv) = __ldcs(reinterpret_cast<const float4*>(vp));
+    *reinterpret_cast<float4*>(uu) = ldcs4_f(up);
+    *reinterpret_cast<float4*>(vv) = ldcs4_f(vp);
     *reinterpret_cast<float4*>(ll) = __ldg(reinterpret_cast<const float4*>(P.lon + x));
   } else {
 #pragma unroll
-    for (int k = 0; k < VEC; ++k) { uu[k] = __ldcs(up + k); vv[k] = __ldcs(vp + k); ll[k] = __ldg(P.lon + x + k); }
+    for (int k = 0; k < VEC; ++k) { uu[k] = ldcs_f(up + k); vv[k] = ldcs_f(vp + k); ll[k] = __ldg(P.lon + x + k); }
   }
 #ifndef PSL_FWD_NO_PAIRS
   if (!EXACT && VEC == 4) {
@@ -240,7 +257,7 @@ __global__ void __launch_bounds__(256) sl_fwd_pair_kernel(const Params P, const 
 #include "sl_rows.cuh"
 #include "sl_partition.cuh"
 
-template <bool EXACT, int INTERP, int VEC, bool PEER>
+template <bool EXACT, int INTERP, int VEC, bool PEER, typename T>
 __global__ void __launch_bounds__(256) sl_bwd_arrival_kernel(const Params P) {
   const int c = blockIdx.y, b = blockIdx.z, pl = b * P.V + c;
   if (P.plane_filter && !P.plane_filter[pl]) return;   // uniform per block
@@ -254,22 +271,22 @@ __global__ void __launch_bounds__(256) sl_bwd_arrival_kernel(const Params P) {
     const int y = P.it_arr0 + (int)r;  // global arrival row
     const bool own = (y >= P.it_own0) && (y < P.it_own0 + P.it_ownN) && (P.gu != nullptr);
     const float sp = __ldg(P.sin_lat + y), cp = __ldg(P.cos_lat + y);
-    const float* up = arr_row<PEER>(P, plane_ptr_bc(P.u, P.u_sB, b, c, P.uvgN, P.W), 0, pl, y) + x;
-    const float* vp = arr_row<PEER>(P, plane_ptr_bc(P.v, P.v_sB, b, c, P.uvgN, P.W), 1, pl, y) + x;
+    const T* up = arr_row<PEER>(P, plane_ptr_bc(as<T>(P.u), P.u_sB, b, c, P.uvgN, P.W), 0, pl, y) + x;
+    const T* vp = arr_row<PEER>(P, plane_ptr_bc(as<T>(P.v), P.v_sB, b, c, P.uvgN, P.W), 1, pl, y) + x;
     float uu[VEC], vv[VEC], ll[VEC], gg[VEC], ou[VEC], ov[VEC];
     signed char cc[VEC];
     if (VEC == 4) {
-      *reinterpret_cast<float4*>(uu) = __ldg(reinterpret_cast<const float4*>(up));
-      *reinterpret_cast<float4*>(vv) = __ldg(reinterpret_cast<const float4*>(vp));
+      *reinterpret_cast<float4*>(uu) = ldg4_f(up);
+      *reinterpret_cast<float4*>(vv) = ldg4_f(vp);
       *reinterpret_cast<float4*>(ll) = __ldg(reinterpret_cast<const float4*>(P.lon + x));
     } else {
 #pragma unroll
-      for (int k = 0; k < VEC; ++k) { uu[k] = __ldg(up + k); vv[k] = __ldg(vp + k); ll[k] = __ldg(P.lon + x + k); }
+      for (int k = 0; k < VEC; ++k) { uu[k] = ldg_f(up + k); vv[k] = ldg_f(vp + k); ll[k] = __ldg(P.lon + x + k); }
     }
-    const float* f = nullptr;
+    const T* f = nullptr;
     float mean0 = 0.0f, mean1 = 0.0f;
     if (own) {
-      f = plane_ptr_bc(P.field, P.field_sB, b, c, P.fldN, P.W);
+      f = plane_ptr_bc(as<T>(P.field), P.field_sB, b, c, P.fldN, P.W);
       const float* gp = arr_row<PEER>(P, plane_ptr_bc(P.gout, P.gout_sB, b, c, P.uvgN, P.W), 2, pl, y) + x;
       if (VEC == 4) *reinterpret_cast<float4*>(gg) = __ldg(reinterpret_cast<const float4*>(gp));
       else {
@@ -314,11 +331,11 @@ __global__ void __launch_bounds__(256) sl_bwd_arrival_kernel(const Params P) {
     if (own) {
       const long long ooff = ((long long)pl * P.ownN + (y - P.own0)) * P.W + x;
       if (VEC == 4) {
-        __stcs(reinterpret_cast<float4*>(P.gu + ooff), *reinterpret_cast<float4*>(ou));
-        __stcs(reinterpret_cast<float4*>(P.gv + ooff), *reinterpret_cast<float4*>(ov));
+        stcs4_f(as<T>(P.gu) + ooff, *reinterpret_cast<float4*>(ou));
+        stcs4_f(as<T>(P.gv) + ooff, *reinterpret_cast<float4*>(ov));
       } else {
 #pragma unroll
-        for (int k = 0; k < VEC; ++k) { __stcs(P.gu + ooff + k, ou[k]); __stcs(P.gv + ooff + k, ov[k]); }
+        for (int k = 0; k < VEC; ++k) { stcs_f(as<T>(P.gu) + ooff + k, ou[k]); stcs_f(as<T>(P.gv) + ooff + k, ov[k]); }
       }
     }
   }
@@ -366,10 +383,11 @@ constexpr int kGatherWarps = 8;
 constexpr int kScan = 8;     // class bytes examined per lane and scan step
 constexpr int kQueue = 32 * kScan + 32;  // >= 31 left over + 32 * kScan new entries
 
-struct GatherPlane { const float* __restrict__ u; const float* __restrict__ v; const float* __restrict__ g; float gm0, gm1; int pl; };
+template <typename T>
+struct GatherPlane { const T* __restrict__ u; const T* __restrict__ v; const float* __restrict__ g; float gm0, gm1; int pl; };
 
-template <bool EXACT, int INTERP, bool PEER>
-__device__ __forceinline__ void gather_chunk(const Params& P, const GatherPlane& G, int Rd, int shift, float* acc,
+template <bool EXACT, int INTERP, bool PEER, typename T>
+__device__ __forceinline__ void gather_chunk(const Params& P, const GatherPlane<T>& G, int Rd, int shift, float* acc,
                                              const unsigned* queue, int n, int lane) {
   constexpr int NT = Stencil<INTERP>::NT, OMIN = Stencil<INTERP>::OMIN;
   float c[NT];
@@ -380,7 +398,7 @@ __device__ __forceinline__ void gather_chunk(const Params& P, const GatherPlane&
   if (lane < n) {
     const unsigned e = queue[lane];
     const int y = (int)(e >> 16), x = (int)(e & 0xffffu);  // global arrival row, column
-    const float uu = __ldg(arr_row<PEER>(P, G.u, 0, G.pl, y) + x), vv = __ldg(arr_row<PEER>(P, G.v, 1, G.pl, y) + x);
+    const float uu = ldg_f(arr_row<PEER>(P, G.u, 0, G.pl, y) + x), vv = ldg_f(arr_row<PEER>(P, G.v, 1, G.pl, y) + x);
     float g = __ldg(arr_row<PEER>(P, G.g, 2, G.pl, y) + x);
     if (P.pole_fix) {                         // adjoint of the output pole mean
       if (y == 0) g = G.gm0;
@@ -441,7 +459,7 @@ __device__ __forceinline__ void gather_chunk(const Params& P, const GatherPlane&
   }
 }
 
-template <bool EXACT, int INTERP, bool PEER>
+template <bool EXACT, int INTERP, bool PEER, typename T>
 __global__ void __launch_bounds__(kGatherWarps * 32) sl_bwd_gather_kernel(const Params P) {
   constexpr int NT = Stencil<INTERP>::NT, OMIN = Stencil<INTERP>::OMIN;
   extern __shared__ float smem[];
@@ -457,10 +475,10 @@ __global__ void __launch_bounds__(kGatherWarps * 32) sl_bwd_gather_kernel(const 
   __syncwarp();
   const int reach = P.plane_reach[pl];
   const signed char* cls = P.cls + (long long)pl * P.arrN * P.W;
-  GatherPlane G;
+  GatherPlane<T> G;
   G.pl = pl;
-  G.u = plane_ptr(P.u, P.u_sB, P.V, P.uvgN, P.W, pl);
-  G.v = plane_ptr(P.v, P.v_sB, P.V, P.uvgN, P.W, pl);
+  G.u = plane_ptr(as<T>(P.u), P.u_sB, P.V, P.uvgN, P.W, pl);
+  G.v = plane_ptr(as<T>(P.v), P.v_sB, P.V, P.uvgN, P.W, pl);
   G.g = plane_ptr(P.gout, P.gout_sB, P.V, P.uvgN, P.W, pl);
   G.gm0 = G.gm1 = 0.0f;
   if (P.pole_fix) { G.gm0 = __ldg(P.gmean + 2 * pl); G.gm1 = __ldg(P.gmean + 2 * pl + 1); }
@@ -680,29 +698,27 @@ extern "C" size_t paradis_sl_advect_fwd_workspace(int B, int V) {
   return align_up((size_t)B * V * 2 * sizeof(float), 256);
 }
 
-template <bool EXACT, int INTERP>
+// Peer halos are fp32 (latitude bands): the bf16 instantiations take the PEER = false kernel for both branches.
+template <bool EXACT, int INTERP, typename T>
 static void launch_fwd(const Params& P, int vec, dim3 grid, cudaStream_t st) {
+  constexpr bool kPeer = kIsF32<T>;
   const bool peer = P.f_halo > 0;
   if (vec == 4) {
-    if (peer) sl_fwd_kernel<EXACT, INTERP, 4, true><<<grid, 256, 0, st>>>(P);
-    else sl_fwd_kernel<EXACT, INTERP, 4, false><<<grid, 256, 0, st>>>(P);
+    if (peer) sl_fwd_kernel<EXACT, INTERP, 4, kPeer, T><<<grid, 256, 0, st>>>(P);
+    else sl_fwd_kernel<EXACT, INTERP, 4, false, T><<<grid, 256, 0, st>>>(P);
   } else {
-    if (peer) sl_fwd_kernel<EXACT, INTERP, 1, true><<<grid, 256, 0, st>>>(P);
-    else sl_fwd_kernel<EXACT, INTERP, 1, false><<<grid, 256, 0, st>>>(P);
+    if (peer) sl_fwd_kernel<EXACT, INTERP, 1, kPeer, T><<<grid, 256, 0, st>>>(P);
+    else sl_fwd_kernel<EXACT, INTERP, 1, false, T><<<grid, 256, 0, st>>>(P);
   }
 }
 
-
-extern "C" int paradis_sl_advect_fwd(const paradis_sl_geom* geom, const float* field, const float* u,
-                                     const float* v, float* out, int B, int V, int64_t field_sB, int64_t u_sB,
-                                     int64_t v_sB, float dt, int interp, int pole_fix, int math, void* workspace,
-                                     size_t workspace_bytes, int32_t* status, void* stream) {
-  Params P;
-  if (int rc = fill_params(P, geom, B, V, dt, interp, pole_fix)) return rc;
-  if (!field || !u || !v || !out) return fail(PARADIS_ERR_NULL_POINTER, "NULL tensor pointer");
-  cudaStream_t st = (cudaStream_t)stream;
+// Forward of either storage type once the arguments are checked; `field`, `u`, `v` hold T.
+template <typename T>
+static int advect_fwd(Params& P, const void* field, const void* u, const void* v, float* out, int B, int V,
+                      int64_t field_sB, int64_t u_sB, int64_t v_sB, int interp, int pole_fix, int math, void* workspace,
+                      size_t workspace_bytes, int32_t* status, cudaStream_t st) {
   const int planes = B * V;
-  P.field = field; P.u = u; P.v = v; P.out = out;
+  P.field = (const float*)field; P.u = (const float*)u; P.v = (const float*)v; P.out = out;
   P.field_sB = field_sB; P.u_sB = u_sB; P.v_sB = v_sB;
   P.status = status;
   if (pole_fix) {
@@ -710,8 +726,8 @@ extern "C" int paradis_sl_advect_fwd(const paradis_sl_geom* geom, const float* f
       return fail(PARADIS_ERR_WORKSPACE, "forward workspace too small (%zu bytes)", workspace_bytes);
     float* fmean = (float*)workspace;
     P.fmean = fmean;
-    pole_means_kernel<<<planes * 2, kPoleThreads, 0, st>>>(field, field_sB, V, P.fldN, P.fld0, P.H, P.W, planes, fmean, nullptr, 0,
-                                                            0, 0, nullptr);
+    pole_means_kernel<T><<<planes * 2, kPoleThreads, 0, st>>>((const T*)field, field_sB, V, P.fldN, P.fld0, P.H, P.W, planes,
+                                                               fmean, nullptr, 0, 0, 0, nullptr);
   }
   const bool vec_ok = (P.W % 4 == 0) && aligned16(field) && aligned16(u) && aligned16(v) && aligned16(out) &&
                       aligned16(P.lon) && (u_sB % 4 == 0) && (v_sB % 4 == 0);
@@ -721,16 +737,30 @@ extern "C" int paradis_sl_advect_fwd(const paradis_sl_geom* geom, const float* f
   dim3 grid((units + 255) / 256, V, B);
   const bool exact = math == PARADIS_MATH_EXACT;
   // experiments: PARADIS_SL_FWD=2 selects the packed-pair forward (consecutive lanes on consecutive columns, FFMA2
-  // trajectory): bit-identical output, measured 0.43 ms against 0.38 ms for the float4-per-thread kernel at C3
+  // trajectory, fp32 storage only): bit-identical output, measured 0.43 ms against 0.38 ms for the float4-per-thread
+  // kernel at C3
   static const int fwd_mode = getenv("PARADIS_SL_FWD") ? atoi(getenv("PARADIS_SL_FWD")) : 0;
-  if (!exact && interp == 1 && fwd_mode == 2) {
+  if (kIsF32<T> && !exact && interp == 1 && fwd_mode == 2) {
     const int gpr = (P.W + 127) / 128;
     dim3 pgrid((unsigned)(((long long)gpr * P.ownN + 7) / 8), V, B);       // 8 warps per CTA
     if (P.f_halo > 0) sl_fwd_pair_kernel<1, true><<<pgrid, 256, 0, st>>>(P, gpr);
     else sl_fwd_pair_kernel<1, false><<<pgrid, 256, 0, st>>>(P, gpr);
-  } else if (interp == 1) { if (exact) launch_fwd<true, 1>(P, vec, grid, st); else launch_fwd<false, 1>(P, vec, grid, st); }
-  else             { if (exact) launch_fwd<true, 2>(P, vec, grid, st); else launch_fwd<false, 2>(P, vec, grid, st); }
+  } else if (interp == 1) { if (exact) launch_fwd<true, 1, T>(P, vec, grid, st); else launch_fwd<false, 1, T>(P, vec, grid, st); }
+  else             { if (exact) launch_fwd<true, 2, T>(P, vec, grid, st); else launch_fwd<false, 2, T>(P, vec, grid, st); }
   if (pole_fix) pole_rows_fix_kernel<<<planes * 2, kPoleThreads, 0, st>>>(out, P.ownN, P.own0, P.H, P.W, planes);
+  return PARADIS_OK;
+}
+
+extern "C" int paradis_sl_advect_fwd(const paradis_sl_geom* geom, const float* field, const float* u,
+                                     const float* v, float* out, int B, int V, int64_t field_sB, int64_t u_sB,
+                                     int64_t v_sB, float dt, int interp, int pole_fix, int math, void* workspace,
+                                     size_t workspace_bytes, int32_t* status, void* stream) {
+  Params P;
+  if (int rc = fill_params(P, geom, B, V, dt, interp, pole_fix)) return rc;
+  if (!field || !u || !v || !out) return fail(PARADIS_ERR_NULL_POINTER, "NULL tensor pointer");
+  if (int rc = advect_fwd<float>(P, field, u, v, out, B, V, field_sB, u_sB, v_sB, interp, pole_fix, math, workspace,
+                                 workspace_bytes, status, (cudaStream_t)stream))
+    return rc;
   return check_launch("paradis_sl_advect_fwd");
 }
 
@@ -767,8 +797,9 @@ extern "C" size_t paradis_sl_advect_bwd_workspace(int B, int V, int arr_rows, in
 }
 
 // General (two-kernel) backward over the iteration windows set in P.
-template <bool EXACT, int INTERP>
+template <bool EXACT, int INTERP, typename T>
 static int launch_general(Params P, int vec, cudaStream_t st, bool want_field, int phases, int max_nblk) {
+  constexpr bool kPeer = kIsF32<T>;   // see launch_fwd
   const int planes = P.B * P.V;
   // the filtered (fallback) launch mostly consists of blocks that exit at once: keep their number small
   vec = (P.plane_filter && vec == 4) ? 4 : points_per_thread(INTERP, vec == 4);
@@ -781,11 +812,11 @@ static int launch_general(Params P, int vec, cudaStream_t st, bool want_field, i
   if (phases & PARADIS_BWD_ARRIVAL) {
     const bool peer = P.f_halo > 0 || P.a_halo > 0;
     if (vec == 4) {
-      if (peer) sl_bwd_arrival_kernel<EXACT, INTERP, 4, true><<<grid, 256, 0, st>>>(P);
-      else sl_bwd_arrival_kernel<EXACT, INTERP, 4, false><<<grid, 256, 0, st>>>(P);
+      if (peer) sl_bwd_arrival_kernel<EXACT, INTERP, 4, kPeer, T><<<grid, 256, 0, st>>>(P);
+      else sl_bwd_arrival_kernel<EXACT, INTERP, 4, false, T><<<grid, 256, 0, st>>>(P);
     } else {
-      if (peer) sl_bwd_arrival_kernel<EXACT, INTERP, 1, true><<<grid, 256, 0, st>>>(P);
-      else sl_bwd_arrival_kernel<EXACT, INTERP, 1, false><<<grid, 256, 0, st>>>(P);
+      if (peer) sl_bwd_arrival_kernel<EXACT, INTERP, 1, kPeer, T><<<grid, 256, 0, st>>>(P);
+      else sl_bwd_arrival_kernel<EXACT, INTERP, 1, false, T><<<grid, 256, 0, st>>>(P);
     }
     if (want_field)
       plane_reach_kernel<<<(planes * 32 + 255) / 256, 256, 0, st>>>(P.blkmax, P.nblk, planes, P.plane_reach,
@@ -794,7 +825,7 @@ static int launch_general(Params P, int vec, cudaStream_t st, bool want_field, i
   if (!want_field || !(phases & PARADIS_BWD_GATHER)) return PARADIS_OK;
   const size_t smem = (size_t)kGatherWarps * (P.W + kQueue) * sizeof(float);
   if (smem > 227 * 1024) return fail(PARADIS_ERR_BAD_SHAPE, "W=%d too wide for the gather kernel's shared memory", P.W);
-  auto kern = P.a_halo > 0 ? sl_bwd_gather_kernel<EXACT, INTERP, true> : sl_bwd_gather_kernel<EXACT, INTERP, false>;
+  auto kern = P.a_halo > 0 ? sl_bwd_gather_kernel<EXACT, INTERP, kPeer, T> : sl_bwd_gather_kernel<EXACT, INTERP, false, T>;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return fail(PARADIS_ERR_CUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
   dim3 ggrid((P.it_ownN + kGatherWarps - 1) / kGatherWarps, planes);
@@ -896,7 +927,7 @@ __global__ void rows_prep_kernel(const float* __restrict__ sin_lat, const float*
   if (i < planes) flag[i] = 0;
 }
 
-template <bool EXACT, int INTERP>
+template <bool EXACT, int INTERP, typename T>
 static bool launch_rows(const Params& P, cudaStream_t st, float cfl_cells, const BwdWs& L, char* ws, bool forced) {
   constexpr int NT = Stencil<INTERP>::NT, OMIN = Stencil<INTERP>::OMIN;
   const int H = P.H, W = P.W, planes = P.B * P.V;
@@ -926,13 +957,13 @@ static bool launch_rows(const Params& P, cudaStream_t st, float cfl_cells, const
   S.pitch = (wc + NT - 1 + 3) & ~3;
   S.ring_stride = (S.ring + NT - 1) * S.pitch;
   size_t off = (size_t)nS * S.ring_stride * sizeof(float);
-  S.off_stage = (unsigned)off; off += (size_t)kRowStages * 3 * W * sizeof(float);
+  S.off_stage = (unsigned)off; off += (size_t)kRowStages * 3 * W * sizeof(float);   // (bf16 u, v use 2 W bytes each of it)
   S.off_rec = (unsigned)off; off += (size_t)kRowRecs * W * sizeof(float4);
   S.off_tag = (unsigned)off; off += (size_t)nS * kTagBytes;
   S.off_bar = (unsigned)off; off += (2 * kRowStages + 2 * kRowRecs) * sizeof(uint64_t);
   const size_t smem = off;
   if (smem > 227 * 1024) return false;
-  auto kern = (P.f_halo > 0 || P.a_halo > 0) ? sl_bwd_rows_kernel<EXACT, INTERP, true> : sl_bwd_rows_kernel<EXACT, INTERP, false>;
+  auto kern = (P.f_halo > 0 || P.a_halo > 0) ? sl_bwd_rows_kernel<EXACT, INTERP, kIsF32<T>, T> : sl_bwd_rows_kernel<EXACT, INTERP, false, T>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
     cudaGetLastError();
     return false;
@@ -1013,7 +1044,7 @@ static int device_capacity(const void* kern, int threads, size_t smem, int& nsm)
   return blocks;
 }
 
-template <bool EXACT, int INTERP>
+template <bool EXACT, int INTERP, typename T>
 static int launch_bwd(Params P, int vec, cudaStream_t st, int phases, float cfl_cells, const BwdWs& L, char* ws) {
   const bool force_rows = (phases & PARADIS_BWD_ROWSWEEP) != 0;
   phases &= PARADIS_BWD_ALL;
@@ -1021,25 +1052,25 @@ static int launch_bwd(Params P, int vec, cudaStream_t st, int phases, float cfl_
   const int planes = P.B * P.V;
   P.plane_filter = nullptr; P.plane_flag = nullptr; P.reach_limit = 1 << 20;
   if (!want_field || phases != PARADIS_BWD_ALL || !(cfl_cells > 0.0f) || vec != 4)   // the sweep needs float4 rows
-    return launch_general<EXACT, INTERP>(P, vec, st, want_field, phases, L.nblk);
+    return launch_general<EXACT, INTERP, T>(P, vec, st, want_field, phases, L.nblk);
 
   // ---- warp-specialised row sweep (all latitudes); planes that break its contract fall back below
   static const int bwd_mode = env_int("PARADIS_SL_BWD", 0);      // experiments: 1 = round-1 strip sweep, 2 = general path only
-  if (bwd_mode == 2) return launch_general<EXACT, INTERP>(P, vec, st, want_field, phases, L.nblk);
+  if (bwd_mode == 2) return launch_general<EXACT, INTERP, T>(P, vec, st, want_field, phases, L.nblk);
   // (4x4 stencil: the round-1 strip sweep is still the faster kernel, 3.65 against 4.6 ms at C3; PARADIS_SL_BWD=3
   // forces the row sweep for it)
   if ((bwd_mode == 3 || force_rows || (bwd_mode == 0 && INTERP == 1)) &&
-      launch_rows<EXACT, INTERP>(P, st, cfl_cells, L, ws, bwd_mode == 3 || force_rows)) {
+      launch_rows<EXACT, INTERP, T>(P, st, cfl_cells, L, ws, bwd_mode == 3 || force_rows)) {
     Params Q = P;
     Q.plane_filter = (unsigned char*)(ws + L.flag);
     Q.gu = nullptr; Q.gv = nullptr;                   // grad_u / grad_v are already complete
-    return launch_general<EXACT, INTERP>(Q, vec, st, true, PARADIS_BWD_ALL, L.nblk);
+    return launch_general<EXACT, INTERP, T>(Q, vec, st, true, PARADIS_BWD_ALL, L.nblk);
   }
   // ---- fused sweep over the mid-latitudes
   constexpr int NT = Stencil<INTERP>::NT;
   SweepPlan S;
   memset(&S, 0, sizeof(S));
-  auto kern = (P.f_halo > 0 || P.a_halo > 0) ? sl_bwd_sweep_kernel<EXACT, INTERP, true> : sl_bwd_sweep_kernel<EXACT, INTERP, false>;
+  auto kern = (P.f_halo > 0 || P.a_halo > 0) ? sl_bwd_sweep_kernel<EXACT, INTERP, kIsF32<T>, T> : sl_bwd_sweep_kernel<EXACT, INTERP, false, T>;
   const int rr = (int)ceil((double)cfl_cells);
   const size_t smem = (size_t)kSweepWarps * sweep_warp_floats(2 * rr + NT, sweep_pitch(kSweepStrip)) * sizeof(float);
   int lo = -1, hi = -1, nsm = 148;
@@ -1049,7 +1080,7 @@ static int launch_bwd(Params P, int vec, cudaStream_t st, int phases, float cfl_
   ok = ok && blocks_per_sm > 0 && plan_sweep<INTERP>(P, cfl_cells, planes, blocks_per_sm * nsm * kSweepWarps, S, lo, hi);
   if (!ok) {
     cudaGetLastError();
-    return launch_general<EXACT, INTERP>(P, vec, st, want_field, phases, L.nblk);
+    return launch_general<EXACT, INTERP, T>(P, vec, st, want_field, phases, L.nblk);
   }
   unsigned char* flag = (unsigned char*)(ws + L.flag);
   cudaMemsetAsync(flag, 0, planes, st);
@@ -1078,7 +1109,7 @@ static int launch_bwd(Params P, int vec, cudaStream_t st, int phases, float cfl_
     Q.blkmax = (unsigned char*)(ws + L.blkmax + (k + 1) * L.blkmax_stride);
     cudaStream_t cs = st;
     if (side) { cs = side->s[k]; cudaStreamWaitEvent(cs, side->fork, 0); forked[k] = true; }
-    if (int rc = launch_general<EXACT, INTERP>(Q, vec, cs, true, PARADIS_BWD_ALL, L.nblk)) return rc;
+    if (int rc = launch_general<EXACT, INTERP, T>(Q, vec, cs, true, PARADIS_BWD_ALL, L.nblk)) return rc;
     if (side) cudaEventRecord(side->join[k], cs);
   }
   for (int k = 0; k < 2; ++k)
@@ -1087,7 +1118,40 @@ static int launch_bwd(Params P, int vec, cudaStream_t st, int phases, float cfl_
   Params Q = P;
   Q.plane_filter = flag;
   Q.gu = nullptr; Q.gv = nullptr;                   // grad_u / grad_v are already complete
-  return launch_general<EXACT, INTERP>(Q, vec, st, true, PARADIS_BWD_ALL, L.nblk);
+  return launch_general<EXACT, INTERP, T>(Q, vec, st, true, PARADIS_BWD_ALL, L.nblk);
+}
+
+// Backward of either storage type once the arguments are checked; `field`, `u`, `v`, `grad_u`, `grad_v` hold T,
+// grad_field is fp32 (the bf16 entry passes its fp32 accumulation buffer).
+template <typename T>
+static int advect_bwd(Params& P, const BwdWs& L, const float* grad_out, const void* field, const void* u, const void* v,
+                      float* grad_field, void* grad_u, void* grad_v, int B, int V, int64_t gout_sB, int64_t field_sB,
+                      int64_t u_sB, int64_t v_sB, int interp, int pole_fix, int math, int phases, float cfl_cells,
+                      char* ws, int32_t* status, cudaStream_t st) {
+  const int planes = B * V;
+  float* fmean = (float*)(ws + L.fmean);
+  float* gmean = (float*)(ws + L.gmean);
+  P.field = (const float*)field; P.u = (const float*)u; P.v = (const float*)v; P.gout = grad_out;
+  P.gfield = grad_field; P.gu = (float*)grad_u; P.gv = (float*)grad_v;
+  P.field_sB = field_sB; P.u_sB = u_sB; P.v_sB = v_sB; P.gout_sB = gout_sB;
+  P.status = status;
+  P.fmean = fmean; P.gmean = gmean;
+  P.plane_reach = (int*)(ws + L.reach);
+  P.blkmax = grad_field ? (unsigned char*)(ws + L.blkmax) : nullptr;
+  P.cls = grad_field ? (signed char*)(ws + L.cls) : nullptr;
+  P.nblk = L.nblk;
+  if (pole_fix && (phases & PARADIS_BWD_ARRIVAL))      // zonal pole means of field and grad_out in one launch
+    pole_means_kernel<T><<<planes * 4, kPoleThreads, 0, st>>>((const T*)field, field_sB, V, P.fldN, P.fld0, P.H, P.W, planes,
+                                                               fmean, grad_out, gout_sB, P.uvgN, P.uvg0, gmean);
+  const bool vec_ok = (P.W % 4 == 0) && aligned16(field) && aligned16(u) && aligned16(v) && aligned16(grad_out) &&
+                      aligned16(P.lon) && (!grad_u || (aligned16(grad_u) && aligned16(grad_v))) &&
+                      (!grad_field || aligned16(grad_field)) &&   // the sweep retires rows with float4 stores
+                      (u_sB % 4 == 0) && (v_sB % 4 == 0) && (gout_sB % 4 == 0);
+  const int vec = vec_ok ? 4 : 1;   // float4 rows available (the sweep needs them); the arrival kernel picks its own
+  const bool exact = math == PARADIS_MATH_EXACT;
+  if (interp == 1)
+    return exact ? launch_bwd<true, 1, T>(P, vec, st, phases, cfl_cells, L, ws) : launch_bwd<false, 1, T>(P, vec, st, phases, cfl_cells, L, ws);
+  return exact ? launch_bwd<true, 2, T>(P, vec, st, phases, cfl_cells, L, ws) : launch_bwd<false, 2, T>(P, vec, st, phases, cfl_cells, L, ws);
 }
 
 extern "C" int paradis_sl_advect_bwd(const paradis_sl_geom* geom, const float* grad_out, const float* field,
@@ -1105,34 +1169,101 @@ extern "C" int paradis_sl_advect_bwd(const paradis_sl_geom* geom, const float* g
   const BwdWs L = bwd_layout(B, V, P.arrN, P.W);
   if (!workspace || workspace_bytes < L.total)
     return fail(PARADIS_ERR_WORKSPACE, "backward workspace too small (%zu < %zu bytes)", workspace_bytes, L.total);
-  cudaStream_t st = (cudaStream_t)stream;
-  const int planes = B * V;
-  char* ws = (char*)workspace;
-  float* fmean = (float*)(ws + L.fmean);
-  float* gmean = (float*)(ws + L.gmean);
-  P.field = field; P.u = u; P.v = v; P.gout = grad_out;
-  P.gfield = grad_field; P.gu = grad_u; P.gv = grad_v;
-  P.field_sB = field_sB; P.u_sB = u_sB; P.v_sB = v_sB; P.gout_sB = gout_sB;
-  P.status = status;
-  P.fmean = fmean; P.gmean = gmean;
-  P.plane_reach = (int*)(ws + L.reach);
-  P.blkmax = grad_field ? (unsigned char*)(ws + L.blkmax) : nullptr;
-  P.cls = grad_field ? (signed char*)(ws + L.cls) : nullptr;
-  P.nblk = L.nblk;
-  if (pole_fix && (phases & PARADIS_BWD_ARRIVAL))      // zonal pole means of field and grad_out in one launch
-    pole_means_kernel<<<planes * 4, kPoleThreads, 0, st>>>(field, field_sB, V, P.fldN, P.fld0, P.H, P.W, planes, fmean, grad_out,
-                                                            gout_sB, P.uvgN, P.uvg0, gmean);
-  const bool vec_ok = (P.W % 4 == 0) && aligned16(field) && aligned16(u) && aligned16(v) && aligned16(grad_out) &&
-                      aligned16(P.lon) && (!grad_u || (aligned16(grad_u) && aligned16(grad_v))) &&
-                      (!grad_field || aligned16(grad_field)) &&   // the sweep retires rows with float4 stores
-                      (u_sB % 4 == 0) && (v_sB % 4 == 0) && (gout_sB % 4 == 0);
-  const int vec = vec_ok ? 4 : 1;   // float4 rows available (the sweep needs them); the arrival kernel picks its own
-  const bool exact = math == PARADIS_MATH_EXACT;
-  int rc;
-  if (interp == 1) rc = exact ? launch_bwd<true, 1>(P, vec, st, phases, cfl_cells, L, ws) : launch_bwd<false, 1>(P, vec, st, phases, cfl_cells, L, ws);
-  else             rc = exact ? launch_bwd<true, 2>(P, vec, st, phases, cfl_cells, L, ws) : launch_bwd<false, 2>(P, vec, st, phases, cfl_cells, L, ws);
-  if (rc) return rc;
+  if (int rc = advect_bwd<float>(P, L, grad_out, field, u, v, grad_field, grad_u, grad_v, B, V, gout_sB, field_sB, u_sB,
+                                 v_sB, interp, pole_fix, math, phases, cfl_cells, (char*)workspace, status,
+                                 (cudaStream_t)stream))
+    return rc;
   return check_launch("paradis_sl_advect_bwd");
+}
+
+// ---------------------------------------------------------------------------------------------
+// bf16 storage (include/paradis_sl_bf16.h): the same kernels instantiated with T = bf16, same plan
+// ---------------------------------------------------------------------------------------------
+// grad_field: fp32 accumulation buffer -> bf16, 8 values per thread, rounded once after the last pass that adds to it
+__global__ void f32_to_bf16_kernel(const float* __restrict__ src, bf16* __restrict__ dst, long long n8) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (long long)gridDim.x * blockDim.x) {
+    const float4 a = __ldcs(reinterpret_cast<const float4*>(src) + 2 * i);
+    const float4 b = __ldcs(reinterpret_cast<const float4*>(src) + 2 * i + 1);
+    __stcs(reinterpret_cast<uint4*>(dst) + i, make_uint4(f2_to_bf2(a.x, a.y), f2_to_bf2(a.z, a.w), f2_to_bf2(b.x, b.y),
+                                                          f2_to_bf2(b.z, b.w)));
+  }
+}
+
+// Native bf16 path: full mesh only (default windows, no peer halos), W % 8 == 0, 16-byte aligned tensors, batch
+// strides in multiples of 8 elements (bf16) resp. 4 elements (fp32): every row then starts on 16 bytes.
+static int bf16_check(const paradis_sl_geom* g, const void* const* ptrs, int nptrs, const int64_t* sB8, int nsB8,
+                      const int64_t* sB4, int nsB4) {
+  const int H = g->H;
+  if (g->own_row0 != 0 || g->own_rows != H || g->arr_row0 != 0 || g->arr_rows != H || g->fld_row0 != 0 ||
+      g->fld_rows != H)
+    return fail(PARADIS_ERR_BAD_SHAPE, "bf16 entry points work on the full mesh (latitude bands: use the fp32 entry points)");
+  bool peers = g->fld_peer_lo || g->fld_peer_hi;
+  for (int k = 0; k < 3; ++k) peers = peers || g->arr_peer_lo[k] || g->arr_peer_hi[k];
+  if (peers) return fail(PARADIS_ERR_BAD_SHAPE, "bf16 entry points take no peer halo pointers");
+  if (g->W % 8) return fail(PARADIS_ERR_BAD_SHAPE, "bf16 entry points need W %% 8 == 0 (W=%d)", g->W);
+  if (!aligned16(g->lon)) return fail(PARADIS_ERR_BAD_SHAPE, "bf16 entry points need a 16-byte aligned lon table");
+  for (int k = 0; k < nptrs; ++k)
+    if (ptrs[k] && !aligned16(ptrs[k])) return fail(PARADIS_ERR_BAD_SHAPE, "bf16 entry points need 16-byte aligned tensors");
+  for (int k = 0; k < nsB8; ++k)
+    if (sB8[k] % 8) return fail(PARADIS_ERR_BAD_SHAPE, "bf16 tensors need batch strides in multiples of 8 elements");
+  for (int k = 0; k < nsB4; ++k)
+    if (sB4[k] % 4) return fail(PARADIS_ERR_BAD_SHAPE, "grad_out needs a batch stride in multiples of 4 elements");
+  return PARADIS_OK;
+}
+
+extern "C" int paradis_sl_advect_fwd_bf16(const paradis_sl_geom* geom, const void* field, const void* u, const void* v,
+                                          float* out, int B, int V, int64_t field_sB, int64_t u_sB, int64_t v_sB,
+                                          float dt, int interp, int pole_fix, int math, void* workspace,
+                                          size_t workspace_bytes, int32_t* status, void* stream) {
+  Params P;
+  if (int rc = fill_params(P, geom, B, V, dt, interp, pole_fix)) return rc;
+  if (!field || !u || !v || !out) return fail(PARADIS_ERR_NULL_POINTER, "NULL tensor pointer");
+  const void* ptrs[4] = {field, u, v, out};
+  const int64_t sB8[3] = {field_sB, u_sB, v_sB};
+  if (int rc = bf16_check(geom, ptrs, 4, sB8, 3, nullptr, 0)) return rc;
+  if (int rc = advect_fwd<bf16>(P, field, u, v, out, B, V, field_sB, u_sB, v_sB, interp, pole_fix, math, workspace,
+                                workspace_bytes, status, (cudaStream_t)stream))
+    return rc;
+  return check_launch("paradis_sl_advect_fwd_bf16");
+}
+
+// fp32 workspace of the backward, then the fp32 grad_field accumulation buffer
+extern "C" size_t paradis_sl_advect_bwd_bf16_workspace(int B, int V, int arr_rows, int W) {
+  return bwd_layout(B, V, arr_rows, W).total + align_up((size_t)B * V * arr_rows * W * sizeof(float), 256);
+}
+
+extern "C" int paradis_sl_advect_bwd_bf16(const paradis_sl_geom* geom, const float* grad_out, const void* field,
+                                          const void* u, const void* v, void* grad_field, void* grad_u, void* grad_v,
+                                          int B, int V, int64_t gout_sB, int64_t field_sB, int64_t u_sB, int64_t v_sB,
+                                          float dt, int interp, int pole_fix, int math, int phases, float cfl_cells,
+                                          void* workspace, size_t workspace_bytes, int32_t* status, void* stream) {
+  Params P;
+  if (int rc = fill_params(P, geom, B, V, dt, interp, pole_fix)) return rc;
+  if (!grad_out || !field || !u || !v) return fail(PARADIS_ERR_NULL_POINTER, "NULL tensor pointer");
+  if ((phases & ~(PARADIS_BWD_ALL | PARADIS_BWD_ROWSWEEP)) || !(phases & PARADIS_BWD_ALL))
+    return fail(PARADIS_ERR_BAD_SHAPE, "phases must be 1, 2 or 3 (optionally | PARADIS_BWD_ROWSWEEP)");
+  if ((grad_u == nullptr) != (grad_v == nullptr)) return fail(PARADIS_ERR_NULL_POINTER, "grad_u and grad_v must both be given or both be NULL");
+  const void* ptrs[7] = {grad_out, field, u, v, grad_field, grad_u, grad_v};
+  const int64_t sB8[3] = {field_sB, u_sB, v_sB}, sB4[1] = {gout_sB};
+  if (int rc = bf16_check(geom, ptrs, 7, sB8, 3, sB4, 1)) return rc;
+  const BwdWs L = bwd_layout(B, V, P.arrN, P.W);
+  if (!workspace || workspace_bytes < paradis_sl_advect_bwd_bf16_workspace(B, V, P.arrN, P.W))
+    return fail(PARADIS_ERR_WORKSPACE, "backward workspace too small (%zu < %zu bytes)", workspace_bytes,
+                paradis_sl_advect_bwd_bf16_workspace(B, V, P.arrN, P.W));
+  cudaStream_t st = (cudaStream_t)stream;
+  // grad_field is accumulated in fp32 (ring retire, guard / cut / pole fix-ups and the recompute of flagged planes all
+  // add to or overwrite fp32 values after the first store) and rounded to bf16 once at the end
+  float* gf32 = grad_field ? (float*)((char*)workspace + L.total) : nullptr;
+  if (int rc = advect_bwd<bf16>(P, L, grad_out, field, u, v, gf32, grad_u, grad_v, B, V, gout_sB, field_sB, u_sB, v_sB,
+                                interp, pole_fix, math, phases, cfl_cells, (char*)workspace, status, st))
+    return rc;
+  if (grad_field && (phases & PARADIS_BWD_GATHER)) {
+    const long long n8 = (long long)B * V * P.ownN * P.W / 8;
+    long long blocks = (n8 + 255) / 256;
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    f32_to_bf16_kernel<<<(unsigned)blocks, 256, 0, st>>>(gf32, (bf16*)grad_field, n8);
+  }
+  return check_launch("paradis_sl_advect_bwd_bf16");
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -323,8 +323,8 @@ __device__ __noinline__ void rows_scatter_fold(int W, int H, const float4 rec, b
 }
 
 // ---- producer: one arrival point -> record (+ grad_u, grad_v for the rows this segment owns) -----
-template <bool EXACT, int INTERP, bool PEER, bool SMALL>
-__device__ __forceinline__ float4 rows_point(const Params& P, const float* __restrict__ f, int pl, float mean0,
+template <bool EXACT, int INTERP, bool PEER, bool SMALL, typename T>
+__device__ __forceinline__ float4 rows_point(const Params& P, const T* __restrict__ f, int pl, float mean0,
                                              float mean1, float sp, float cp, int y, int x, int rr, int hx, int hbase,
                                              int ring, bool core, float uu, float vv, float g, float lonp,
                                              bool& violated, float& ou, float& ov) {
@@ -356,8 +356,8 @@ __device__ __forceinline__ float4 rows_point(const Params& P, const float* __res
 
 // FAST math: two arrival points of one row at a time, trajectory and Jacobian on the packed fp32x2 pipe
 // (bit-identical to rows_point<false, ...> for each of them)
-template <int INTERP, bool PEER>
-__device__ __forceinline__ void rows_pair(const Params& P, const float* __restrict__ f, int pl, float mean0, float mean1,
+template <int INTERP, bool PEER, typename T>
+__device__ __forceinline__ void rows_pair(const Params& P, const T* __restrict__ f, int pl, float mean0, float mean1,
                                           float sp, float cp, int y, const int (&x)[2], int rr, int hx, int hbase, int ring,
                                           bool core, f2 uu, f2 vv, f2 g, f2 lonp, bool& violated, float4 (&rec)[2], f2& ou,
                                           f2& ov) {
@@ -428,7 +428,9 @@ __device__ __noinline__ void rows_flush_row(float* ringp, int head, int ring, in
   __syncwarp();
 }
 
-template <bool EXACT, int INTERP, bool PEER>
+// T: storage type of field, u, v, grad_u, grad_v.  A stage holds the u, v rows (W * sizeof(T) bytes each) and the fp32
+// grad_out row, back to back; its size is 3 W floats whatever T is, so the plan does not depend on it.
+template <bool EXACT, int INTERP, bool PEER, typename T>
 __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const Params P, const RowsPlan S) {
   constexpr int NT = Stencil<INTERP>::NT, OMIN = Stencil<INTERP>::OMIN;
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -467,18 +469,18 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
     // measured: no effect, 1.837 against 1.835 ms)
     if (lane != 0) return;
     int n = 0;
-    const uint32_t row_bytes = (uint32_t)W * 4u;
+    const uint32_t row_bytes = (uint32_t)W * 4u, uv_bytes = (uint32_t)(W * sizeof(T));   // bf16: W % 8 == 0 (16-byte copies)
     while (rows_next_seg<INTERP>(P, S, g, g1, sg)) {
-      const float* up = plane_ptr(P.u, P.u_sB, P.V, P.uvgN, W, sg.pl);
-      const float* vp = plane_ptr(P.v, P.v_sB, P.V, P.uvgN, W, sg.pl);
+      const T* up = plane_ptr(as<T>(P.u), P.u_sB, P.V, P.uvgN, W, sg.pl);
+      const T* vp = plane_ptr(as<T>(P.v), P.v_sB, P.V, P.uvgN, W, sg.pl);
       const float* gp = plane_ptr(P.gout, P.gout_sB, P.V, P.uvgN, W, sg.pl);
       for (int y = max(sg.y_first, arr_lo); y <= min(sg.y_last, arr_hi - 1); ++y, ++n) {
         const int st = n % kRowStages;
         mbar_wait(&stage_free[st], ((n / kRowStages) & 1) ^ 1);
-        float* dst = stage_base + (size_t)st * 3 * W;
-        mbar_arrive_expect_tx(&stage_full[st], 3 * row_bytes);
-        bulk_g2s(dst, arr_row<PEER>(P, up, 0, sg.pl, y), row_bytes, &stage_full[st]);
-        bulk_g2s(dst + W, arr_row<PEER>(P, vp, 1, sg.pl, y), row_bytes, &stage_full[st]);
+        T* dst = reinterpret_cast<T*>(stage_base + (size_t)st * 3 * W);
+        mbar_arrive_expect_tx(&stage_full[st], kIsF32<T> ? 3 * row_bytes : 2 * uv_bytes + row_bytes);
+        bulk_g2s(dst, arr_row<PEER>(P, up, 0, sg.pl, y), uv_bytes, &stage_full[st]);
+        bulk_g2s(dst + W, arr_row<PEER>(P, vp, 1, sg.pl, y), uv_bytes, &stage_full[st]);
         bulk_g2s(dst + 2 * W, arr_row<PEER>(P, gp, 2, sg.pl, y), row_bytes, &stage_full[st]);
       }
     }
@@ -495,9 +497,9 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
     while (rows_next_seg<INTERP>(P, S, g, g1, sg)) {
       const int pl = sg.pl;
       const int b = pl / P.V, c = pl - b * P.V;
-      const float* f = plane_ptr_bc(P.field, P.field_sB, b, c, P.fldN, W);
-      float* gu_pl = P.gu ? P.gu + (long long)pl * S.outN * W : nullptr;
-      float* gv_pl = P.gu ? P.gv + (long long)pl * S.outN * W : nullptr;
+      const T* f = plane_ptr_bc(as<T>(P.field), P.field_sB, b, c, P.fldN, W);
+      T* gu_pl = P.gu ? as<T>(P.gu) + (long long)pl * S.outN * W : nullptr;
+      T* gv_pl = P.gu ? as<T>(P.gv) + (long long)pl * S.outN * W : nullptr;
       float mean0 = 0.0f, mean1 = 0.0f, gm0 = 0.0f, gm1 = 0.0f;
       if (P.pole_fix) {
         mean0 = __ldg(P.fmean + 2 * pl); mean1 = __ldg(P.fmean + 2 * pl + 1);
@@ -517,7 +519,8 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
           if (lane == 0) { mbar_arrive(&stage_free[st]); mbar_arrive(&rec_full[rs]); }
           continue;
         }
-        const float* su = stage_base + (size_t)st * 3 * W;
+        const T* su = reinterpret_cast<const T*>(stage_base + (size_t)st * 3 * W);     // u | v | grad_out (fp32)
+        const float* sg_row = reinterpret_cast<const float*>(su + 2 * W);
         float4* recs = rec_base + (size_t)rs * W;
         const float sp = __ldg(P.sin_lat + y), cp = __ldg(P.cos_lat + y);
         const int hx = __ldg(S.hx_tab + y);
@@ -530,9 +533,9 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
 #pragma unroll
           for (int j = 0; j < kStepSub; ++j) {
             const int x = min(xb + 32 * j + lane, W - 1);   // lanes past the row end redo its last point (not stored)
-            uu[j] = su[x];
-            vv[j] = su[W + x];
-            gg[j] = pole_row ? gpole : su[2 * W + x];       // adjoint of the output pole mean (advection.py:169)
+            uu[j] = ld_f(su + x);
+            vv[j] = ld_f(su + W + x);
+            gg[j] = pole_row ? gpole : sg_row[x];           // adjoint of the output pole mean (advection.py:169)
             ll[j] = __ldg(P.lon + x);
           }
           const bool last_step = next + S.nP >= row_end;     // this warp's last step in this row
@@ -540,8 +543,8 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
           if (last_step && lane == 0) mbar_arrive(&stage_free[st]);
           // one sub-block after the other, results stored at once: the compiler interleaves as far as the register
           // budget allows (the kernel runs 1024 threads per SM at 64 registers)
-          float* gu_row = core ? gu_pl + (long long)(y - S.out0) * W : nullptr;
-          float* gv_row = core ? gv_pl + (long long)(y - S.out0) * W : nullptr;
+          T* gu_row = core ? gu_pl + (long long)(y - S.out0) * W : nullptr;
+          T* gv_row = core ? gv_pl + (long long)(y - S.out0) * W : nullptr;
 #if !defined(PSL_DBG_NOPRODUCE) && !defined(PSL_ROWS_NO_PAIRS)
           if (!EXACT && (kStepSub % 2) == 0) {
 #pragma unroll
@@ -556,11 +559,11 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
                                         make_float2(gg[j], gg[j + 1]), make_float2(ll[j], ll[j + 1]), violated, rec, ou, ov);
                 if (x0 < W) {
                   recs[x0] = rec[0];
-                  if (core) { __stcs(gu_row + x0, ou.x); __stcs(gv_row + x0, ov.x); }
+                  if (core) { stcs_f(gu_row + x0, ou.x); stcs_f(gv_row + x0, ov.x); }
                 }
                 if (x1 < W) {
                   recs[x1] = rec[1];
-                  if (core) { __stcs(gu_row + x1, ou.y); __stcs(gv_row + x1, ov.y); }
+                  if (core) { stcs_f(gu_row + x1, ou.y); stcs_f(gv_row + x1, ov.y); }
                 }
               }
             }
@@ -581,7 +584,7 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
 #endif
               if (x < W) {
                 recs[x] = rec;
-                if (core) { __stcs(gu_row + x, ou); __stcs(gv_row + x, ov); }
+                if (core) { stcs_f(gu_row + x, ou); stcs_f(gv_row + x, ov); }
               }
             }
           }

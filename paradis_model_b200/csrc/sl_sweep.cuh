@@ -107,13 +107,14 @@ __device__ __forceinline__ void resolve_clashes(int key, int tkey, unsigned char
   }
 }
 
-// Warp-uniform state of the row being swept.
+// Warp-uniform state of the row being swept (T: storage type of u, v, grad_u, grad_v).
+template <typename T>
 struct SweepRow {
-  const float* __restrict__ urow;
-  const float* __restrict__ vrow;
+  const T* __restrict__ urow;
+  const T* __restrict__ vrow;
   const float* __restrict__ grow;
-  float* __restrict__ gu_row;      // nullptr when this row's grad_u / grad_v are not produced here
-  float* __restrict__ gv_row;
+  T* __restrict__ gu_row;          // nullptr when this row's grad_u / grad_v are not produced here
+  T* __restrict__ gv_row;
   float sp, cp;
   int y, head, hx;
 };
@@ -128,8 +129,8 @@ template <int NT> struct StepOut {
 
 // Trajectory, contract check, (for own points) grad_u / grad_v, and the stencil weights of one
 // arrival point.  x: column (unwrapped, for the ring index), xw: wrapped column.
-template <bool EXACT, int INTERP, bool CORE, bool PEER, bool SMALL = false>
-__device__ __forceinline__ void sweep_compute(const Params& P, const SweepRow& R, const float* __restrict__ f,
+template <bool EXACT, int INTERP, bool CORE, bool PEER, bool SMALL = false, typename T>
+__device__ __forceinline__ void sweep_compute(const Params& P, const SweepRow<T>& R, const T* __restrict__ f,
                                               int pl, float mean0, float mean1, int ja, int wc, int ring, int pitch,
                                               int rr, int x, int xw, float uu, float vv, float g, float lonp, bool& violated,
                                               StepOut<Stencil<INTERP>::NT>& o, float& ou, float& ov) {
@@ -220,7 +221,7 @@ __device__ __forceinline__ void sweep_scatter(StepOut<NT>& o, float* acc, unsign
   }
 }
 
-template <bool EXACT, int INTERP, bool PEER>
+template <bool EXACT, int INTERP, bool PEER, typename T>
 __global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const SweepPlan S) {
   constexpr int NT = Stencil<INTERP>::NT, OMIN = Stencil<INTERP>::OMIN;
   extern __shared__ __align__(16) float smem[];
@@ -241,12 +242,12 @@ __global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const Sweep
   for (int i = lane; i < cells; i += 32) acc[i] = 0.0f;
   __syncwarp();
 
-  const float* up = plane_ptr_bc(P.u, P.u_sB, b, c, P.uvgN, P.W);
-  const float* vp = plane_ptr_bc(P.v, P.v_sB, b, c, P.uvgN, P.W);
+  const T* up = plane_ptr_bc(as<T>(P.u), P.u_sB, b, c, P.uvgN, P.W);
+  const T* vp = plane_ptr_bc(as<T>(P.v), P.v_sB, b, c, P.uvgN, P.W);
   const float* gp = plane_ptr_bc(P.gout, P.gout_sB, b, c, P.uvgN, P.W);
-  const float* f = plane_ptr_bc(P.field, P.field_sB, b, c, P.fldN, P.W);
-  float* gu_pl = P.gu ? P.gu + (long long)pl * S.outN * P.W : nullptr;
-  float* gv_pl = P.gu ? P.gv + (long long)pl * S.outN * P.W : nullptr;
+  const T* f = plane_ptr_bc(as<T>(P.field), P.field_sB, b, c, P.fldN, P.W);
+  T* gu_pl = P.gu ? as<T>(P.gu) + (long long)pl * S.outN * P.W : nullptr;
+  T* gv_pl = P.gu ? as<T>(P.gv) + (long long)pl * S.outN * P.W : nullptr;
   float* gf_pl = P.gfield + (long long)pl * S.outN * P.W + ja;
   float mean0 = 0.0f, mean1 = 0.0f;
   if (P.pole_fix) { mean0 = __ldg(P.fmean + 2 * pl); mean1 = __ldg(P.fmean + 2 * pl + 1); }
@@ -255,7 +256,7 @@ __global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const Sweep
 
   // destination row i_done(y) = y - rr + OMIN is complete after arrival row y; it sits in slot `head`
   const int y_first = ra - (ring - 1) + rr - OMIN, y_last = rb - 1 + rr - OMIN;
-  SweepRow R;
+  SweepRow<T> R;
   R.head = 0;
   // Warm-up loads ("touches"): while a row is processed, each lane loads one word of a 128-byte line the NEXT
   // row step will need -- u, v, grad_out of the next arrival row and the field row that enters the stencil
@@ -279,15 +280,27 @@ __global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const Sweep
     if (kTouch) {
       const int yn = y + 1;
       if (yn >= arr_lo && yn < arr_hi && yn <= y_last) {
-        const float* q = nullptr;
-        if (pf_arr == 0) q = arr_row<PEER>(P, up, 0, pl, yn);
-        else if (pf_arr == 1) q = arr_row<PEER>(P, vp, 1, pl, yn);
-        else if (pf_arr == 2) q = arr_row<PEER>(P, gp, 2, pl, yn);
-        else {
-          const int yf = yn + rr + NT - 1 + OMIN;   // last stencil row the next arrival row can reach
-          if (!PEER && yf >= P.fld0 && yf < P.fld0 + P.fldN) q = f + (long long)(yf - P.fld0) * W;
+        if constexpr (kIsF32<T>) {
+          const float* q = nullptr;
+          if (pf_arr == 0) q = arr_row<PEER>(P, up, 0, pl, yn);
+          else if (pf_arr == 1) q = arr_row<PEER>(P, vp, 1, pl, yn);
+          else if (pf_arr == 2) q = arr_row<PEER>(P, gp, 2, pl, yn);
+          else {
+            const int yf = yn + rr + NT - 1 + OMIN;   // last stencil row the next arrival row can reach
+            if (!PEER && yf >= P.fld0 && yf < P.fld0 + P.fldN) q = f + (long long)(yf - P.fld0) * W;
+          }
+          if (q) pf_val = __ldg(q + pf_col);
+        } else {                                      // bf16 rows: same words, half the bytes (over-touches u, v, field)
+          const T* q = nullptr;
+          if (pf_arr == 0) q = arr_row<PEER>(P, up, 0, pl, yn);
+          else if (pf_arr == 1) q = arr_row<PEER>(P, vp, 1, pl, yn);
+          else if (pf_arr == 3) {
+            const int yf = yn + rr + NT - 1 + OMIN;
+            if (yf >= P.fld0 && yf < P.fld0 + P.fldN) q = f + (long long)(yf - P.fld0) * W;
+          }
+          if (q) pf_val = ldg_f(q + pf_col);
+          else if (pf_arr == 2) pf_val = __ldg(arr_row<PEER>(P, gp, 2, pl, yn) + pf_col);
         }
-        if (q) pf_val = __ldg(q + pf_col);
       }
     }
     if (y >= arr_lo && y < arr_hi) {
@@ -316,8 +329,8 @@ __global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const Sweep
           }
           if (x < jb) {
             float uu[4], vv[4], gg[4], ll[4], ou[4], ov[4];
-            *reinterpret_cast<float4*>(uu) = __ldg(reinterpret_cast<const float4*>(R.urow + x));
-            *reinterpret_cast<float4*>(vv) = __ldg(reinterpret_cast<const float4*>(R.vrow + x));
+            *reinterpret_cast<float4*>(uu) = ldg4_f(R.urow + x);
+            *reinterpret_cast<float4*>(vv) = ldg4_f(R.vrow + x);
             *reinterpret_cast<float4*>(gg) = __ldg(reinterpret_cast<const float4*>(R.grow + x));
             *reinterpret_cast<float4*>(ll) = __ldg(reinterpret_cast<const float4*>(P.lon + x));
             // one range check for the lane's 8 backtrack angles instead of one per point (-1 % here; the same
@@ -334,8 +347,8 @@ __global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const Sweep
                                                          vv[k], gg[k], ll[k], violated, o[k], ou[k], ov[k]);
             }
             if (R.gu_row) {
-              __stcs(reinterpret_cast<float4*>(R.gu_row + x), *reinterpret_cast<float4*>(ou));
-              __stcs(reinterpret_cast<float4*>(R.gv_row + x), *reinterpret_cast<float4*>(ov));
+              stcs4_f(R.gu_row + x, *reinterpret_cast<float4*>(ou));
+              stcs4_f(R.gv_row + x, *reinterpret_cast<float4*>(ov));
             }
           }
 #pragma unroll
@@ -351,10 +364,10 @@ __global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const Sweep
           const int xa = ja + (ch << 5) + lane;
           if (xa < jb) {
             float ou = 0.0f, ov = 0.0f;
-            sweep_compute<EXACT, INTERP, true, PEER>(P, R, f, pl, mean0, mean1, ja, wc, ring, pitch, rr, xa, xa, __ldg(R.urow + xa),
-                                               __ldg(R.vrow + xa), __ldg(R.grow + xa), __ldg(P.lon + xa), violated, oa, ou,
+            sweep_compute<EXACT, INTERP, true, PEER>(P, R, f, pl, mean0, mean1, ja, wc, ring, pitch, rr, xa, xa, ldg_f(R.urow + xa),
+                                               ldg_f(R.vrow + xa), __ldg(R.grow + xa), __ldg(P.lon + xa), violated, oa, ou,
                                                ov);
-            if (R.gu_row) { __stcs(R.gu_row + xa, ou); __stcs(R.gv_row + xa, ov); }
+            if (R.gu_row) { stcs_f(R.gu_row + xa, ou); stcs_f(R.gv_row + xa, ov); }
           }
           sweep_scatter<NT>(oa, acc, tag, ring, pitch, lane);
         }
@@ -371,8 +384,8 @@ __global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const Sweep
         if (xw < 0) xw += W; else if (xw >= W) xw -= W;
         if (h < 2 * R.hx) {
           float ou, ov;
-          sweep_compute<EXACT, INTERP, false, PEER>(P, R, f, pl, mean0, mean1, ja, wc, ring, pitch, rr, xa, xw, __ldg(R.urow + xw),
-                                              __ldg(R.vrow + xw), __ldg(R.grow + xw), __ldg(P.lon + xw), violated, oa, ou,
+          sweep_compute<EXACT, INTERP, false, PEER>(P, R, f, pl, mean0, mean1, ja, wc, ring, pitch, rr, xa, xw, ldg_f(R.urow + xw),
+                                              ldg_f(R.vrow + xw), __ldg(R.grow + xw), __ldg(P.lon + xw), violated, oa, ou,
                                               ov);
         }
         sweep_scatter<NT>(oa, acc, tag, ring, pitch, lane);

@@ -6,9 +6,17 @@ Ops (namespace ``paradis``)
 
 Each op has a fake (meta) implementation and an autograd formula, so it works under
 ``torch.compile(fullgraph=True)``, non-reentrant activation checkpointing (nothing but
-the inputs is saved; the trajectory is recomputed in backward) and bf16 autocast (inputs
-are cast to fp32, as torch's own autocast policy does for grid_sampler / asin / atan2).
+the inputs is saved; the trajectory is recomputed in backward) and bf16 autocast.
 CUDA only: there is no CPU implementation.
+
+Storage types of sl_advect.  The arithmetic is always fp32 (torch's own autocast policy runs
+grid_sampler / asin / atan2 in fp32) and ``out`` is fp32.  When field, u and v are all bf16 (what
+autocast hands the op: down_projection and velocity_net outputs) on the full mesh, with W % 8 == 0,
+16-byte aligned bases and batch strides in multiples of 8 elements, the kernels read them as bf16 and
+write bf16 gradients (``paradis::sl_advect_backward_bf16``, include/paradis_sl_bf16.h): no fp32 copy is
+made, and the results are bit-identical to the fp32 op on ``.float()`` copies with the gradients cast
+back by ``.to(torch.bfloat16)``.  Any other combination (fp16, mixed dtypes, latitude bands, other
+alignments) is upcast to fp32 and the gradients are cast back to the input dtypes.
 """
 from __future__ import annotations
 
@@ -196,6 +204,24 @@ def _check_inputs(field: Tensor, u: Tensor, v: Tensor, windows: List[int]):
     return B, V, H, W, ownN, arrN
 
 
+def _full_mesh(windows: List[int]) -> bool:
+    H = int(windows[0])
+    return len(windows) == 8 and [int(w) for w in windows[2:8]] == [0, H, 0, H, 0, H]
+
+
+def _bf16_candidate(dtypes, windows: List[int]) -> bool:
+    """What the native bf16 path needs that is known without the data (dtypes, windows, W): safe in traced code."""
+    return (NATIVE_BF16 and all(d == torch.bfloat16 for d in dtypes) and _full_mesh(windows)
+            and int(windows[1]) % 8 == 0)
+
+
+def _bf16_layout_ok(bf: List[Tensor], f32: List[Tensor]) -> bool:
+    """Alignment part of the native bf16 rule: 16-byte bases, batch strides in multiples of 8 (bf16) / 4 (fp32)
+    elements, so that every row starts on 16 bytes (include/paradis_sl_bf16.h)."""
+    return (all(t.data_ptr() % 16 == 0 and t.stride(0) % 8 == 0 for t in bf)
+            and all(t.data_ptr() % 16 == 0 and t.stride(0) % 4 == 0 for t in f32))
+
+
 # --------------------------------------------------------------------------------------
 # sl_advect
 # --------------------------------------------------------------------------------------
@@ -211,18 +237,24 @@ def _sl_advect(field: Tensor, u: Tensor, v: Tensor, tables: Tensor, scalars: Lis
     if tables.device != field.device:
         raise RuntimeError(f"paradis::sl_advect: geometry tables live on {tables.device}, the tensors on {field.device}; "
                            "move the geometry with SLGeometry.to(device)")
-    field = _inner_contig(field.float())
-    u = _inner_contig(u.float())
-    v = _inner_contig(v.float())
+    native = _bf16_candidate((field.dtype, u.dtype, v.dtype), windows)
+    if native:
+        field, u, v = _inner_contig(field), _inner_contig(u), _inner_contig(v)
+        native = _bf16_layout_ok([field, u, v], [])
+    if not native:
+        field = _inner_contig(field.float())
+        u = _inner_contig(u.float())
+        v = _inner_contig(v.float())
     out = torch.empty((B, V, ownN, W), dtype=torch.float32, device=field.device)
     g = _geom_struct(tables, scalars, windows)
     ws_bytes = L.paradis_sl_advect_fwd_workspace(B, V)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=field.device)
+    fwd = L.paradis_sl_advect_fwd_bf16 if native else L.paradis_sl_advect_fwd
     with torch.cuda.device(field.device):
-        rc = L.paradis_sl_advect_fwd(C.byref(g), _ptr(field), _ptr(u), _ptr(v), _ptr(out), B, V,
-                                     field.stride(0), u.stride(0), v.stride(0), dt, interp, int(pole_fix), math,
-                                     _ptr(ws), ws_bytes, _ptr(_status_word(field.device)), _stream(field))
-    _lib.check(rc, "paradis_sl_advect_fwd")
+        rc = fwd(C.byref(g), _ptr(field), _ptr(u), _ptr(v), _ptr(out), B, V,
+                 field.stride(0), u.stride(0), v.stride(0), dt, interp, int(pole_fix), math,
+                 _ptr(ws), ws_bytes, _ptr(_status_word(field.device)), _stream(field))
+    _lib.check(rc, "paradis_sl_advect_fwd_bf16" if native else "paradis_sl_advect_fwd")
     return out
 
 
@@ -232,36 +264,52 @@ def _(field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl):
     return field.new_empty((B, V, windows[3], windows[1]), dtype=torch.float32)
 
 
-@torch.library.custom_op("paradis::sl_advect_backward", mutates_args=(), device_types="cuda")
-def _sl_advect_backward(grad_out: Tensor, field: Tensor, u: Tensor, v: Tensor, tables: Tensor,
-                        scalars: List[float], dt: float, interp: int, pole_fix: bool, math: int,
-                        windows: List[int], cfl: float, need_field: bool,
-                        need_uv: bool) -> Tuple[Tensor, Tensor, Tensor]:
+def _backward_impl(grad_out: Tensor, field: Tensor, u: Tensor, v: Tensor, tables: Tensor, scalars: List[float],
+                   dt: float, interp: int, pole_fix: bool, math: int, windows: List[int], cfl: float,
+                   need_field: bool, need_uv: bool, native: bool, what: str):
+    """Both backward ops.  native: bf16 field / u / v read in place, bf16 gradients (paradis_sl_advect_bwd_bf16);
+    otherwise the inputs are upcast and the gradients are fp32.  Returns (gf, gu, gv, dtype of the gradients)."""
     B, V, H, W, ownN, arrN = _check_inputs(field, u, v, windows)
     L = _lib.lib()
     dev = field.device
     poll_status(dev)
     if tables.device != dev:
-        raise RuntimeError(f"paradis::sl_advect_backward: geometry tables live on {tables.device}, the tensors on {dev}")
-    field = _inner_contig(field.float())
-    u = _inner_contig(u.float())
-    v = _inner_contig(v.float())
+        raise RuntimeError(f"{what}: geometry tables live on {tables.device}, the tensors on {dev}")
     grad_out = _inner_contig(grad_out.float())
+    if native:
+        field, u, v = _inner_contig(field), _inner_contig(u), _inner_contig(v)
+        native = _bf16_layout_ok([field, u, v], [grad_out])
+    if not native:
+        field = _inner_contig(field.float())
+        u = _inner_contig(u.float())
+        v = _inner_contig(v.float())
     if tuple(grad_out.shape) != tuple(u.shape):
-        raise RuntimeError("paradis::sl_advect_backward: grad_out must cover the arrival window like u and v")
-    gf = torch.empty((B, V, ownN, W), dtype=torch.float32, device=dev) if need_field else None
-    gu = torch.empty((B, V, ownN, W), dtype=torch.float32, device=dev) if need_uv else None
-    gv = torch.empty((B, V, ownN, W), dtype=torch.float32, device=dev) if need_uv else None
+        raise RuntimeError(f"{what}: grad_out must cover the arrival window like u and v")
+    gdt = torch.bfloat16 if native else torch.float32
+    gf = torch.empty((B, V, ownN, W), dtype=gdt, device=dev) if need_field else None
+    gu = torch.empty((B, V, ownN, W), dtype=gdt, device=dev) if need_uv else None
+    gv = torch.empty((B, V, ownN, W), dtype=gdt, device=dev) if need_uv else None
     g = _geom_struct(tables, scalars, windows)
-    ws_bytes = L.paradis_sl_advect_bwd_workspace(B, V, arrN, W)
+    ws_bytes = (L.paradis_sl_advect_bwd_bf16_workspace if native else L.paradis_sl_advect_bwd_workspace)(B, V, arrN, W)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    bwd = L.paradis_sl_advect_bwd_bf16 if native else L.paradis_sl_advect_bwd
     with torch.cuda.device(dev):
-        rc = L.paradis_sl_advect_bwd(C.byref(g), _ptr(grad_out), _ptr(field), _ptr(u), _ptr(v), _ptr(gf), _ptr(gu),
-                                     _ptr(gv), B, V, grad_out.stride(0), field.stride(0), u.stride(0), v.stride(0),
-                                     dt, interp, int(pole_fix), math, 3 | (8 if FORCE_ROW_SWEEP else 0), cfl, _ptr(ws),
-                                     ws_bytes, _ptr(_status_word(dev)), _stream(field))
-    _lib.check(rc, "paradis_sl_advect_bwd")
-    none = lambda: torch.empty(0, dtype=torch.float32, device=dev)
+        rc = bwd(C.byref(g), _ptr(grad_out), _ptr(field), _ptr(u), _ptr(v), _ptr(gf), _ptr(gu),
+                 _ptr(gv), B, V, grad_out.stride(0), field.stride(0), u.stride(0), v.stride(0),
+                 dt, interp, int(pole_fix), math, 3 | (8 if FORCE_ROW_SWEEP else 0), cfl, _ptr(ws),
+                 ws_bytes, _ptr(_status_word(dev)), _stream(field))
+    _lib.check(rc, "paradis_sl_advect_bwd_bf16" if native else "paradis_sl_advect_bwd")
+    return gf, gu, gv, gdt
+
+
+@torch.library.custom_op("paradis::sl_advect_backward", mutates_args=(), device_types="cuda")
+def _sl_advect_backward(grad_out: Tensor, field: Tensor, u: Tensor, v: Tensor, tables: Tensor,
+                        scalars: List[float], dt: float, interp: int, pole_fix: bool, math: int,
+                        windows: List[int], cfl: float, need_field: bool,
+                        need_uv: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    gf, gu, gv, _ = _backward_impl(grad_out, field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl,
+                                   need_field, need_uv, False, "paradis::sl_advect_backward")
+    none = lambda: torch.empty(0, dtype=torch.float32, device=field.device)
     return (gf if need_field else none(), gu if need_uv else none(), gv if need_uv else none())
 
 
@@ -271,6 +319,31 @@ def _(grad_out, field, u, v, tables, scalars, dt, interp, pole_fix, math, window
     shape = (B, V, windows[3], windows[1])
     full = lambda: field.new_empty(shape, dtype=torch.float32)
     none = lambda: field.new_empty((0,), dtype=torch.float32)
+    return (full() if need_field else none(), full() if need_uv else none(), full() if need_uv else none())
+
+
+@torch.library.custom_op("paradis::sl_advect_backward_bf16", mutates_args=(), device_types="cuda")
+def _sl_advect_backward_bf16(grad_out: Tensor, field: Tensor, u: Tensor, v: Tensor, tables: Tensor,
+                             scalars: List[float], dt: float, interp: int, pole_fix: bool, math: int,
+                             windows: List[int], cfl: float, need_field: bool,
+                             need_uv: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """Backward of sl_advect for bf16 field / u / v: bf16 gradients.  Read in place by the bf16 kernels when the
+    layout allows it (see the module docstring), otherwise computed from fp32 copies and rounded by .to()."""
+    native = _bf16_candidate((field.dtype, u.dtype, v.dtype), windows)
+    gf, gu, gv, gdt = _backward_impl(grad_out, field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl,
+                                     need_field, need_uv, native, "paradis::sl_advect_backward_bf16")
+    if gdt != torch.bfloat16:
+        gf, gu, gv = [t.to(torch.bfloat16) if t is not None else None for t in (gf, gu, gv)]
+    none = lambda: torch.empty(0, dtype=torch.bfloat16, device=field.device)
+    return (gf if need_field else none(), gu if need_uv else none(), gv if need_uv else none())
+
+
+@_sl_advect_backward_bf16.register_fake
+def _(grad_out, field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl, need_field, need_uv):
+    B, V = field.shape[:2]
+    shape = (B, V, windows[3], windows[1])
+    full = lambda: field.new_empty(shape, dtype=torch.bfloat16)
+    none = lambda: field.new_empty((0,), dtype=torch.bfloat16)
     return (full() if need_field else none(), full() if need_uv else none(), full() if need_uv else none())
 
 
@@ -289,8 +362,11 @@ def _sl_backward(ctx, grad_out):
                            "use paradis_model_b200.halo.LatBandAdvection")
     need_field = ctx.needs_input_grad[0]
     need_uv = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
-    gf, gu, gv = torch.ops.paradis.sl_advect_backward(grad_out, field, u, v, tables, scalars, dt, interp,
-                                                      pole_fix, math, windows, cfl, need_field, need_uv)
+    # bf16 inputs on the full mesh: bf16 gradients straight from the kernels (no fp32 copies, no casts)
+    bwd = (torch.ops.paradis.sl_advect_backward_bf16 if _bf16_candidate(ctx.dtypes, windows)
+           else torch.ops.paradis.sl_advect_backward)
+    gf, gu, gv = bwd(grad_out, field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl, need_field,
+                     need_uv)
     gf = gf.to(ctx.dtypes[0]) if need_field else None
     gu = gu.to(ctx.dtypes[1]) if ctx.needs_input_grad[1] else None
     gv = gv.to(ctx.dtypes[2]) if ctx.needs_input_grad[2] else None
@@ -302,6 +378,8 @@ _sl_advect.register_autograd(_sl_backward, setup_context=_sl_setup)
 
 DEFAULT_CFL_CELLS = 8.0
 FORCE_ROW_SWEEP = False     # tests: run the row-sweep backward also where the strip sweep is the default (PARADIS_BWD_ROWSWEEP)
+NATIVE_BF16 = True          # bf16 field / u / v read and bf16 gradients written by the kernels where eligible (read at
+                            # call time; False runs the upcast path, for tests and timings of the two in one process)
 # read once at import (not inside traced code): PARADIS_SL_MATH=fast|exact overrides the math mode,
 # PARADIS_SL_CHECK=1 synchronises after every call and raises on a device-side contract violation
 _ENV_MATH = os.environ.get("PARADIS_SL_MATH", "")
