@@ -1,5 +1,5 @@
 """ctypes binding of the C ABI declared in include/paradis_sl.h (and the bf16 entry points of
-include/paradis_sl_bf16.h, in a table of their own).
+include/paradis_sl_bf16.h and include/paradis_geocyclic.h, each in a table of its own).
 
 The product has no CPU fallback: if the shared library is missing this module
 raises, it never substitutes another implementation.
@@ -74,6 +74,22 @@ _PROTOS_BF16 = {
 }
 
 
+# include/paradis_geocyclic.h: bf16 storage of the padding / depthwise-convolution / downsampling ops and the
+# avgpool5 adjoint (same ABI version: entry points added)
+_PROTOS_GEO = {
+    "paradis_geocyclic_pad_fwd_bf16": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.c_int, C.c_int, _P]),
+    "paradis_geocyclic_pad_bwd_bf16": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.c_int, C.c_int, _P]),
+    "paradis_geocyclic_dwconv_fwd_bf16": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
+    "paradis_geocyclic_dwconv_bwd_input_bf16": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                          _P]),
+    "paradis_geocyclic_dwconv_bwd_weight_bf16": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int,
+                                                           C.c_int, _P, C.c_size_t, _P]),
+    "paradis_geocyclic_avgpool5_fwd_bf16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
+    "paradis_geocyclic_avgpool5_bwd": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
+    "paradis_geocyclic_avgpool5_bwd_bf16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
+}
+
+
 def exported_symbols():
     """The functions of include/paradis_sl.h."""
     return list(_PROTOS)
@@ -82,6 +98,11 @@ def exported_symbols():
 def exported_symbols_bf16():
     """The functions of include/paradis_sl_bf16.h."""
     return list(_PROTOS_BF16)
+
+
+def exported_symbols_geocyclic():
+    """The functions of include/paradis_geocyclic.h."""
+    return list(_PROTOS_GEO)
 
 
 def lib():
@@ -110,7 +131,7 @@ def lib():
             except Exception:
                 pass
         handle = C.CDLL(path)
-        for name, (res, args) in list(_PROTOS.items()) + list(_PROTOS_BF16.items()):
+        for name, (res, args) in list(_PROTOS.items()) + list(_PROTOS_BF16.items()) + list(_PROTOS_GEO.items()):
             fn = getattr(handle, name)
             fn.restype, fn.argtypes = res, args
         if handle.paradis_sl_abi_version() != 2 and not os.environ.get("PARADIS_SL_SKIP_ABI_CHECK"):

@@ -14,7 +14,8 @@ HEADERS = [os.path.join(_HERE, "csrc", "sl_device.cuh"), os.path.join(_HERE, "cs
            os.path.join(_HERE, "csrc", "sl_partition.cuh"),
            os.path.join(_HERE, "csrc", "sl_rows.cuh"),
            os.path.join(_HERE, "..", "include", "paradis_sl.h"),
-           os.path.join(_HERE, "..", "include", "paradis_sl_bf16.h")]
+           os.path.join(_HERE, "..", "include", "paradis_sl_bf16.h"),
+           os.path.join(_HERE, "..", "include", "paradis_geocyclic.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
 

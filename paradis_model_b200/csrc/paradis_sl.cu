@@ -24,6 +24,7 @@
 
 #include "../../include/paradis_sl.h"
 #include "../../include/paradis_sl_bf16.h"
+#include "../../include/paradis_geocyclic.h"
 #include "sl_device.cuh"
 
 using namespace psl;
@@ -565,29 +566,44 @@ __global__ void __launch_bounds__(kGatherWarps * 32) sl_bwd_gather_kernel(const 
 // ---------------------------------------------------------------------------------------------
 // standalone GeoCyclic padding (model/padding.py:11-39) and its adjoint
 // ---------------------------------------------------------------------------------------------
-__global__ void geocyclic_pad_fwd_kernel(const float* __restrict__ x, float* __restrict__ y, int H, int W, int p) {
+// T = storage type of x / y (fp32 or bf16).  The bf16 forward copies the 2-byte words as they are, two padded columns
+// per thread and one 4-byte store (Wp and every row start are even).
+template <typename T>
+__global__ void geocyclic_pad_fwd_kernel(const T* __restrict__ x, T* __restrict__ y, int H, int W, int p) {
   const int Hp = H + 2 * p, Wp = W + 2 * p;
   const long long pl = blockIdx.z;
   const int R = blockIdx.y;
   int i = R - p, shift = 0;
   if (i < 0) { i = -i; shift = W / 2; }
   else if (i >= H) { i = 2 * (H - 1) - i; shift = W / 2; }
-  const float* src = x + (pl * H + i) * W;
-  float* dst = y + (pl * Hp + R) * Wp;
-  for (int C = blockIdx.x * blockDim.x + threadIdx.x; C < Wp; C += gridDim.x * blockDim.x) {
-    int j = C - p - shift;
-    if (j < 0) j += W; else if (j >= W) j -= W;
-    dst[C] = __ldg(src + j);
+  const T* src = x + (pl * H + i) * W;
+  T* dst = y + (pl * Hp + R) * Wp;
+  if constexpr (kIsF32<T>) {
+    for (int C = blockIdx.x * blockDim.x + threadIdx.x; C < Wp; C += gridDim.x * blockDim.x) {
+      int j = C - p - shift;
+      if (j < 0) j += W; else if (j >= W) j -= W;
+      dst[C] = __ldg(src + j);
+    }
+  } else {
+    const unsigned short* s16 = reinterpret_cast<const unsigned short*>(src);
+    for (int C = 2 * (blockIdx.x * blockDim.x + threadIdx.x); C < Wp; C += 2 * gridDim.x * blockDim.x) {
+      int j = C - p - shift;
+      if (j < 0) j += W; else if (j >= W) j -= W;
+      const int j1 = j + 1 == W ? 0 : j + 1;
+      *reinterpret_cast<unsigned*>(dst + C) = (unsigned)__ldg(s16 + j) | ((unsigned)__ldg(s16 + j1) << 16);
+    }
   }
 }
 
 // gx[i, j] = sum of every padded cell whose source is (i, j); fixed order: interior row first,
-// then north cap, then south cap; within a row: centre, left wrap, right wrap.
-__global__ void geocyclic_pad_bwd_kernel(const float* __restrict__ gy, float* __restrict__ gx, int H, int W, int p) {
+// then north cap, then south cap; within a row: centre, left wrap, right wrap.  fp32 sums for either storage type,
+// one rounding per bf16 output.
+template <typename T>
+__global__ void geocyclic_pad_bwd_kernel(const T* __restrict__ gy, T* __restrict__ gx, int H, int W, int p) {
   const int Hp = H + 2 * p, Wp = W + 2 * p;
   const long long pl = blockIdx.z;
   const int i = blockIdx.y;
-  const float* g = gy + pl * (long long)Hp * Wp;
+  const T* g = gy + pl * (long long)Hp * Wp;
   for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < W; j += gridDim.x * blockDim.x) {
     float s = 0.0f;
     for (int src = 0; src < 3; ++src) {
@@ -597,12 +613,12 @@ __global__ void geocyclic_pad_bwd_kernel(const float* __restrict__ gy, float* __
       else { const int ii = 2 * (H - 1) - i; if (ii < H || ii >= H + p) continue; R = ii + p; shift = W / 2; }
       // padded columns C with (C - p - shift) mod W == j
       int c = j + shift; if (c >= W) c -= W;   // C - p in [0, W)
-      const float* row = g + (long long)R * Wp + p;
-      s += row[c];
-      if (c >= W - p) s += row[c - W];         // left wrap columns  C - p in [-p, 0)
-      if (c < p) s += row[c + W];              // right wrap columns C - p in [W, W + p)
+      const T* row = g + (long long)R * Wp + p;
+      s += ld_f(row + c);
+      if (c >= W - p) s += ld_f(row + (c - W));  // left wrap columns  C - p in [-p, 0)
+      if (c < p) s += ld_f(row + (c + W));     // right wrap columns C - p in [W, W + p)
     }
-    gx[(pl * H + i) * W + j] = s;
+    st_f(gx + (pl * H + i) * W + j, s);
   }
 }
 
@@ -1358,19 +1374,39 @@ extern "C" int paradis_halo_pack(const float* const* src, const int64_t* src_sB,
   return e == cudaSuccess ? PARADIS_OK : fail(PARADIS_ERR_CUDA, "halo_pack: %s", cudaGetErrorString(e));
 }
 
-extern "C" int paradis_geocyclic_pad_fwd(const float* x, float* y, int64_t planes, int H, int W, int p, void* stream) {
+template <typename T>
+static int pad_fwd(const T* x, T* y, int64_t planes, int H, int W, int p, void* stream, const char* what) {
   if (int rc = pad_check(x, y, planes, H, W, p)) return rc;
-  const int Wp = W + 2 * p;
-  dim3 grid((Wp + 255) / 256, H + 2 * p, (unsigned)planes);
-  geocyclic_pad_fwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x, y, H, W, p);
-  return check_launch("paradis_geocyclic_pad_fwd");
+  const int Wp = W + 2 * p, per_thread = kIsF32<T> ? 1 : 2;
+  dim3 grid((Wp / per_thread + 255) / 256, H + 2 * p, (unsigned)planes);
+  geocyclic_pad_fwd_kernel<T><<<grid, 256, 0, (cudaStream_t)stream>>>(x, y, H, W, p);
+  return check_launch(what);
+}
+
+template <typename T>
+static int pad_bwd(const T* gy, T* gx, int64_t planes, int H, int W, int p, void* stream, const char* what) {
+  if (int rc = pad_check(gy, gx, planes, H, W, p)) return rc;
+  dim3 grid((W + 255) / 256, H, (unsigned)planes);
+  geocyclic_pad_bwd_kernel<T><<<grid, 256, 0, (cudaStream_t)stream>>>(gy, gx, H, W, p);
+  return check_launch(what);
+}
+
+extern "C" int paradis_geocyclic_pad_fwd(const float* x, float* y, int64_t planes, int H, int W, int p, void* stream) {
+  return pad_fwd(x, y, planes, H, W, p, stream, "paradis_geocyclic_pad_fwd");
 }
 
 extern "C" int paradis_geocyclic_pad_bwd(const float* gy, float* gx, int64_t planes, int H, int W, int p, void* stream) {
-  if (int rc = pad_check(gy, gx, planes, H, W, p)) return rc;
-  dim3 grid((W + 255) / 256, H, (unsigned)planes);
-  geocyclic_pad_bwd_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(gy, gx, H, W, p);
-  return check_launch("paradis_geocyclic_pad_bwd");
+  return pad_bwd(gy, gx, planes, H, W, p, stream, "paradis_geocyclic_pad_bwd");
+}
+
+// bf16 storage (include/paradis_geocyclic.h); the forward writes its output in 4-byte words
+extern "C" int paradis_geocyclic_pad_fwd_bf16(const void* x, void* y, int64_t planes, int H, int W, int p, void* stream) {
+  if (x && y && (uintptr_t)y % 4) return fail(PARADIS_ERR_BAD_SHAPE, "geocyclic_pad bf16: output must be 4-byte aligned");
+  return pad_fwd((const bf16*)x, (bf16*)y, planes, H, W, p, stream, "paradis_geocyclic_pad_fwd_bf16");
+}
+
+extern "C" int paradis_geocyclic_pad_bwd_bf16(const void* gy, void* gx, int64_t planes, int H, int W, int p, void* stream) {
+  return pad_bwd((const bf16*)gy, (bf16*)gx, planes, H, W, p, stream, "paradis_geocyclic_pad_bwd_bf16");
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -3,6 +3,8 @@
 Ops (namespace ``paradis``)
     sl_advect / sl_advect_backward      model/advection.py:129-169, fused
     geocyclic_pad / geocyclic_pad_backward   model/padding.py:11-39
+    geocyclic_dwconv / geocyclic_dwconv_backward(_bf16)   SepConv's pad + depthwise conv, model/blocks.py:112-114
+    geocyclic_avgpool5 / geocyclic_avgpool5_backward      PhysicalDownsample, model/blocks.py:57-71
 
 Each op has a fake (meta) implementation and an autograd formula, so it works under
 ``torch.compile(fullgraph=True)``, non-reentrant activation checkpointing (nothing but
@@ -17,6 +19,13 @@ write bf16 gradients (``paradis::sl_advect_backward_bf16``, include/paradis_sl_b
 made, and the results are bit-identical to the fp32 op on ``.float()`` copies with the gradients cast
 back by ``.to(torch.bfloat16)``.  Any other combination (fp16, mixed dtypes, latitude bands, other
 alignments) is upcast to fp32 and the gradients are cast back to the input dtypes.
+
+Storage types of geocyclic_pad, geocyclic_dwconv and geocyclic_avgpool5.  When the large tensors are bf16 (the input,
+and grad_y in backward), the kernels read and write bf16 (include/paradis_geocyclic.h); weight and bias stay fp32 (a
+bf16 weight of C * k * k elements is upcast) and so do grad weight / grad bias.  The results are bit-identical to the
+fp32 kernels run on ``.float()`` copies with the outputs cast back by ``.to(torch.bfloat16)``.  fp16, fp32 and
+mixed-dtype calls take the fp32 kernels (on fp32 copies where needed).  ``NATIVE_BF16 = False`` forces the upcast path
+for these ops as well.
 """
 from __future__ import annotations
 
@@ -215,6 +224,12 @@ def _bf16_candidate(dtypes, windows: List[int]) -> bool:
             and int(windows[1]) % 8 == 0)
 
 
+def _geo_bf16(*tensors: Tensor) -> bool:
+    """Native bf16 storage of the GeoCyclic ops: every large tensor is bf16.  Decided from dtypes only (call time, safe
+    in traced code)."""
+    return NATIVE_BF16 and all(t.dtype == torch.bfloat16 for t in tensors)
+
+
 def _bf16_layout_ok(bf: List[Tensor], f32: List[Tensor]) -> bool:
     """Alignment part of the native bf16 rule: 16-byte bases, batch strides in multiples of 8 (bf16) / 4 (fp32)
     elements, so that every row starts on 16 bytes (include/paradis_sl_bf16.h)."""
@@ -378,8 +393,9 @@ _sl_advect.register_autograd(_sl_backward, setup_context=_sl_setup)
 
 DEFAULT_CFL_CELLS = 8.0
 FORCE_ROW_SWEEP = False     # tests: run the row-sweep backward also where the strip sweep is the default (PARADIS_BWD_ROWSWEEP)
-NATIVE_BF16 = True          # bf16 field / u / v read and bf16 gradients written by the kernels where eligible (read at
-                            # call time; False runs the upcast path, for tests and timings of the two in one process)
+NATIVE_BF16 = True          # bf16 field / u / v read and bf16 gradients written by the kernels where eligible, and bf16
+                            # storage in the geocyclic pad / dwconv / avgpool5 kernels (read at call time; False runs
+                            # the upcast path, for tests and timings of the two in one process)
 # read once at import (not inside traced code): PARADIS_SL_MATH=fast|exact overrides the math mode,
 # PARADIS_SL_CHECK=1 synchronises after every call and raises on a device-side contract violation
 _ENV_MATH = os.environ.get("PARADIS_SL_MATH", "")
@@ -416,11 +432,13 @@ def _geocyclic_pad(x: Tensor, p: int) -> Tensor:
     if not x.is_cuda:
         raise RuntimeError("paradis::geocyclic_pad is a CUDA-only operator (no CPU fallback)")
     B, Cn, H, W = x.shape
-    xf = x.float().contiguous()
-    y = torch.empty((B, Cn, H + 2 * p, W + 2 * p), dtype=torch.float32, device=x.device)
+    native = _geo_bf16(x)
+    xs = x.contiguous() if native else x.float().contiguous()
+    y = torch.empty((B, Cn, H + 2 * p, W + 2 * p), dtype=xs.dtype, device=x.device)
+    name = "paradis_geocyclic_pad_fwd_bf16" if native else "paradis_geocyclic_pad_fwd"
     with torch.cuda.device(x.device):
-        rc = _lib.lib().paradis_geocyclic_pad_fwd(_ptr(xf), _ptr(y), B * Cn, H, W, p, _stream(x))
-    _lib.check(rc, "paradis_geocyclic_pad_fwd")
+        rc = getattr(_lib.lib(), name)(_ptr(xs), _ptr(y), B * Cn, H, W, p, _stream(x))
+    _lib.check(rc, name)
     return y.to(x.dtype)
 
 
@@ -434,11 +452,13 @@ def _(x, p):
 def _geocyclic_pad_backward(gy: Tensor, p: int) -> Tensor:
     B, Cn, Hp, Wp = gy.shape
     H, W = Hp - 2 * p, Wp - 2 * p
-    gyf = gy.float().contiguous()
-    gx = torch.empty((B, Cn, H, W), dtype=torch.float32, device=gy.device)
+    native = _geo_bf16(gy)
+    gs = gy.contiguous() if native else gy.float().contiguous()
+    gx = torch.empty((B, Cn, H, W), dtype=gs.dtype, device=gy.device)
+    name = "paradis_geocyclic_pad_bwd_bf16" if native else "paradis_geocyclic_pad_bwd"
     with torch.cuda.device(gy.device):
-        rc = _lib.lib().paradis_geocyclic_pad_bwd(_ptr(gyf), _ptr(gx), B * Cn, H, W, p, _stream(gy))
-    _lib.check(rc, "paradis_geocyclic_pad_bwd")
+        rc = getattr(_lib.lib(), name)(_ptr(gs), _ptr(gx), B * Cn, H, W, p, _stream(gy))
+    _lib.check(rc, name)
     return gx.to(gy.dtype)
 
 
@@ -477,12 +497,15 @@ def _geocyclic_dwconv(x: Tensor, weight: Tensor, bias: Optional[Tensor]) -> Tens
     k = weight.shape[-1]
     if tuple(weight.shape) != (Cn, 1, k, k):
         raise RuntimeError("paradis::geocyclic_dwconv expects a depthwise weight [C, 1, k, k]")
-    xf, wf = x.float().contiguous(), weight.float().contiguous()
+    native = _geo_bf16(x)
+    xs = x.contiguous() if native else x.float().contiguous()
+    wf = weight.float().contiguous()
     bf = bias.float().contiguous() if bias is not None else None
-    y = torch.empty_like(xf)
+    y = torch.empty_like(xs)
+    name = "paradis_geocyclic_dwconv_fwd_bf16" if native else "paradis_geocyclic_dwconv_fwd"
     with torch.cuda.device(x.device):
-        rc = _lib.lib().paradis_geocyclic_dwconv_fwd(_ptr(xf), _ptr(wf), _ptr(bf), _ptr(y), B, Cn, H, W, k, _stream(x))
-    _lib.check(rc, "paradis_geocyclic_dwconv_fwd")
+        rc = getattr(_lib.lib(), name)(_ptr(xs), _ptr(wf), _ptr(bf), _ptr(y), B, Cn, H, W, k, _stream(x))
+    _lib.check(rc, name)
     return y.to(x.dtype)
 
 
@@ -491,32 +514,43 @@ def _(x, weight, bias):
     return torch.empty_like(x)
 
 
-@torch.library.custom_op("paradis::geocyclic_dwconv_backward", mutates_args=(), device_types="cuda")
-def _geocyclic_dwconv_backward(gy: Tensor, x: Tensor, weight: Tensor, need_input: bool, need_weight: bool,
-                               need_bias: bool) -> Tuple[Tensor, Tensor, Tensor]:
-    """Only the requested gradients are computed (a constant filter, e.g. the box of PhysicalDownsample, skips the
-    weight-gradient pass and its workspace)."""
+def _dw_backward_impl(gy: Tensor, x: Tensor, weight: Tensor, need_input: bool, need_weight: bool, need_bias: bool,
+                      native: bool):
+    """Both backward ops.  native: bf16 gy / x read in place and a bf16 grad input; otherwise fp32 copies and an fp32
+    grad input.  grad weight / grad bias are fp32 either way.  Only the requested gradients are computed (a constant
+    filter skips the weight-gradient pass and its workspace)."""
     B, Cn, H, W = x.shape
     k = weight.shape[-1]
     L = _lib.lib()
-    gyf, wf = gy.float().contiguous(), weight.float().contiguous()
+    gs = gy.contiguous() if native else gy.float().contiguous()
+    wf = weight.float().contiguous()
+    sfx = "_bf16" if native else ""
     empty = lambda: torch.empty(0, dtype=torch.float32, device=x.device)
     gx, gw, gb = empty(), empty(), empty()
     with torch.cuda.device(x.device):
         if need_input:
-            gx = torch.empty((B, Cn, H, W), dtype=torch.float32, device=x.device)
-            rc = L.paradis_geocyclic_dwconv_bwd_input(_ptr(gyf), _ptr(wf), _ptr(gx), B, Cn, H, W, k, _stream(x))
-            _lib.check(rc, "paradis_geocyclic_dwconv_bwd_input")
+            gx = torch.empty((B, Cn, H, W), dtype=gs.dtype, device=x.device)
+            name = "paradis_geocyclic_dwconv_bwd_input" + sfx
+            rc = getattr(L, name)(_ptr(gs), _ptr(wf), _ptr(gx), B, Cn, H, W, k, _stream(x))
+            _lib.check(rc, name)
         if need_weight or need_bias:
-            xf = x.float().contiguous()
+            xs = x.contiguous() if native else x.float().contiguous()
             gw = torch.empty_like(wf)
             gb = torch.empty(Cn if need_bias else 0, dtype=torch.float32, device=x.device)
             ws_bytes = L.paradis_geocyclic_dwconv_wgrad_workspace(B, Cn, H, W, k)
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
-            rc = L.paradis_geocyclic_dwconv_bwd_weight(_ptr(xf), _ptr(gyf), _ptr(gw), _ptr(gb) if need_bias else _ptr(None),
-                                                       B, Cn, H, W, k, _ptr(ws), ws_bytes, _stream(x))
-            _lib.check(rc, "paradis_geocyclic_dwconv_bwd_weight")
+            name = "paradis_geocyclic_dwconv_bwd_weight" + sfx
+            rc = getattr(L, name)(_ptr(xs), _ptr(gs), _ptr(gw), _ptr(gb) if need_bias else _ptr(None),
+                                  B, Cn, H, W, k, _ptr(ws), ws_bytes, _stream(x))
+            _lib.check(rc, name)
     return gx, gw, gb
+
+
+@torch.library.custom_op("paradis::geocyclic_dwconv_backward", mutates_args=(), device_types="cuda")
+def _geocyclic_dwconv_backward(gy: Tensor, x: Tensor, weight: Tensor, need_input: bool, need_weight: bool,
+                               need_bias: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """fp32 gradients from fp32 copies of gy and x."""
+    return _dw_backward_impl(gy, x, weight, need_input, need_weight, need_bias, False)
 
 
 @_geocyclic_dwconv_backward.register_fake
@@ -525,6 +559,25 @@ def _(gy, x, weight, need_input, need_weight, need_bias):
     return (torch.empty_like(x, dtype=torch.float32) if need_input else none(),
             torch.empty_like(weight, dtype=torch.float32) if (need_weight or need_bias) else none(),
             x.new_empty((x.shape[1],), dtype=torch.float32) if need_bias else none())
+
+
+@torch.library.custom_op("paradis::geocyclic_dwconv_backward_bf16", mutates_args=(), device_types="cuda")
+def _geocyclic_dwconv_backward_bf16(gy: Tensor, x: Tensor, weight: Tensor, need_input: bool, need_weight: bool,
+                                    need_bias: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """Backward for a bf16 x: bf16 grad input, fp32 grad weight / grad bias.  gy and x are read in place by the bf16
+    kernels when both are bf16, otherwise the grad input is computed from fp32 copies and rounded by .to()."""
+    native = _geo_bf16(gy, x)
+    gx, gw, gb = _dw_backward_impl(gy, x, weight, need_input, need_weight, need_bias, native)
+    gx = gx.to(torch.bfloat16) if need_input else torch.empty(0, dtype=torch.bfloat16, device=x.device)
+    return gx, gw, gb
+
+
+@_geocyclic_dwconv_backward_bf16.register_fake
+def _(gy, x, weight, need_input, need_weight, need_bias):
+    none = lambda dt: x.new_empty((0,), dtype=dt)
+    return (torch.empty_like(x, dtype=torch.bfloat16) if need_input else none(torch.bfloat16),
+            torch.empty_like(weight, dtype=torch.float32) if (need_weight or need_bias) else none(torch.float32),
+            x.new_empty((x.shape[1],), dtype=torch.float32) if need_bias else none(torch.float32))
 
 
 def _dw_setup(ctx, inputs, output):
@@ -540,7 +593,10 @@ def _dw_backward(ctx, gy):
     need_b = ctx.has_bias and ctx.needs_input_grad[2]
     if not (need_x or need_w or need_b):
         return None, None, None
-    gx, gw, gb = torch.ops.paradis.geocyclic_dwconv_backward(gy, x, weight, need_x, need_w, need_b)
+    # bf16 x and grad_y: bf16 grad input straight from the kernels (no fp32 copies, no casts)
+    bwd = (torch.ops.paradis.geocyclic_dwconv_backward_bf16 if _geo_bf16(gy) and ctx.dtypes[0] == torch.bfloat16
+           else torch.ops.paradis.geocyclic_dwconv_backward)
+    gx, gw, gb = bwd(gy, x, weight, need_x, need_w, need_b)
     return (gx.to(ctx.dtypes[0]) if need_x else None, gw.to(ctx.dtypes[1]) if need_w else None,
             gb.to(ctx.dtypes[2]) if need_b else None)
 
@@ -554,11 +610,13 @@ _geocyclic_dwconv.register_autograd(_dw_backward, setup_context=_dw_setup)
 @torch.library.custom_op("paradis::geocyclic_avgpool5", mutates_args=(), device_types="cuda")
 def _geocyclic_avgpool5(x: Tensor, stride: int) -> Tensor:
     B, Cn, H, W = x.shape
-    xf = x.float().contiguous()
-    y = torch.empty((B, Cn, (H - 1) // stride + 1, (W - 1) // stride + 1), dtype=torch.float32, device=x.device)
+    native = _geo_bf16(x)
+    xs = x.contiguous() if native else x.float().contiguous()
+    y = torch.empty((B, Cn, (H - 1) // stride + 1, (W - 1) // stride + 1), dtype=xs.dtype, device=x.device)
+    name = "paradis_geocyclic_avgpool5_fwd_bf16" if native else "paradis_geocyclic_avgpool5_fwd"
     with torch.cuda.device(x.device):
-        rc = _lib.lib().paradis_geocyclic_avgpool5_fwd(_ptr(xf), _ptr(y), B, Cn, H, W, stride, _stream(x))
-    _lib.check(rc, "paradis_geocyclic_avgpool5_fwd")
+        rc = getattr(_lib.lib(), name)(_ptr(xs), _ptr(y), B, Cn, H, W, stride, _stream(x))
+    _lib.check(rc, name)
     return y.to(x.dtype)
 
 
@@ -568,20 +626,37 @@ def _(x, stride):
     return x.new_empty((B, Cn, (H - 1) // stride + 1, (W - 1) // stride + 1))
 
 
+@torch.library.custom_op("paradis::geocyclic_avgpool5_backward", mutates_args=(), device_types="cuda")
+def _geocyclic_avgpool5_backward(gy: Tensor, H: int, W: int, stride: int) -> Tensor:
+    """Adjoint of geocyclic_avgpool5 for an [B, C, H, W] input: one kernel that gathers, for every input point, the
+    strided outputs whose 5x5 window covers it.  Returns gy's dtype."""
+    B, Cn, Ho, Wo = gy.shape
+    if (Ho, Wo) != ((H - 1) // stride + 1, (W - 1) // stride + 1):
+        raise RuntimeError(f"paradis::geocyclic_avgpool5_backward: grad_y {tuple(gy.shape)} does not match an "
+                           f"input of {H} x {W} with stride {stride}")
+    native = _geo_bf16(gy)
+    gs = gy.contiguous() if native else gy.float().contiguous()
+    gx = torch.empty((B, Cn, H, W), dtype=gs.dtype, device=gy.device)
+    name = "paradis_geocyclic_avgpool5_bwd_bf16" if native else "paradis_geocyclic_avgpool5_bwd"
+    with torch.cuda.device(gy.device):
+        rc = getattr(_lib.lib(), name)(_ptr(gs), _ptr(gx), B, Cn, H, W, stride, _stream(gy))
+    _lib.check(rc, name)
+    return gx.to(gy.dtype)
+
+
+@_geocyclic_avgpool5_backward.register_fake
+def _(gy, H, W, stride):
+    return gy.new_empty((gy.shape[0], gy.shape[1], H, W))
+
+
 def _pool_setup(ctx, inputs, output):
     x, stride = inputs
     ctx.stride, ctx.shape, ctx.dtype = stride, tuple(x.shape), x.dtype
 
 
 def _pool_backward(ctx, gy):
-    # adjoint = the box filter's input gradient applied to grad_y scattered back onto the full-resolution mesh
     B, Cn, H, W = ctx.shape
-    s = ctx.stride
-    g_full = torch.zeros((B, Cn, H, W), dtype=torch.float32, device=gy.device)
-    g_full[:, :, ::s, ::s] = gy.float()
-    box = torch.full((Cn, 1, 5, 5), 1.0 / 25.0, dtype=torch.float32, device=gy.device)
-    gx, _, _ = torch.ops.paradis.geocyclic_dwconv_backward(g_full, g_full, box, True, False, False)
-    return gx.to(ctx.dtype), None
+    return torch.ops.paradis.geocyclic_avgpool5_backward(gy, H, W, ctx.stride).to(ctx.dtype), None
 
 
 _geocyclic_avgpool5.register_autograd(_pool_backward, setup_context=_pool_setup)
