@@ -258,13 +258,12 @@ def sl_advect_explicit(field, u, v, lat_grid, lon_grid, dt, grad_out=None,
     Forward : out = sum_taps w * field[src(R, C)]                      (SURVEY 8a)
     Backward: grad_u, grad_v through the Jacobian of the rotated-pole map,
               grad_field by the adjoint scatter through the GeoCyclic map.
-    Works in the dtype of the inputs (use fp64 for formula checks).
+    The departure coordinates are computed in the dtype of the inputs (use fp64 for formula
+    checks); the interpolation and its adjoint are :func:`sl_advect_at_coords` at them.
     """
-    B, V, H, W = field.shape
+    H, W = field.shape[-2:]
     p = INTERP_PAD[interpolation]
-    Hp, Wp = H + 2 * p, W + 2 * p
     geo = Geometry(lat_grid, lon_grid)
-    src = pole_mean(field) if pole_fix else field
 
     lon_r, lat_r = -u * dt, -v * dt
     sa, ca = torch.sin(lat_r), torch.cos(lat_r)          # phi'
@@ -281,57 +280,398 @@ def sl_advect_explicit(field, u, v, lat_grid, lon_grid, dt, grad_out=None,
     Ay = (geo.Hf - 1.0) / geo.d_lat
     ix = (lon_dep - geo.min_lon) * Ax + p
     iy = (lat_dep - geo.min_lat) * Ay + p
+    coords = torch.stack(torch.broadcast_tensors(ix, iy, sa, ca, sb, cb, s, num, den, lat_dep, lon_dep), dim=2)
+
+    r = sl_advect_at_coords(field, grad_out, coords, sp[0, 0, :, 0], cp[0, 0, :, 0], dt, geo, interpolation,
+                            pole_fix)
+    if grad_out is None:
+        return r.out.to(field.dtype)
+    return tuple(t.to(field.dtype) for t in (r.out, r.grad_field, r.grad_u, r.grad_v))
+
+
+# --------------------------------------------------------------------------
+# fp64 reference at given departure coordinates, with per-point rounding bounds
+# --------------------------------------------------------------------------
+U32 = 2.0 ** -24          # unit roundoff of fp32
+U_BF16 = 2.0 ** -8        # unit roundoff of bf16 (8-bit significand): |bf16(x) - x| <= 2^-8 |x|
+K_OUT = 8                 # roundings per forward term, see sl_advect_at_coords
+K_GFIELD = 4              # roundings per grad_field contribution before the sum
+K_GRAD_UV = 24            # roundings along the longest chain of grad_u / grad_v
+
+
+class AtCoords:
+    """Result of :func:`sl_advect_at_coords`: fp64 values and per-point bounds of |kernel - value|."""
+
+    def __init__(self, **kw):
+        self.__dict__.update(kw)
+
+    def values(self):
+        return self.out, self.grad_field, self.grad_u, self.grad_v
+
+    def bounds(self):
+        return self.out_bound, self.grad_field_bound, self.grad_u_bound, self.grad_v_bound
+
+
+def pixel_scales(geometry, dt):
+    """(Ax, Ay, dt) as the kernels hold them.
+
+    ``geometry`` is either an ``SLGeometry`` (anything with ``scalars`` = [min_lat, d_lat, min_lon, d_lon], ``H``,
+    ``W``): fp32 ``(W - 1) / d_lon``, ``(H - 1) / d_lat`` and fp32 ``dt``, like ``fill_params`` in paradis_sl.cu; or
+    this module's :class:`Geometry`, whose scales are taken in the dtype of its grids (the closed form)."""
+    if hasattr(geometry, "scalars"):
+        _, d_lat, _, d_lon = geometry.scalars
+        f = np.float32
+        return (float(f(f(geometry.W) - f(1)) / f(d_lon)), float(f(f(geometry.H) - f(1)) / f(d_lat)),
+                float(f(dt)))
+    return (float((geometry.Wf - 1.0) / geometry.d_lon), float((geometry.Hf - 1.0) / geometry.d_lat), float(dt))
+
+
+class _RunErr:
+    """First-order running error of an fp32 chain: value (fp64) and error bound in units of U32.
+    Each rounded operation adds |its result|; inputs carry their own bounds (Higham, ASNA 2nd ed., 3.3)."""
+
+    def __init__(self, v, r=0.0):
+        self.v, self.r = v, r
+
+    def neg(self):                  # exact
+        return _RunErr(-self.v, self.r)
+
+    def add(self, o):
+        o = o if isinstance(o, _RunErr) else _RunErr(o)
+        v = self.v + o.v
+        return _RunErr(v, self.r + o.r + abs(v))
+
+    def mul(self, o):
+        o = o if isinstance(o, _RunErr) else _RunErr(o)
+        v = self.v * o.v
+        return _RunErr(v, abs(self.v) * o.r + abs(o.v) * self.r + abs(v))
+
+    def fma(self, o, c):            # self * o + c, one rounding
+        o = o if isinstance(o, _RunErr) else _RunErr(o)
+        c = c if isinstance(c, _RunErr) else _RunErr(c)
+        v = self.v * o.v + c.v
+        return _RunErr(v, abs(self.v) * o.r + abs(o.v) * self.r + c.r + abs(v))
+
+
+class _F32:
+    """The same chains evaluated in fp32, one rounding per operation.  fma: the product of two fp32 values is exact in
+    fp64, so ``a * b + c`` rounds to fp64 and then to fp32 (a double rounding, at most 2^-29 ulp from the fused
+    result)."""
+
+    def __init__(self, v):
+        self.v = v
+
+    @staticmethod
+    def _val(o):
+        return o.v if isinstance(o, _F32) else o
+
+    def neg(self):
+        return _F32(-self.v)
+
+    def add(self, o):
+        return _F32(self.v + self._val(o))
+
+    def mul(self, o):
+        return _F32(self.v * self._val(o))
+
+    def fma(self, o, c):
+        d = lambda x: x.double() if torch.is_tensor(x) else x
+        return _F32((d(self.v) * d(self._val(o)) + d(self._val(c))).float())
+
+
+def _axis_weights(t, interpolation, num):
+    """The kernels' fp32 axis weights and their derivatives at fraction ``t`` (``axis_weights`` in sl_device.cuh, same
+    operation order), with ``num`` = :class:`_RunErr` (running-error bounds) or :class:`_F32` (fp32 values).  The
+    sampler coordinates are >= p - 1/2 > 0, so ``t = ix - floor(ix)`` is exact in fp32.  Bilinear: ``1 - t`` is one
+    rounding, ``t`` is exact.  The cubic weights cancel (w -> 0 at the stencil's edge while the Horner terms stay
+    O(1)), so their error is not relative to the weight: it is carried as an absolute bound instead of a count in K."""
+    T = num(t)
+    if interpolation == "bilinear":
+        return [num(1.0).add(T.neg()), T], [num(-1.0), num(1.0)]
+    A = -0.75
+    t1 = T.add(1.0)
+    u0 = num(1.0).add(T.neg())
+    u1 = u0.add(1.0)
+
+    def outer(x):           # fma(fma(fma(A, x, -5A), x, 8A), x, -4A)
+        return num(A).fma(x, -5 * A).fma(x, 8 * A).fma(x, -4 * A)
+
+    def inner(x):           # fma(fma(A + 2, x, -(A + 3)) * x, x, 1)
+        return num(A + 2).fma(x, -(A + 3)).mul(x).fma(x, 1.0)
+
+    def d_outer(x):         # fma(fma(3A, x, -10A), x, 8A)
+        return num(3 * A).fma(x, -10 * A).fma(x, 8 * A)
+
+    def d_inner(x):         # fma(3(A + 2), x, -2(A + 3)) * x
+        return num(3 * (A + 2)).fma(x, -2 * (A + 3)).mul(x)
+
+    return ([outer(t1), inner(T), inner(u0), outer(u1)],
+            [d_outer(t1), d_inner(T), d_inner(u0).neg(), d_outer(u1).neg()])
+
+
+def _weight_rounding(t, interpolation):
+    """Running-error bounds (units of U32) of the kernels' fp32 axis weights and derivatives (:func:`_axis_weights`)."""
+    w, dw = _axis_weights(t.double(), interpolation, _RunErr)
+    z = torch.zeros_like(t, dtype=torch.float64)
+    return [x.r + z for x in w], [x.r + z for x in dw]
+
+
+def _pole_mean_adjoint(g):
+    gg = g.clone()
+    gg[:, :, 0, :] = g[:, :, 0, :].mean(dim=-1, keepdim=True)
+    gg[:, :, -1, :] = g[:, :, -1, :].mean(dim=-1, keepdim=True)
+    return gg
+
+
+def _pole_mean_sequential(x):
+    """Rows 0 and H-1 replaced by their zonal mean, summed one value after the other in the dtype of ``x`` (the
+    order with the largest error bound) and divided by W."""
+    y = x.clone()
+    for r in (0, x.shape[2] - 1):
+        acc = torch.zeros_like(x[:, :, r, 0])
+        for j in range(x.shape[3]):
+            acc = acc + x[:, :, r, j]
+        y[:, :, r, :] = (acc / x.shape[3])[..., None]
+    return y
+
+
+def _row_mean_at_poles(x, extra):
+    """Rows 0 and H-1 of a bound replaced by their zonal mean plus ``extra`` (same rows)."""
+    y = x.clone()
+    for r in (0, -1):
+        y[:, :, r, :] = (x[:, :, r, :] + extra[:, :, r, :]).mean(dim=-1, keepdim=True)
+    return y
+
+
+def _ordered_scatter(n, idx, val, gen):
+    """fp32 sum of ``val`` into ``n`` cells at ``idx`` (1-D), each cell's terms added one by one in an order drawn
+    from ``gen``: what a kernel with any fixed summation order could do."""
+    perm = torch.randperm(idx.numel(), generator=gen)
+    idx, val = idx[perm], val[perm]
+    order = torch.sort(idx, stable=True).indices
+    idx, val = idx[order], val[order]
+    _, counts = torch.unique_consecutive(idx, return_counts=True)
+    starts = torch.cumsum(counts, 0) - counts
+    rank = torch.arange(idx.numel()) - torch.repeat_interleave(starts, counts)
+    acc = torch.zeros(n, dtype=val.dtype)
+    for k in range(int(rank.max()) + 1 if rank.numel() else 0):
+        sel = rank == k
+        acc[idx[sel]] = acc[idx[sel]] + val[sel]
+    return acc
+
+
+def sl_advect_at_coords(field, grad_out, coords, sin_lat, cos_lat, dt, geometry, interpolation="bilinear",
+                        pole_fix=True, compute_dtype=torch.float64, scatter_order=None):
+    """The operator and its adjoint evaluated AT GIVEN departure coordinates, with a rounding bound per point.
+
+    ``coords`` [B, V, 11, H, W] is what ``ops.departure_coords`` returns (ix, iy, sin lat', cos lat', sin lon',
+    cos lon', s, num, den, lat, lon); ``sin_lat``, ``cos_lat`` [H] are the geometry's fp32 tables (``SLGeometry.tables``)
+    for a kernel check.  ``out`` and ``grad_field`` are linear in ``field`` / ``grad_out`` with weights that are exact
+    functions of (ix, iy), so evaluated in fp64 there is no ``floor()`` ambiguity left: any misrouted, missing or doubled
+    term shows up at its point, whatever its weight.  ``grad_u`` / ``grad_v`` use the kernels' Jacobian formula
+    (``velocity_grads`` in sl_device.cuh) on the fp32 intermediates, evaluated in fp64, except that ``1 - s^2`` is
+    rounded like the kernels and torch's autograd round it, ``fl32(1 - fl32(sc * sc))`` (DESIGN §7), when the
+    coordinates are fp32.  Everything runs on the device of the inputs.
+
+    Bounds (first order in u = 2^-24; fp32 kernel minus the fp64 value, per point, no allowance for outliers):
+
+    * out: ``u * sum_t (K_OUT + m_t) |w_t| |f_t| + u * sum_t |f_t| (|wy| rx + ry |wx|)``.  K_OUT = 8: one rounding
+      forms the tap weight ``wx * wy`` (bilinear forward), or the taps are summed along x and then along y by FMA
+      chains of NT = 4 (bicubic), and a term passes through at most 4 + 4 accumulations.  ``rx``, ``ry`` are the
+      running-error bounds of the fp32 axis weights (:func:`_weight_rounding`): 0 or ``|1 - t|`` for bilinear, the
+      Horner chain's bound for the cancelling cubic weights.  A pole-mean tap (``pole_fix``) stands for an fp32 sum of
+      W values: ``|f_t|`` is the row's mean absolute value and m_t = W (W - 1 additions and one scaling); m_t = 0
+      otherwise.  On the output pole rows the bound is the row mean of the bounds plus ``u W`` times the row mean of
+      ``sum_t |w_t f_t|``.
+    * grad_field: ``u * (K_GFIELD + n_c + m) * sum |w g'|`` over the contributions a cell receives, plus the weights'
+      running errors as above.  K_GFIELD = 4 covers the products ``g * wx * wy`` in any association (2 roundings) with
+      a margin of 2; n_c (a second scatter_add counts them) bounds the rounding of their sum in ANY order; g' is
+      ``grad_out`` after the pole-mean adjoint, and a pole row's g' is a mean (m = W, ``|g'|`` = mean ``|grad_out|``).
+      Pole rows of ``grad_field`` (``pole_fix``) are row means again, as for ``out``.
+    * grad_u, grad_v: ``u * (K_GRAD_UV + m)`` times the same formula with every sum replaced by the sum of absolute
+      values, plus the weights' running errors through it.  K_GRAD_UV = 24: the longest chain is the bicubic
+      derivative sum (4 + 4 accumulations), ``g * dx``, ``* Ax``, ``dlam_da`` (``sa cb``, FMA, product, FMA,
+      ``* inv_r2``, and 3 for ``inv_r2``: FMA, product, approximate reciprocal of <= 1 ulp), the final FMA and ``* -dt``
+      = 19; ``ky`` adds the approximate rsqrt (<= 2 ulp).  m = W when a pole mean enters the point.
+    * bf16 gradients (``|ref| + bound``) times U_BF16 = 2^-8 on top: one round-to-nearest of a value with an 8-bit
+      significand (half an ulp is up to 2^-8 relative, at the bottom of a binade).
+
+    ``compute_dtype`` / ``scatter_order`` (a torch.Generator) run the same computation in fp32 instead: the axis weights
+    by the kernels' fp32 Horner chains, the pole means summed one value after the other, the grad_field sum taken in a
+    random order.  That is the test that the bounds are not too tight.  Bounds are only formed in fp64.
+    """
+    B, V, H, W = field.shape
+    p = INTERP_PAD[interpolation]
+    Hp, Wp = H + 2 * p, W + 2 * p
+    dev = field.device
+    fp64 = compute_dtype == torch.float64
+    cd = compute_dtype
+    Ax, Ay, dt = pixel_scales(geometry, dt)
+    c = coords.to(torch.float64)
+    ix, iy = c[:, :, 0], c[:, :, 1]
+    sa, ca, sb, cb, s, num, den = [c[:, :, k].to(cd) for k in range(2, 9)]
+    sp = sin_lat.to(dev, cd).reshape(1, 1, H, 1)
+    cp = cos_lat.to(dev, cd).reshape(1, 1, H, 1)
+
+    f = field.to(cd)
+    pmean = pole_mean if fp64 else _pole_mean_sequential
+    src = pmean(f) if pole_fix else f
+    fmag = f.abs()
+    if pole_fix:           # a pole tap is an fp32 mean of W values: bound it by the mean absolute value
+        fmag = fmag.clone()
+        fmag[:, :, 0, :] = f[:, :, 0, :].abs().mean(dim=-1, keepdim=True)
+        fmag[:, :, -1, :] = f[:, :, -1, :].abs().mean(dim=-1, keepdim=True)
 
     x0, y0, offs, wx, wy, dwx, dwy = _stencil(ix, iy, interpolation)
+    if not fp64:           # fp32 run: the kernels' fp32 weight chains, fp32 arithmetic from there on
+        (wx, dwx), (wy, dwy) = [[[w.v for w in ws] for ws in _axis_weights((t - torch.floor(t)).float(), interpolation,
+                                                                           _F32)] for t in (ix, iy)]
+    rwx, rdwx = _weight_rounding(ix - torch.floor(ix), interpolation)
+    rwy, rdwy = _weight_rounding(iy - torch.floor(iy), interpolation)
     row_map, col_map = geocyclic_source_index(H, W, p)
-    flat_map = torch.from_numpy(row_map * W + col_map).to(field.device)      # [Hp, Wp]
+    flat_map = torch.from_numpy(row_map * W + col_map).to(dev)      # [Hp, Wp]
     src_flat = src.reshape(B, V, H * W)
+    mag_flat = fmag.reshape(B, V, H * W)
 
-    out = torch.zeros_like(field)
-    dsum_x = torch.zeros_like(field)
-    dsum_y = torch.zeros_like(field)
+    def gather(t, idx):
+        return torch.gather(t, 2, idx.reshape(B, V, -1)).reshape(B, V, H, W)
+
+    zero = torch.zeros(B, V, H, W, dtype=cd, device=dev)
+    out, dsum_x, dsum_y = zero.clone(), zero.clone(), zero.clone()
+    m_out = zero.clone().double()         # sum |w f|
+    b_out = zero.clone().double()         # sum (K + m_t) |w f| + weight rounding, units of u
+    mx, my, ex, ey = [zero.clone().double() for _ in range(4)]   # |.|-sums of dsum_x / dsum_y and weight terms
+    pole_pt = torch.zeros(B, V, H, W, dtype=torch.bool, device=dev)
     taps = []
     for a, oy in enumerate(offs):
+        row, drow = zero.clone(), zero.clone()          # along x first, then along y (the kernels' order)
         for b, ox in enumerate(offs):
             R, C = y0 + oy, x0 + ox
             ok = (R >= 0) & (R < Hp) & (C >= 0) & (C < Wp)          # padding_mode="zeros"
-            idx = flat_map[R.clamp(0, Hp - 1), C.clamp(0, Wp - 1)]   # [B,V,H,W]
-            val = torch.gather(src_flat, 2, idx.reshape(B, V, -1)).reshape(B, V, H, W)
-            val = torch.where(ok, val, torch.zeros_like(val))
-            out = out + wy[a] * wx[b] * val
-            dsum_x = dsum_x + wy[a] * dwx[b] * val
-            dsum_y = dsum_y + dwy[a] * wx[b] * val
-            taps.append((idx, ok, wy[a] * wx[b]))
-    res = pole_mean(out) if pole_fix else out
+            Rc, Cc = R.clamp(0, Hp - 1), C.clamp(0, Wp - 1)
+            idx = flat_map[Rc, Cc]                                   # [B,V,H,W]
+            val = torch.where(ok, gather(src_flat, idx), zero)
+            row = row + wx[b] * val
+            drow = drow + dwx[b] * val
+            taps.append((idx, ok, wy[a] * wx[b], (a, b, Rc, Cc)))
+            if not fp64:
+                continue
+            fm = torch.where(ok, gather(mag_flat, idx), zero)
+            srow = idx // W
+            pole_tap = ok & bool(pole_fix) & ((srow == 0) | (srow == H - 1))
+            pole_pt |= pole_tap
+            awx, awy, adx, ady = wx[b].abs(), wy[a].abs(), dwx[b].abs(), dwy[a].abs()
+            m_out += awy * awx * fm
+            b_out += fm * ((K_OUT + W * pole_tap) * awy * awx + awy * rwx[b] + rwy[a] * awx)
+            mx += awy * adx * fm
+            my += ady * awx * fm
+            ex += fm * (awy * rdwx[b] + rwy[a] * adx)
+            ey += fm * (ady * rwx[b] + rdwy[a] * awx)
+        out = out + wy[a] * row
+        dsum_x = dsum_x + wy[a] * drow
+        dsum_y = dsum_y + dwy[a] * row
+    res = pmean(out) if pole_fix else out
+    if fp64:
+        out_bound = b_out
+        if pole_fix:
+            out_bound = _row_mean_at_poles(b_out, W * m_out)
+        out_bound = out_bound * U32
     if grad_out is None:
-        return res
+        if not fp64:
+            return AtCoords(out=res)
+        return AtCoords(out=res, out_bound=out_bound)
 
-    def pole_mean_adjoint(g):
-        gg = g.clone()
-        gg[:, :, 0, :] = g[:, :, 0, :].mean(dim=-1, keepdim=True)
-        gg[:, :, -1, :] = g[:, :, -1, :].mean(dim=-1, keepdim=True)
-        return gg
-
-    g = pole_mean_adjoint(grad_out) if pole_fix else grad_out
+    g0 = grad_out.to(cd)
+    g = (_pole_mean_adjoint if fp64 else _pole_mean_sequential)(g0) if pole_fix else g0
+    gmag = g0.abs().double()
+    if pole_fix:
+        gmag = _pole_mean_adjoint(gmag)
+        pole_pt[:, :, 0, :] = True
+        pole_pt[:, :, -1, :] = True
     gix, giy = g * dsum_x, g * dsum_y
 
     r2 = num * num + den * den
     dlam_db = (den * ca * cb + num * ca * sb * cp) / r2
     dlam_da = (-den * sa * sb + num * (sa * cb * cp + ca * sp)) / r2
-    inside = ((s >= lo) & (s <= hi)).to(field.dtype)
-    dphi_ds = inside / torch.sqrt(1 - s_c * s_c)
+    lo = torch.tensor(-1 + 1e-7, dtype=coords.dtype).item()
+    hi = torch.tensor(1 - 1e-7, dtype=coords.dtype).item()
+    s_in = coords[:, :, 6]
+    inside = ((s_in >= lo) & (s_in <= hi)).to(cd)
+    sc = torch.clamp(s_in, lo, hi)
+    om = (1 - sc * sc).to(cd)              # rounded in the dtype of the coordinates, like the kernels
+    dphi_ds = inside / torch.sqrt(om)
     ds_db = -ca * sb * sp
     ds_da = ca * cp - sa * cb * sp
     grad_u = -dt * (gix * Ax * dlam_db + giy * Ay * dphi_ds * ds_db)
     grad_v = -dt * (gix * Ax * dlam_da + giy * Ay * dphi_ds * ds_da)
 
-    gsrc = torch.zeros(B, V, H * W, dtype=field.dtype, device=field.device)
-    for idx, ok, w in taps:
-        contrib = torch.where(ok, w * g, torch.zeros_like(g))
-        gsrc.scatter_add_(2, idx.reshape(B, V, -1), contrib.reshape(B, V, -1))
+    gsrc = torch.zeros(B, V, H * W, dtype=cd, device=dev)
+    if scatter_order is not None:
+        all_idx = (torch.cat([idx.reshape(B * V, -1) for idx, *_ in taps], 1)
+                   + (torch.arange(B * V, device=dev) * (H * W))[:, None]).reshape(-1)
+        all_val = torch.cat([torch.where(ok, w * g, torch.zeros_like(g)).reshape(B * V, -1)
+                             for idx, ok, w, _ in taps], 1).reshape(-1)
+        gsrc = _ordered_scatter(B * V * H * W, all_idx.cpu(), all_val.cpu(), scatter_order).to(dev).reshape(
+            B, V, H * W)
+    else:
+        for idx, ok, w, _ in taps:
+            contrib = torch.where(ok, w * g, torch.zeros_like(g))
+            gsrc.scatter_add_(2, idx.reshape(B, V, -1), contrib.reshape(B, V, -1))
     gsrc = gsrc.reshape(B, V, H, W)
-    grad_field = pole_mean_adjoint(gsrc) if pole_fix else gsrc
-    return res, grad_field, grad_u, grad_v
+    grad_field = (_pole_mean_adjoint if fp64 else _pole_mean_sequential)(gsrc) if pole_fix else gsrc
+    if not fp64:
+        return AtCoords(out=res, grad_field=grad_field, grad_u=grad_u, grad_v=grad_v)
+
+    # grad_field: sum |w g'| with (K + m) per contribution, the weights' rounding, and the count n_c
+    m_arr = torch.zeros(B, V, H, W, dtype=torch.float64, device=dev)
+    if pole_fix:
+        m_arr[:, :, 0, :] = W
+        m_arr[:, :, -1, :] = W
+    s_mag = torch.zeros(B, V, H * W, dtype=torch.float64, device=dev)
+    s_bnd = torch.zeros_like(s_mag)
+    n_c = torch.zeros_like(s_mag)
+    for idx, ok, w, (a, b, _, _) in taps:
+        okd = ok.double()
+        mag = okd * gmag * wy[a].abs() * wx[b].abs()
+        bnd = (K_GFIELD + m_arr) * mag + okd * gmag * (wy[a].abs() * rwx[b] + rwy[a] * wx[b].abs())
+        for acc, t in ((s_mag, mag), (s_bnd, bnd), (n_c, okd)):
+            acc.scatter_add_(2, idx.reshape(B, V, -1), t.reshape(B, V, -1))
+    gf_bound = (s_bnd + n_c * s_mag).reshape(B, V, H, W)
+    if pole_fix:
+        gf_bound = _row_mean_at_poles(gf_bound, W * s_mag.reshape(B, V, H, W))
+    gf_bound = gf_bound * U32
+
+    # grad_u / grad_v: absolute-value version of the formula
+    kx_m, ky_m = gmag * mx * Ax, gmag * my * Ay * dphi_ds
+    kx_e, ky_e = gmag * ex * Ax, gmag * ey * Ay * dphi_ds
+    adb = ((den * ca * cb).abs() + (num * ca * sb * cp).abs()) / r2
+    ada = ((den * sa * sb).abs() + (num * sa * cb * cp).abs() + (num * ca * sp).abs()) / r2
+    adsb, adsa = (ca * sb * sp).abs(), (ca * cp).abs() + (sa * cb * sp).abs()
+    kk = K_GRAD_UV + W * pole_pt.double()
+    gu_bound = U32 * abs(dt) * (kk * (kx_m * adb + ky_m * adsb) + kx_e * adb + ky_e * adsb)
+    gv_bound = U32 * abs(dt) * (kk * (kx_m * ada + ky_m * adsa) + kx_e * ada + ky_e * adsa)
+    return AtCoords(out=res, grad_field=grad_field, grad_u=grad_u, grad_v=grad_v, out_bound=out_bound,
+                    grad_field_bound=gf_bound, grad_u_bound=gu_bound, grad_v_bound=gv_bound, n_c=n_c.reshape(
+                        B, V, H, W), taps=taps)
+
+
+def bf16_bounds(ref, bound):
+    """Bound of a bf16 result: the fp32 bound plus one bf16 rounding of a value within it."""
+    return bound + U_BF16 * (ref.abs() + bound)
+
+
+def over_bound(got, ref, bound):
+    """Boolean mask of the points where |got - ref| exceeds the bound (NaN counts as over)."""
+    err = (got.double() - ref).abs()
+    return ~(err <= bound)
+
+
+def worst_ratio(got, ref, bound):
+    """max |got - ref| / bound (0 where both are 0)."""
+    err = (got.double() - ref).abs()
+    r = torch.where(bound > 0, err / torch.where(bound > 0, bound, torch.ones_like(bound)),
+                    torch.where(err > 0, torch.full_like(err, math.inf), torch.zeros_like(err)))
+    return float(r.max())
 
 
 # --------------------------------------------------------------------------
