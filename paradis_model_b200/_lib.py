@@ -1,5 +1,5 @@
 """ctypes binding of the C ABI declared in include/paradis_sl.h (and the bf16 entry points of
-include/paradis_sl_bf16.h and include/paradis_geocyclic.h, each in a table of its own).
+include/paradis_sl_bf16.h, include/paradis_geocyclic.h and include/paradis_sl_tl.h, each in a table of its own).
 
 The product has no CPU fallback: if the shared library is missing this module
 raises, it never substitutes another implementation.
@@ -90,6 +90,15 @@ _PROTOS_GEO = {
 }
 
 
+# include/paradis_sl_tl.h: tangent-linear model of the advection (same ABI version: entry points added)
+_PROTOS_TL = {
+    "paradis_sl_advect_jvp_workspace": (C.c_size_t, [C.c_int, C.c_int]),
+    "paradis_sl_advect_jvp": (C.c_int, [C.POINTER(Geom), _P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int64,
+                                        C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_float, C.c_int,
+                                        C.c_int, C.c_int, _P, C.c_size_t, _P, _P]),
+}
+
+
 def exported_symbols():
     """The functions of include/paradis_sl.h."""
     return list(_PROTOS)
@@ -103,6 +112,11 @@ def exported_symbols_bf16():
 def exported_symbols_geocyclic():
     """The functions of include/paradis_geocyclic.h."""
     return list(_PROTOS_GEO)
+
+
+def exported_symbols_tl():
+    """The functions of include/paradis_sl_tl.h."""
+    return list(_PROTOS_TL)
 
 
 def lib():
@@ -131,7 +145,8 @@ def lib():
             except Exception:
                 pass
         handle = C.CDLL(path)
-        for name, (res, args) in list(_PROTOS.items()) + list(_PROTOS_BF16.items()) + list(_PROTOS_GEO.items()):
+        for name, (res, args) in (list(_PROTOS.items()) + list(_PROTOS_BF16.items()) + list(_PROTOS_GEO.items())
+                           + list(_PROTOS_TL.items())):
             fn = getattr(handle, name)
             fn.restype, fn.argtypes = res, args
         if handle.paradis_sl_abi_version() != 2 and not os.environ.get("PARADIS_SL_SKIP_ABI_CHECK"):

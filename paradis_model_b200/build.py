@@ -12,8 +12,9 @@ LIB_PATH = os.path.join(LIB_DIR, "libparadis_sl.so")
 SOURCES = [os.path.join(_HERE, "csrc", "paradis_sl.cu"), os.path.join(_HERE, "csrc", "geo_dwconv.cu")]
 HEADERS = [os.path.join(_HERE, "csrc", "sl_device.cuh"), os.path.join(_HERE, "csrc", "sl_sweep.cuh"),
            os.path.join(_HERE, "csrc", "sl_partition.cuh"),
-           os.path.join(_HERE, "csrc", "sl_rows.cuh"),
+           os.path.join(_HERE, "csrc", "sl_rows.cuh"), os.path.join(_HERE, "csrc", "sl_tangent.cuh"),
            os.path.join(_HERE, "..", "include", "paradis_sl.h"),
+           os.path.join(_HERE, "..", "include", "paradis_sl_tl.h"),
            os.path.join(_HERE, "..", "include", "paradis_sl_bf16.h"),
            os.path.join(_HERE, "..", "include", "paradis_geocyclic.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -12,6 +12,7 @@
 //   sl_bwd_gather_kernel   grad_field: each output row gathers the arrival points whose stencil
 //                          covers it (inverse stencils), fixed order, no atomics
 //   geocyclic_pad_{fwd,bwd}_kernel  standalone padding op and its adjoint
+//   sl_tl_kernel           tangent-linear model: d out along (dfield, du, dv), one gather per point (sl_tangent.cuh)
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -25,6 +26,7 @@
 #include "../../include/paradis_sl.h"
 #include "../../include/paradis_sl_bf16.h"
 #include "../../include/paradis_geocyclic.h"
+#include "../../include/paradis_sl_tl.h"
 #include "sl_device.cuh"
 
 using namespace psl;
@@ -1205,17 +1207,23 @@ __global__ void f32_to_bf16_kernel(const float* __restrict__ src, bf16* __restri
   }
 }
 
-// Native bf16 path: full mesh only (default windows, no peer halos), W % 8 == 0, 16-byte aligned tensors, batch
-// strides in multiples of 8 elements (bf16) resp. 4 elements (fp32): every row then starts on 16 bytes.
-static int bf16_check(const paradis_sl_geom* g, const void* const* ptrs, int nptrs, const int64_t* sB8, int nsB8,
-                      const int64_t* sB4, int nsB4) {
+// Entry points that serve the full mesh only (default windows, no peer halos): PARADIS_ERR_BAD_SHAPE otherwise.
+static int full_mesh_check(const paradis_sl_geom* g, const char* who, const char* bands) {
   const int H = g->H;
   if (g->own_row0 != 0 || g->own_rows != H || g->arr_row0 != 0 || g->arr_rows != H || g->fld_row0 != 0 ||
       g->fld_rows != H)
-    return fail(PARADIS_ERR_BAD_SHAPE, "bf16 entry points work on the full mesh (latitude bands: use the fp32 entry points)");
+    return fail(PARADIS_ERR_BAD_SHAPE, "%s work on the full mesh (latitude bands: %s)", who, bands);
   bool peers = g->fld_peer_lo || g->fld_peer_hi;
   for (int k = 0; k < 3; ++k) peers = peers || g->arr_peer_lo[k] || g->arr_peer_hi[k];
-  if (peers) return fail(PARADIS_ERR_BAD_SHAPE, "bf16 entry points take no peer halo pointers");
+  if (peers) return fail(PARADIS_ERR_BAD_SHAPE, "%s take no peer halo pointers", who);
+  return PARADIS_OK;
+}
+
+// Native bf16 path: full mesh only, W % 8 == 0, 16-byte aligned tensors, batch strides in multiples of 8 elements
+// (bf16) resp. 4 elements (fp32): every row then starts on 16 bytes.
+static int bf16_check(const paradis_sl_geom* g, const void* const* ptrs, int nptrs, const int64_t* sB8, int nsB8,
+                      const int64_t* sB4, int nsB4) {
+  if (int rc = full_mesh_check(g, "bf16 entry points", "use the fp32 entry points")) return rc;
   if (g->W % 8) return fail(PARADIS_ERR_BAD_SHAPE, "bf16 entry points need W %% 8 == 0 (W=%d)", g->W);
   if (!aligned16(g->lon)) return fail(PARADIS_ERR_BAD_SHAPE, "bf16 entry points need a 16-byte aligned lon table");
   for (int k = 0; k < nptrs; ++k)
@@ -1496,4 +1504,54 @@ extern "C" int paradis_sl_advect_fwd_bwd_host(const paradis_sl_geom* geom, const
     cudaStreamDestroy(st[i]);
   }
   return rc;
+}
+
+// ---------------------------------------------------------------------------------------------
+// tangent-linear model (include/paradis_sl_tl.h)
+// ---------------------------------------------------------------------------------------------
+#include "sl_tangent.cuh"
+
+extern "C" size_t paradis_sl_advect_jvp_workspace(int B, int V) {
+  return 2 * paradis_sl_advect_fwd_workspace(B, V);      // zonal pole means of field | of dfield
+}
+
+extern "C" int paradis_sl_advect_jvp(const paradis_sl_geom* geom, const float* field, const float* dfield,
+                                     const float* u, const float* v, const float* du, const float* dv, float* dout,
+                                     int B, int V, int64_t field_sB, int64_t dfield_sB, int64_t u_sB, int64_t v_sB,
+                                     int64_t du_sB, int64_t dv_sB, float dt, int interp, int pole_fix, int math,
+                                     void* workspace, size_t workspace_bytes, int32_t* status, void* stream) {
+  Params P;
+  if (int rc = fill_params(P, geom, B, V, dt, interp, pole_fix)) return rc;
+  if (!field || !u || !v || !dout) return fail(PARADIS_ERR_NULL_POINTER, "NULL tensor pointer");
+  if ((du == nullptr) != (dv == nullptr)) return fail(PARADIS_ERR_NULL_POINTER, "du and dv must both be given or both be NULL");
+  if (int rc = full_mesh_check(geom, "tangent-linear entry points", "not supported")) return rc;
+  if (pole_fix && (!workspace || workspace_bytes < paradis_sl_advect_jvp_workspace(B, V)))
+    return fail(PARADIS_ERR_WORKSPACE, "jvp workspace too small (%zu bytes)", workspace_bytes);
+  cudaStream_t st = (cudaStream_t)stream;
+  const int planes = B * V;
+  P.field = field; P.u = u; P.v = v; P.out = dout;
+  P.field_sB = field_sB; P.u_sB = u_sB; P.v_sB = v_sB;
+  P.status = status;
+  TLArgs A;
+  A.dfield = dfield; A.du = du; A.dv = dv; A.dmean = nullptr;
+  A.dfield_sB = dfield_sB; A.du_sB = du_sB; A.dv_sB = dv_sB;
+  if (pole_fix) {      // zonal pole means of field and dfield in one launch
+    P.fmean = (const float*)workspace;
+    A.dmean = (const float*)((char*)workspace + paradis_sl_advect_fwd_workspace(B, V));
+    pole_means_kernel<float><<<planes * (dfield ? 4 : 2), kPoleThreads, 0, st>>>(
+        field, field_sB, V, P.fldN, P.fld0, P.H, P.W, planes, (float*)P.fmean, dfield, dfield_sB, P.fldN, P.fld0,
+        (float*)A.dmean);
+  }
+  const bool vec_ok = (P.W % 4 == 0) && aligned16(field) && aligned16(u) && aligned16(v) && aligned16(dout) &&
+                      aligned16(P.lon) && (!dfield || aligned16(dfield)) && (!du || (aligned16(du) && aligned16(dv))) &&
+                      (field_sB % 4 == 0) && (dfield_sB % 4 == 0) && (u_sB % 4 == 0) && (v_sB % 4 == 0) &&
+                      (du_sB % 4 == 0) && (dv_sB % 4 == 0);
+  const int vec = points_per_thread(interp, vec_ok);
+  set_units(P, vec, P.ownN);
+  dim3 grid(((unsigned)P.ownN * P.upr + 255) / 256, V, B);
+  const bool exact = math == PARADIS_MATH_EXACT;
+  if (interp == 1) { if (exact) launch_tl<true, 1>(P, A, vec, grid, st); else launch_tl<false, 1>(P, A, vec, grid, st); }
+  else             { if (exact) launch_tl<true, 2>(P, A, vec, grid, st); else launch_tl<false, 2>(P, A, vec, grid, st); }
+  if (pole_fix) pole_rows_fix_kernel<<<planes * 2, kPoleThreads, 0, st>>>(dout, P.ownN, P.own0, P.H, P.W, planes);
+  return check_launch("paradis_sl_advect_jvp");
 }

@@ -2,6 +2,7 @@
 
 Ops (namespace ``paradis``)
     sl_advect / sl_advect_backward      model/advection.py:129-169, fused
+    sl_advect_jvp                        its tangent-linear model (forward-mode AD), fused
     geocyclic_pad / geocyclic_pad_backward   model/padding.py:11-39
     geocyclic_dwconv / geocyclic_dwconv_backward(_bf16)   SepConv's pad + depthwise conv, model/blocks.py:112-114
     geocyclic_avgpool5 / geocyclic_avgpool5_backward      PhysicalDownsample, model/blocks.py:57-71
@@ -10,6 +11,12 @@ Each op has a fake (meta) implementation and an autograd formula, so it works un
 ``torch.compile(fullgraph=True)``, non-reentrant activation checkpointing (nothing but
 the inputs is saved; the trajectory is recomputed in backward) and bf16 autocast.
 CUDA only: there is no CPU implementation.
+
+Forward-mode AD (``torch.func.jvp``, ``torch.autograd.forward_ad``) works through every public wrapper: when an input
+carries a tangent, the wrapper calls its op through an autograd.Function with a jvp rule (sl_advect: the fused
+tangent-linear kernel on the full mesh; the GeoCyclic ops: compositions of their own kernels).  Without a tangent the
+op is called directly, as before.  vmap / jacfwd over a tangent, forward-over-reverse and tangents on latitude-band
+geometries raise NotImplementedError.
 
 Storage types of sl_advect.  The arithmetic is always fp32 (torch's own autocast policy runs
 grid_sampler / asin / atan2 in fp32) and ``out`` is fp32.  When field, u and v are all bf16 (what
@@ -34,7 +41,10 @@ import os
 from typing import List, Optional, Tuple
 
 import torch
+import torch.autograd.forward_ad as fwAD
 from torch import Tensor
+from torch._C._functorch import TransformType
+from torch._functorch.pyfunctorch import retrieve_all_functorch_interpreters
 
 from . import _lib
 
@@ -238,6 +248,51 @@ def _bf16_layout_ok(bf: List[Tensor], f32: List[Tensor]) -> bool:
 
 
 # --------------------------------------------------------------------------------------
+# forward-mode AD.  torch gives a custom op no forward-AD formula (its tangent would come out None or zero), so a
+# public wrapper whose inputs carry a tangent (torch.autograd.forward_ad or torch.func.jvp) calls the op through an
+# autograd.Function with a jvp rule instead.  Calls without a tangent call the op directly: dynamo refuses an
+# autograd.Function that defines jvp, and compiled training steps must not break their graph.
+# --------------------------------------------------------------------------------------
+def _has_tangent(*tensors) -> bool:
+    return any(t is not None and fwAD.unpack_dual(t).tangent is not None for t in tensors)
+
+
+def _transforms() -> list:
+    """The functorch transforms active around this call (outermost first); none while dynamo traces."""
+    if torch.compiler.is_compiling():
+        return []
+    return [i.key() for i in retrieve_all_functorch_interpreters()]
+
+
+def _tangent_path(*tensors) -> bool:
+    """True when an input carries a forward-mode tangent: the call must take the autograd.Function with a jvp rule.
+    Raises NotImplementedError where no rule exists (vmap / jacfwd, forward-over-reverse)."""
+    if _has_tangent(*tensors):
+        if TransformType.Vmap in _transforms():
+            raise NotImplementedError("paradis ops have no vmap rule: torch.func.vmap / jacfwd over a forward-mode tangent "
+                                      "is not supported (use torch.func.jvp or torch.autograd.forward_ad per direction)")
+        return True
+    t = _transforms()
+    if TransformType.Jvp in t and TransformType.Grad in t[t.index(TransformType.Jvp):]:
+        raise NotImplementedError("paradis ops support forward mode (jvp) and reverse mode (vjp / grad), not forward-over-"
+                                  "reverse: the backward ops have no tangent rule")
+    return False
+
+
+def _no_fwd_over_rev(*tensors) -> None:
+    """Guard of the backward formulas: the backward ops have no tangent rule, so a tangent on grad_out or on a saved
+    input (forward-over-reverse, e.g. Hessian-vector products) must not be dropped silently."""
+    if _has_tangent(*tensors):
+        raise NotImplementedError("paradis ops support forward mode (jvp) and reverse mode (vjp / grad), not forward-over-"
+                                  "reverse: the backward ops have no tangent rule")
+
+
+def _no_vmap(info, in_dims, *args):
+    raise NotImplementedError("paradis ops have no vmap rule: torch.func.vmap / jacfwd over a forward-mode tangent is "
+                              "not supported (use torch.func.jvp or torch.autograd.forward_ad per direction)")
+
+
+# --------------------------------------------------------------------------------------
 # sl_advect
 # --------------------------------------------------------------------------------------
 @torch.library.custom_op("paradis::sl_advect", mutates_args=(), device_types="cuda")
@@ -371,6 +426,7 @@ def _sl_setup(ctx, inputs, output):
 
 def _sl_backward(ctx, grad_out):
     field, u, v, tables = ctx.saved_tensors
+    _no_fwd_over_rev(grad_out, field, u, v)
     scalars, dt, interp, pole_fix, math, windows, cfl = ctx.attrs
     if list(windows[2:4]) != list(windows[4:6]):
         raise RuntimeError("autograd through a latitude-band sl_advect needs halo'd grad_out: "
@@ -389,6 +445,73 @@ def _sl_backward(ctx, grad_out):
 
 
 _sl_advect.register_autograd(_sl_backward, setup_context=_sl_setup)
+
+
+@torch.library.custom_op("paradis::sl_advect_jvp", mutates_args=(), device_types="cuda")
+def _sl_advect_jvp(field: Tensor, u: Tensor, v: Tensor, dfield: Optional[Tensor], du: Tensor, dv: Tensor,
+                   tables: Tensor, scalars: List[float], dt: float, interp: int, pole_fix: bool, math: int,
+                   windows: List[int]) -> Tensor:
+    """Tangent-linear model of sl_advect (include/paradis_sl_tl.h): d out along (dfield, du, dv), fp32.  dfield may be
+    None (velocity tangents only).  Full mesh only; every input is read as fp32 (bf16 / fp16 are upcast)."""
+    B, V, H, W, ownN, arrN = _check_inputs(field, u, v, windows)
+    if not _full_mesh(windows):
+        raise RuntimeError("paradis::sl_advect_jvp works on the full mesh only")
+    for name, t in (("dfield", dfield), ("du", du), ("dv", dv)):
+        if t is not None and tuple(t.shape) != tuple(field.shape if name == "dfield" else u.shape):
+            raise RuntimeError(f"paradis::sl_advect_jvp: {name} {tuple(t.shape)} does not match its primal")
+    if any(t is not None and t.dtype == torch.float64 for t in (field, u, v, dfield, du, dv)):
+        raise RuntimeError("paradis::sl_advect_jvp computes in fp32; cast float64 inputs explicitly")
+    poll_status(field.device)
+    if tables.device != field.device:
+        raise RuntimeError(f"paradis::sl_advect_jvp: geometry tables live on {tables.device}, the tensors on {field.device}")
+    field, u, v, du, dv = [_inner_contig(t.float()) for t in (field, u, v, du, dv)]
+    dfield = _inner_contig(dfield.float()) if dfield is not None else None
+    L = _lib.lib()
+    dout = torch.empty((B, V, ownN, W), dtype=torch.float32, device=field.device)
+    g = _geom_struct(tables, scalars, windows)
+    ws_bytes = L.paradis_sl_advect_jvp_workspace(B, V)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=field.device)
+    with torch.cuda.device(field.device):
+        rc = L.paradis_sl_advect_jvp(C.byref(g), _ptr(field), _ptr(dfield), _ptr(u), _ptr(v), _ptr(du), _ptr(dv),
+                                     _ptr(dout), B, V, field.stride(0), dfield.stride(0) if dfield is not None else 0,
+                                     u.stride(0), v.stride(0), du.stride(0), dv.stride(0), dt, interp, int(pole_fix),
+                                     math, _ptr(ws), ws_bytes, _ptr(_status_word(field.device)), _stream(field))
+    _lib.check(rc, "paradis_sl_advect_jvp")
+    return dout
+
+
+@_sl_advect_jvp.register_fake
+def _(field, u, v, dfield, du, dv, tables, scalars, dt, interp, pole_fix, math, windows):
+    B, V = field.shape[:2]
+    return field.new_empty((B, V, windows[3], windows[1]), dtype=torch.float32)
+
+
+class _SLAdvectFn(torch.autograd.Function):
+    """paradis::sl_advect with a jvp rule (forward-mode AD); same setup and backward as the op's own autograd."""
+
+    @staticmethod
+    def forward(field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl):
+        return torch.ops.paradis.sl_advect(field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl)
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        _sl_setup(ctx, inputs, output)
+        ctx.save_for_forward(*inputs[:4])
+        ctx.set_materialize_grads(False)        # inputs without a tangent reach jvp as None, not as zeros
+
+    backward = staticmethod(_sl_backward)
+    vmap = staticmethod(_no_vmap)
+
+    @staticmethod
+    def jvp(ctx, dfield, du, dv, *_):
+        field, u, v, tables = ctx.saved_tensors
+        scalars, dt, interp, pole_fix, math, windows, cfl = ctx.attrs
+        if du is None and dv is None:        # the op is linear in field: its tangent is the op applied to dfield
+            return torch.ops.paradis.sl_advect(dfield, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl)
+        du = du if du is not None else torch.zeros_like(u)
+        dv = dv if dv is not None else torch.zeros_like(v)
+        return torch.ops.paradis.sl_advect_jvp(field, u, v, dfield, du, dv, tables, scalars, dt, interp, pole_fix,
+                                               math, windows)
 
 
 DEFAULT_CFL_CELLS = 8.0
@@ -413,12 +536,21 @@ def sl_advect(field: Tensor, u: Tensor, v: Tensor, geometry: SLGeometry, dt: flo
     for the backward (expected bound on |(u, v)| * dt in latitude cells): planes that exceed it
     are detected on the device and recomputed by the general path, results never depend on it;
     ``0`` disables the fused backward.
+
+    Forward-mode AD (``torch.func.jvp``, ``torch.autograd.forward_ad``) gives the tangent-linear model on the full
+    mesh, in fp32 (``paradis::sl_advect_jvp``).
     """
     if _ENV_MATH:
         math = _ENV_MATH
-    out = torch.ops.paradis.sl_advect(field, u, v, geometry.tables, geometry.scalars, float(dt),
-                                      _lib.INTERP[interpolation], bool(pole_fix), _lib.MATH[math],
-                                      geometry.windows, float(cfl_cells))
+    args = (geometry.tables, geometry.scalars, float(dt), _lib.INTERP[interpolation], bool(pole_fix), _lib.MATH[math],
+            geometry.windows, float(cfl_cells))
+    if _tangent_path(field, u, v):
+        if not _full_mesh(geometry.windows):
+            raise NotImplementedError("forward-mode AD through sl_advect is supported on the full mesh only, not on "
+                                      "latitude-band geometries")
+        out = _SLAdvectFn.apply(field, u, v, *args)
+    else:
+        out = torch.ops.paradis.sl_advect(field, u, v, *args)
     if _ENV_CHECK:
         check_status(field.device)
     return out
@@ -473,10 +605,27 @@ def _pad_setup(ctx, inputs, output):
 
 
 def _pad_backward(ctx, gy):
+    _no_fwd_over_rev(gy)
     return torch.ops.paradis.geocyclic_pad_backward(gy, ctx.p), None
 
 
 _geocyclic_pad.register_autograd(_pad_backward, setup_context=_pad_setup)
+
+
+class _PadFn(torch.autograd.Function):
+    """paradis::geocyclic_pad with a jvp rule: the op is linear, its tangent is the op applied to the tangent."""
+
+    @staticmethod
+    def forward(x, p):
+        return torch.ops.paradis.geocyclic_pad(x, p)
+
+    setup_context = staticmethod(_pad_setup)
+    backward = staticmethod(_pad_backward)
+    vmap = staticmethod(_no_vmap)
+
+    @staticmethod
+    def jvp(ctx, dx, _):
+        return torch.ops.paradis.geocyclic_pad(dx, ctx.p)
 
 
 def geocyclic_pad(x: Tensor, pad_width: int) -> Tensor:
@@ -485,6 +634,8 @@ def geocyclic_pad(x: Tensor, pad_width: int) -> Tensor:
         return x
     assert x.dim() == 4, "Input must be 4-dimensional [batch, channels, lat, lon]"
     assert x.shape[3] % 2 == 0, "Number of longitude points must be even"
+    if _tangent_path(x):
+        return _PadFn.apply(x, int(pad_width))
     return torch.ops.paradis.geocyclic_pad(x, int(pad_width))
 
 
@@ -589,6 +740,7 @@ def _dw_setup(ctx, inputs, output):
 
 def _dw_backward(ctx, gy):
     x, weight = ctx.saved_tensors
+    _no_fwd_over_rev(gy, x, weight)
     need_x, need_w = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
     need_b = ctx.has_bias and ctx.needs_input_grad[2]
     if not (need_x or need_w or need_b):
@@ -602,6 +754,39 @@ def _dw_backward(ctx, gy):
 
 
 _geocyclic_dwconv.register_autograd(_dw_backward, setup_context=_dw_setup)
+
+
+class _DwConvFn(torch.autograd.Function):
+    """paradis::geocyclic_dwconv with a jvp rule.  The op is bilinear in (x, weight) and affine in bias:
+    d y = dwconv(dx, w) + dwconv(x, dw) + db, each term summed in fp32 and rounded once to y's dtype."""
+
+    @staticmethod
+    def forward(x, weight, bias):
+        return torch.ops.paradis.geocyclic_dwconv(x, weight, bias)
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        _dw_setup(ctx, inputs, output)
+        ctx.save_for_forward(inputs[0], inputs[1])
+        ctx.set_materialize_grads(False)        # inputs without a tangent reach jvp as None, not as zeros
+
+    backward = staticmethod(_dw_backward)
+    vmap = staticmethod(_no_vmap)
+
+    @staticmethod
+    def jvp(ctx, dx, dw, db):
+        x, weight = ctx.saved_tensors
+        terms = []
+        if dx is not None:
+            terms.append(torch.ops.paradis.geocyclic_dwconv(dx, weight, None).float())
+        if dw is not None:
+            terms.append(torch.ops.paradis.geocyclic_dwconv(x, dw, None).float())
+        if db is not None and ctx.has_bias:
+            terms.append(db.float().view(1, -1, 1, 1).expand(x.shape))
+        dy = terms[0]
+        for t in terms[1:]:
+            dy = dy + t
+        return dy.to(x.dtype).contiguous()
 
 
 # --------------------------------------------------------------------------------------
@@ -655,6 +840,7 @@ def _pool_setup(ctx, inputs, output):
 
 
 def _pool_backward(ctx, gy):
+    _no_fwd_over_rev(gy)
     B, Cn, H, W = ctx.shape
     return torch.ops.paradis.geocyclic_avgpool5_backward(gy, H, W, ctx.stride).to(ctx.dtype), None
 
@@ -662,10 +848,28 @@ def _pool_backward(ctx, gy):
 _geocyclic_avgpool5.register_autograd(_pool_backward, setup_context=_pool_setup)
 
 
+class _PoolFn(torch.autograd.Function):
+    """paradis::geocyclic_avgpool5 with a jvp rule: the op is linear, its tangent is the op applied to the tangent."""
+
+    @staticmethod
+    def forward(x, stride):
+        return torch.ops.paradis.geocyclic_avgpool5(x, stride)
+
+    setup_context = staticmethod(_pool_setup)
+    backward = staticmethod(_pool_backward)
+    vmap = staticmethod(_no_vmap)
+
+    @staticmethod
+    def jvp(ctx, dx, _):
+        return torch.ops.paradis.geocyclic_avgpool5(dx, ctx.stride)
+
+
 def geocyclic_avgpool5(x: Tensor, stride: int) -> Tensor:
     """``AvgPool2d(5, stride)(GeoCyclicPadding(2)(x))`` (model/blocks.py:57-71) in one kernel."""
     assert x.dim() == 4, "Input must be 4-dimensional [batch, channels, lat, lon]"
     assert x.shape[3] % 2 == 0, "Number of longitude points must be even"
+    if _tangent_path(x):
+        return _PoolFn.apply(x, int(stride))
     return torch.ops.paradis.geocyclic_avgpool5(x, int(stride))
 
 
@@ -700,6 +904,8 @@ def geocyclic_dwconv(x: Tensor, weight: Tensor, bias: Optional[Tensor] = None) -
     two lines of SepConv.forward (model/blocks.py:112-114).  Differentiable w.r.t. x, weight and bias."""
     assert x.dim() == 4, "Input must be 4-dimensional [batch, channels, lat, lon]"
     assert x.shape[3] % 2 == 0, "Number of longitude points must be even"
+    if _tangent_path(x, weight, bias):
+        return _DwConvFn.apply(x, weight, bias)
     return torch.ops.paradis.geocyclic_dwconv(x, weight, bias)
 
 
