@@ -170,7 +170,6 @@ __global__ void __launch_bounds__(256) sl_fwd_kernel(const Params P) {
 #pragma unroll
     for (int k = 0; k < VEC; ++k) { uu[k] = ldcs_f(up + k); vv[k] = ldcs_f(vp + k); ll[k] = __ldg(P.lon + x + k); }
   }
-#ifndef PSL_FWD_NO_PAIRS
   if (!EXACT && VEC == 4) {
     // FAST math: the 4 departure points of the thread as two packed pairs (FFMA2 / FMUL2 / FADD2), bit-identical to
     // the scalar chain
@@ -186,9 +185,7 @@ __global__ void __launch_bounds__(256) sl_fwd_kernel(const Params P) {
         stencil_eval<INTERP, false, PEER>(P, f, pl, t, mean0, mean1, oo[2 * h + e], dx, dy);
       }
     }
-  } else
-#endif
-  {
+  } else {
 #pragma unroll
     for (int k = 0; k < VEC; ++k) {
       Traj t;
@@ -203,54 +200,6 @@ __global__ void __launch_bounds__(256) sl_fwd_kernel(const Params P) {
 #pragma unroll
     for (int k = 0; k < VEC; ++k) __stcs(op + k, oo[k]);
   }
-}
-
-// FAST-math forward, round 2: the own rows of a plane are one flat array of points; a warp takes 128
-// consecutive points, lane l the points l, l + 32, l + 64, l + 96 -- consecutive lanes on consecutive columns, so
-// every load, store and stencil tap of a warp touches one or two 128-byte lines (the float4-per-thread layout
-// spread the 4 taps of a warp over 5 lines each: the L1 data pipe was 77 % busy) -- and the 4 departure points
-// are computed as two packed pairs (FFMA2 / FMUL2 / FADD2: two points per instruction).  Any W, any alignment.
-template <int INTERP, bool PEER>
-__global__ void __launch_bounds__(256) sl_fwd_pair_kernel(const Params P, const int gpr) {
-  // one warp = 128 consecutive columns of one row (gpr groups per row; the last group of a row may be short)
-  const int c = blockIdx.y, b = blockIdx.z, pl = b * P.V + c;
-  const int lane = threadIdx.x & 31;
-  const int G = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  const int r = G / gpr;
-  if (r >= P.ownN) return;
-  const int xb = (G - r * gpr) * 128 + lane, y = P.own0 + r;
-  const float sp = __ldg(P.sin_lat + y), cp = __ldg(P.cos_lat + y);
-  const float* f = plane_ptr_bc(P.field, P.field_sB, b, c, P.fldN, P.W);
-  const int aoff = (y - P.uvg0) * P.W;
-  const float* up = plane_ptr_bc(P.u, P.u_sB, b, c, P.uvgN, P.W) + aoff;
-  const float* vp = plane_ptr_bc(P.v, P.v_sB, b, c, P.uvgN, P.W) + aoff;
-  float* op = P.out + ((long long)pl * P.ownN + r) * P.W;
-  float mean0 = 0.0f, mean1 = 0.0f;
-  if (P.pole_fix) { mean0 = __ldg(P.fmean + 2 * pl); mean1 = __ldg(P.fmean + 2 * pl + 1); }
-  float uu[4], vv[4], ll[4];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const int x = min(xb + 32 * k, P.W - 1);              // lanes past the row end redo its last point (not stored)
-    uu[k] = __ldcs(up + x); vv[k] = __ldcs(vp + x); ll[k] = __ldg(P.lon + x);
-  }
-  float oo[4];
-#pragma unroll
-  for (int h = 0; h < 2; ++h) {
-    if (xb - lane + 64 * h < P.W) {                        // uniform: skip a pair that lies past the row end
-      Traj2 t2;
-      trajectory_2(P, make_float2(uu[2 * h], uu[2 * h + 1]), make_float2(vv[2 * h], vv[2 * h + 1]), f2s(sp), f2s(cp),
-                   make_float2(ll[2 * h], ll[2 * h + 1]), t2);
-#pragma unroll
-      for (int e = 0; e < 2; ++e) {
-        const Traj t = traj_half(t2, e);
-        float dx, dy;
-        stencil_eval<INTERP, false, PEER>(P, f, pl, t, mean0, mean1, oo[2 * h + e], dx, dy);
-      }
-    }
-  }
-#pragma unroll
-  for (int k = 0; k < 4; ++k)
-    if (xb + 32 * k < P.W) __stcs(op + xb + 32 * k, oo[k]);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -633,9 +582,7 @@ static size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 // stencil is bound by its gathers and wants one point per lane -- consecutive lanes hit consecutive
 // addresses (few sectors per request) and 32 registers give full occupancy (0.97 vs 1.89 ms at C3).
 static int points_per_thread(int interp, bool vec_ok) {
-  static const int env = getenv("PARADIS_SL_VEC") ? atoi(getenv("PARADIS_SL_VEC")) : 0;   // experiments: 1 or 4
   if (!vec_ok) return 1;
-  if (env == 1 || env == 4) return env;
   return interp == PARADIS_INTERP_BICUBIC ? 1 : 4;
 }
 
@@ -754,16 +701,7 @@ static int advect_fwd(Params& P, const void* field, const void* u, const void* v
   const unsigned units = (unsigned)P.ownN * P.upr;
   dim3 grid((units + 255) / 256, V, B);
   const bool exact = math == PARADIS_MATH_EXACT;
-  // experiments: PARADIS_SL_FWD=2 selects the packed-pair forward (consecutive lanes on consecutive columns, FFMA2
-  // trajectory, fp32 storage only): bit-identical output, measured 0.43 ms against 0.38 ms for the float4-per-thread
-  // kernel at C3
-  static const int fwd_mode = getenv("PARADIS_SL_FWD") ? atoi(getenv("PARADIS_SL_FWD")) : 0;
-  if (kIsF32<T> && !exact && interp == 1 && fwd_mode == 2) {
-    const int gpr = (P.W + 127) / 128;
-    dim3 pgrid((unsigned)(((long long)gpr * P.ownN + 7) / 8), V, B);       // 8 warps per CTA
-    if (P.f_halo > 0) sl_fwd_pair_kernel<1, true><<<pgrid, 256, 0, st>>>(P, gpr);
-    else sl_fwd_pair_kernel<1, false><<<pgrid, 256, 0, st>>>(P, gpr);
-  } else if (interp == 1) { if (exact) launch_fwd<true, 1, T>(P, vec, grid, st); else launch_fwd<false, 1, T>(P, vec, grid, st); }
+  if (interp == 1) { if (exact) launch_fwd<true, 1, T>(P, vec, grid, st); else launch_fwd<false, 1, T>(P, vec, grid, st); }
   else             { if (exact) launch_fwd<true, 2, T>(P, vec, grid, st); else launch_fwd<false, 2, T>(P, vec, grid, st); }
   if (pole_fix) pole_rows_fix_kernel<<<planes * 2, kPoleThreads, 0, st>>>(out, P.ownN, P.own0, P.H, P.W, planes);
   return PARADIS_OK;
@@ -798,8 +736,8 @@ static BwdWs bwd_layout(int B, int V, int arr_rows, int W) {
   w.reach = off; off += 3 * w.reach_stride;
   w.flag = off; off += align_up(planes, 256);
   w.hx = off; off += 65536 * sizeof(int);          // longitudinal reach per arrival row (rows kernel)
-  // guard columns of the rows kernel: [planes][rows][consumers][NT - 1]
-  w.guard = off; off += align_up(planes * (size_t)arr_rows * kRowsWarps * kStreams * 3 * sizeof(float), 256);
+  // guard columns of the rows kernel: [planes][rows][strips][NT - 1], sized for kRowsWarps strips and NT = 4
+  w.guard = off; off += align_up(planes * (size_t)arr_rows * kRowsWarps * 3 * sizeof(float), 256);
   // partial destination rows either side of the cuts of the rows kernel: [CTAs][2][GR][strips * pitch]
   w.grow_bytes = align_up((size_t)kRowsMaxCtas * 2 * kRowsMaxGuardRows * ((size_t)W + 256) * sizeof(float), 256);
   w.grow = off; off += w.grow_bytes;
@@ -914,9 +852,6 @@ static bool plan_sweep(const Params& P, float cfl_cells, int planes, int capacit
   int nb = capacity_warps / (planes * nstrips);  // bands so that all tasks are resident at once
   if (nb < 1) nb = 1;
   while (nb > 1 && (hi - lo) / nb < 4 * yh) --nb;  // keep the row halo a minor cost
-#ifdef PSL_FORCE_NB
-  nb = PSL_FORCE_NB;
-#endif
   if (nb > kMaxBands) nb = kMaxBands;
   S.nbands = nb;
   {
@@ -957,15 +892,13 @@ static bool launch_rows(const Params& P, cudaStream_t st, float cfl_cells, const
   RowsPlan S;
   memset(&S, 0, sizeof(S));
   S.planes = planes; S.rr = rr; S.ring = 2 * rr + NT;
-  static const int env_nc = env_int("PARADIS_SL_ROWS_NC", 0);
-  int nC = env_nc > 0 ? env_nc : (INTERP == 1 ? 6 : 8);
-  if (nC > kRowsMaxConsumers) nC = kRowsMaxConsumers;
-  int nS = nC * kStreams;                                  // strips: kStreams per consumer warp
+  // one strip per consumer warp, at least 32 columns wide: 6 consumer warps for the 2x2 stencil (1.58 ms at C3 against
+  // 1.69 / 1.63 / 1.71 for 5 / 7 / 8, DESIGN.md section 8), 8 for the 4x4 stencil
+  int nS = INTERP == 1 ? 6 : 8;
   int wc = ((W + nS - 1) / nS + 3) & ~3;
   if (wc < 32) wc = 32;
   nS = (W + wc - 1) / wc;
-  nC = (nS + kStreams - 1) / kStreams;
-  S.nC = nC; S.nS = nS; S.wc = wc; S.nP = kRowsWarps - 1 - nC;
+  S.nC = nS; S.nS = nS; S.wc = wc; S.nP = kRowsWarps - 1 - nS;
   if (S.nP < 1) return false;
   S.nsteps = (W + 32 * kStepSub - 1) / (32 * kStepSub);
   // a row is cut into nsteps producer steps and at most kRowRecs rows are in flight: narrow meshes leave most of the
@@ -999,19 +932,16 @@ static bool launch_rows(const Params& P, cudaStream_t st, float cfl_cells, const
   S.guard = (float*)(ws + L.guard);
   // one CTA per SM unless that leaves a CTA fewer than ~12 own rows (a ring warm-up is ring - 1 rows).  The floor was 24
   // at first: the 47-row polar band of the 8-way split then ran on 125 of the 148 SMs (backward 0.38 instead of 0.32 ms)
-  static const int env_rows = env_int("PARADIS_SL_ROWS_PER_CTA", 12);
-  int grid = S.total_rows / (env_rows > 0 ? env_rows : 12);
+  int grid = S.total_rows / 12;
   if (grid < 1) grid = 1;
   if (grid > nsm) grid = nsm;
   if (grid > kRowsMaxCtas) grid = kRowsMaxCtas;
   // Cut mode (see RowsPlan::cut): on for latitude bands, where a CTA owns few rows and the ring - 1 warm-up rows of
   // every segment weigh most (8-way split of C3: band backward 0.32 / 0.30 -> 0.275 ms); a full mesh gains nothing
-  // (1.58 ms either way).  PARADIS_SL_ROWS_CUT = 0 / 1 forces it off / on.
-  static const int env_cut = env_int("PARADIS_SL_ROWS_CUT", -1);
-  const bool want_cut = env_cut < 0 ? P.ownN < H : env_cut != 0;
+  // (1.58 ms either way).
   S.GR = rr + NT;
   S.grow = (float*)(ws + L.grow);
-  S.cut = (want_cut && S.GR <= kRowsMaxGuardRows &&
+  S.cut = (P.ownN < H && S.GR <= kRowsMaxGuardRows &&
            (size_t)grid * 2 * S.GR * nS * S.pitch * sizeof(float) <= L.grow_bytes) ? 1 : 0;
   rows_partition<INTERP>(P, S, reach, wc, planes, grid);
   kern<<<grid, kRowsWarps * 32, smem, st>>>(P, S);
@@ -1073,12 +1003,9 @@ static int launch_bwd(Params P, int vec, cudaStream_t st, int phases, float cfl_
     return launch_general<EXACT, INTERP, T>(P, vec, st, want_field, phases, L.nblk);
 
   // ---- warp-specialised row sweep (all latitudes); planes that break its contract fall back below
-  static const int bwd_mode = env_int("PARADIS_SL_BWD", 0);      // experiments: 1 = round-1 strip sweep, 2 = general path only
-  if (bwd_mode == 2) return launch_general<EXACT, INTERP, T>(P, vec, st, want_field, phases, L.nblk);
-  // (4x4 stencil: the round-1 strip sweep is still the faster kernel, 3.65 against 4.6 ms at C3; PARADIS_SL_BWD=3
+  // (4x4 stencil: the round-1 strip sweep is still the faster kernel, 3.65 against 4.6 ms at C3; PARADIS_BWD_ROWSWEEP
   // forces the row sweep for it)
-  if ((bwd_mode == 3 || force_rows || (bwd_mode == 0 && INTERP == 1)) &&
-      launch_rows<EXACT, INTERP, T>(P, st, cfl_cells, L, ws, bwd_mode == 3 || force_rows)) {
+  if ((force_rows || INTERP == 1) && launch_rows<EXACT, INTERP, T>(P, st, cfl_cells, L, ws, force_rows)) {
     Params Q = P;
     Q.plane_filter = (unsigned char*)(ws + L.flag);
     Q.gu = nullptr; Q.gv = nullptr;                   // grad_u / grad_v are already complete
@@ -1422,12 +1349,8 @@ extern "C" int paradis_geocyclic_pad_bwd_bf16(const void* gy, void* gx, int64_t 
 // across chunks because consecutive chunks live on different streams and slots)
 // ---------------------------------------------------------------------------------------------
 // chunks in flight (each on its own stream): H2D of one, kernels of another, D2H of a third overlap; more slots keep
-// both copy engines busy across the slot-reuse dependency.  PARADIS_SL_HOST_SLOTS overrides (2..8).
-static constexpr int kMaxSlots = 8;
-static int host_slots() {
-  static const int n = [] { const char* v = getenv("PARADIS_SL_HOST_SLOTS"); int k = v ? atoi(v) : 4;   /* 25.4-26.5 ms at C3 for 3-6 slots: PCIe bound */ return k < 2 ? 2 : (k > kMaxSlots ? kMaxSlots : k); }();
-  return n;
-}
+// both copy engines busy across the slot-reuse dependency (25.4-26.5 ms at C3 for 3-6 slots: PCIe bound)
+static constexpr int kSlots = 4;
 
 struct HostSlot { size_t field, u, v, gout, out, gfield, gu, gv, wsf, wsb, status, total; };
 static HostSlot host_slot_layout(int H, int W, int c) {
@@ -1445,7 +1368,7 @@ static HostSlot host_slot_layout(int H, int W, int c) {
 
 extern "C" size_t paradis_sl_host_scratch_bytes(int H, int W, int chunk_planes) {
   if (H <= 0 || W <= 0 || chunk_planes <= 0) return 0;
-  return host_slot_layout(H, W, chunk_planes).total * host_slots();
+  return host_slot_layout(H, W, chunk_planes).total * kSlots;
 }
 
 extern "C" int paradis_sl_advect_fwd_bwd_host(const paradis_sl_geom* geom, const float* h_field, const float* h_u,
@@ -1462,10 +1385,9 @@ extern "C" int paradis_sl_advect_fwd_bwd_host(const paradis_sl_geom* geom, const
   if (geom->own_row0 != 0 || geom->own_rows != H || geom->arr_rows != H || geom->fld_rows != H)
     return fail(PARADIS_ERR_BAD_SHAPE, "host entry works on the full mesh");
   const HostSlot L = host_slot_layout(H, W, chunk_planes);
-  const int kSlots = host_slots();
   if (!d_scratch || scratch_bytes < L.total * kSlots)
     return fail(PARADIS_ERR_WORKSPACE, "host-entry scratch too small (%zu < %zu bytes)", scratch_bytes, L.total * kSlots);
-  cudaStream_t st[kMaxSlots];
+  cudaStream_t st[kSlots];
   for (int i = 0; i < kSlots; ++i)
     if (cudaStreamCreateWithFlags(&st[i], cudaStreamNonBlocking) != cudaSuccess)
       return fail(PARADIS_ERR_CUDA, "cudaStreamCreate failed");

@@ -2,10 +2,8 @@
 // owns.  Pure host code (no CUDA calls): paradis_sl.cu includes it, and tests/partition_harness.cu compiles it alone so
 // that the CPU test-suite can check its invariants (tests/test_partition.py).
 #pragma once
-#include <stdlib.h>
 #include <string.h>
 #include <math.h>
-#include <stdio.h>
 #include <vector>
 #include "sl_device.cuh"
 #include "sl_sweep.cuh"
@@ -13,28 +11,21 @@
 
 namespace psl {
 
-static inline int env_int(const char* name, int dflt) {
-  const char* v = getenv(name);
-  return v ? atoi(v) : dflt;
-}
-
 // Min-max partition of the concatenated (plane, own row) space into `grid` contiguous CTA ranges.
 // Cost of a range = sum over its segments (one per plane it touches) of the cost of the ARRIVAL rows the segment sweeps:
-// its own rows plus the ring - 1 warm-up rows, clipped to the arrival window.  A row costs w0 + k(y), k = 32-record
+// its own rows plus the ring - 1 warm-up rows, clipped to the arrival window.  A row costs kRowW0 + k(y), k = 32-record
 // steps a consumer scans for it (the whole circle near the poles).  The smallest per-CTA budget T for which a greedy
 // left-to-right fill needs at most `grid` ranges is found by bisection; tiny segments are avoided by construction
 // (they pay a full warm-up).  An earlier version split proportionally to the own rows' cost and snapped boundaries
 // onto plane boundaries: 5 % slower at C3, 11-22 % on thin latitude bands.  Only balance depends on the model.
 // The result is cached per shape (it costs ~1 ms of host time).
-struct RowsPartKey { long long v[14]; };
+constexpr int kRowW0 = 4;   // shallow optimum at 3-6 (DESIGN.md section 8)
+struct RowsPartKey { long long v[13]; };
 struct RowsPartEntry { RowsPartKey key; int bound[kRowsMaxCtas + 1]; int cut; bool valid; };
 
 template <int INTERP>
 static void rows_partition(const Params& P, RowsPlan& S, const ReachModel& reach, int wc, int planes, int grid) {
   constexpr int NT = Stencil<INTERP>::NT, OMIN = Stencil<INTERP>::OMIN;
-  static const int env_w0 = env_int("PARADIS_SL_ROWS_W0", 4);
-  static const double env_capw = env_int("PARADIS_SL_ROWS_CAPW100", 100) / 100.0;   // weight of the whole-circle rows
-  static const int env_wcore = env_int("PARADIS_SL_ROWS_WCORE", 0);   // extra cost of a row whose grad_u / grad_v the segment writes
   static thread_local RowsPartEntry cache[8];
   static thread_local int cache_next = 0;
   RowsPartKey key;
@@ -42,7 +33,7 @@ static void rows_partition(const Params& P, RowsPlan& S, const ReachModel& reach
   const int H = P.H, W = P.W, ownN = P.ownN;
   int fbits[2];
   memcpy(&fbits[0], &P.min_lat, 4); memcpy(&fbits[1], &P.d_lat, 4);
-  const long long kv[14] = {H, W, planes, P.own0, ownN, P.arr0, P.arrN, S.rr + 1000 * S.cut, NT, wc, grid, env_w0, fbits[0], fbits[1]};
+  const long long kv[13] = {H, W, planes, P.own0, ownN, P.arr0, P.arrN, S.rr + 1000 * S.cut, NT, wc, grid, fbits[0], fbits[1]};
   memcpy(key.v, kv, sizeof(kv));
   for (auto& e : cache)
     if (e.valid && memcmp(&e.key, &key, sizeof(key)) == 0) { memcpy(S.bound, e.bound, sizeof(S.bound)); S.cut = e.cut; return; }
@@ -56,7 +47,7 @@ static void rows_partition(const Params& P, RowsPlan& S, const ReachModel& reach
     if (len > W) len = W;
     int k = (len + 31) >> 5;
     if ((k & 3) == 0) ++k;
-    A[y + 1] = A[y] + env_w0 + (len >= W ? k * env_capw : (double)k);
+    A[y + 1] = A[y] + kRowW0 + k;
   }
   const int arr_lo = P.arr0, arr_hi = P.arr0 + P.arrN;
   auto seg_cost = [&](int ra, int rb) {                     // destination rows [ra, rb) (global) of one plane
@@ -66,8 +57,7 @@ static void rows_partition(const Params& P, RowsPlan& S, const ReachModel& reach
     int y0 = cut_lo ? ra : ra - (S.ring - 1) + S.rr - OMIN, y1 = cut_hi ? rb - 1 : rb - 1 + S.rr - OMIN;
     if (y0 < arr_lo) y0 = arr_lo;
     if (y1 > arr_hi - 1) y1 = arr_hi - 1;
-    return (y1 >= y0 ? A[y1 + 1] - A[y0] : 0.0) + (double)env_wcore * (rb - ra) +
-           (double)env_w0 * S.GR * ((cut_lo ? 1 : 0) + (cut_hi ? 1 : 0));
+    return (y1 >= y0 ? A[y1 + 1] - A[y0] : 0.0) + (double)kRowW0 * S.GR * ((cut_lo ? 1 : 0) + (cut_hi ? 1 : 0));
   };
   const long long total = (long long)planes * ownN;
   const double plane_cost = seg_cost(P.own0, P.own0 + ownN);
@@ -130,18 +120,6 @@ static void rows_partition(const Params& P, RowsPlan& S, const ReachModel& reach
       S.cut = 0;
       rows_partition<INTERP>(P, S, reach, wc, planes, grid);        // (cached under its own key)
     }
-  }
-  static const int env_dump = env_int("PARADIS_SL_ROWS_DUMP", 0);
-  if (env_dump) {
-    int ncut = 0, minlen = 1 << 30, maxlen = 0, used = 0;
-    for (int c = 0; c < grid; ++c) {
-      const int n = S.bound[c + 1] - S.bound[c];
-      if (n <= 0) continue;
-      ++used; if (n < minlen) minlen = n; if (n > maxlen) maxlen = n;
-      if (S.bound[c + 1] % ownN != 0) ++ncut;
-    }
-    fprintf(stderr, "[paradis_sl] rows partition: %d of %d CTAs, %d cuts, rows per CTA %d..%d, cut mode %d, budget %.0f\n",
-            used, grid, ncut, minlen, maxlen, S.cut, hi);
   }
   RowsPartEntry& e = cache[cache_next];
   cache_next = (cache_next + 1) % 8;

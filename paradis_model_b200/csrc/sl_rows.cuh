@@ -44,37 +44,20 @@
 
 namespace psl {
 
-#ifndef PSL_ROWS_STAGES
-#define PSL_ROWS_STAGES 2
-#endif
-#ifndef PSL_ROWS_RECS
-#define PSL_ROWS_RECS 3
-#endif
-constexpr int kRowStages = PSL_ROWS_STAGES;   // u, v, grad_out rows in flight (TMA)
-constexpr int kRowRecs = PSL_ROWS_RECS;       // record rows in flight between producers and consumers
-#ifndef PSL_ROWS_SUB
-#define PSL_ROWS_SUB 4
-#endif
-constexpr int kStepSub = PSL_ROWS_SUB;   // 32-column sub-blocks per producer step
-constexpr int kTagBytes = 512;     // clash tags per strip (hashed, power of two)
-#ifndef PSL_ROWS_STREAMS
-#define PSL_ROWS_STREAMS 1
-#endif
-constexpr int kStreams = PSL_ROWS_STREAMS;   // strips a consumer warp works on in an interleaved manner
+constexpr int kRowStages = 2;   // u, v, grad_out rows in flight (TMA)
+constexpr int kRowRecs = 3;     // record rows in flight between producers and consumers
+constexpr int kStepSub = 4;     // 32-column sub-blocks per producer step
+constexpr int kTagBytes = 512;  // clash tags per strip (hashed, power of two)
 constexpr int kRowsMaxCtas = 192;
 // Warp budget: loader + producers + consumers.  20 warps = 640 threads -> 96 registers, no spills.  (Re-partitioning
 // the register file between the roles with setmaxnreg -- 16 producers at 96-104 registers, loader + 7 consumers at
 // 40-64 -- was tried: slower, 2.2-2.9 ms against 1.82, and two of the four splits hung; removed.)
-#ifndef PSL_ROWS_WARPS
-#define PSL_ROWS_WARPS 20
-#endif
-constexpr int kRowsWarps = PSL_ROWS_WARPS;
-constexpr int kRowsMaxConsumers = kRowsWarps - 2;
+constexpr int kRowsWarps = 20;
 
 struct RowsPlan {
   int planes, rr, ring;            // ring = 2 rr + NT destination rows
   int nP, nC;                      // producer / consumer warps (warp 0 is the loader)
-  int nS;                          // strips = private rings (kStreams per consumer warp)
+  int nS;                          // strips = private rings, one per consumer warp (nS == nC)
   int wc;                          // strip width (multiple of 4)
   int pitch, ring_stride;          // private ring of a consumer: (ring + NT - 1) rows of `pitch` floats = ring_stride
   float* guard;                    // [planes][outN][nS][NT - 1] guard columns of the retired rows (added by a post-kernel)
@@ -205,63 +188,38 @@ __device__ __forceinline__ void rows_weights(const float4 rec, bool act, bool la
   }
 }
 
-// ---- consumer: one step (32 records of each of the warp's kStreams strips), rows whose stencils stay inside
-// rows 0 .. H-1 (no cap fold).
+// ---- consumer: one step (32 records of the warp's strip), rows whose stencils stay inside rows 0 .. H-1 (no cap
+// fold).
 // A strip's ring is private: `pitch` columns = its wc own columns + NT-1 guard columns (taps that spill into the
 // next strip; a post-kernel adds them to that strip's first columns), ring + NT-1 rows (the last NT-1 alias the
 // first ones, folded together when a row retires).  A record belongs to the strip that owns the column of its
 // tap 0, and all its taps sit at base + a * pitch + b: no wrap, no per-tap ownership test.
-// The strips of a warp are advanced together: their rings are disjoint, so between two warp barriers there are
-// kStreams independent load-add-store chains instead of one (the consumers are latency bound).
+// A consumer warp owns one strip (two strips per warp, advanced together as two independent load-add-store chains,
+// were slower: DESIGN.md section 8).
 struct RowsStrip { float* ring; unsigned char* tag; int ja, wc; };
 
 template <int INTERP>
-__device__ __forceinline__ void rows_scatter_plain(const float4 (&rec)[kStreams], const bool (&inr)[kStreams],
-                                                   const RowsStrip (&T)[kStreams], int pitch, int lane) {
+__device__ __forceinline__ void rows_scatter_plain(const float4 rec, bool inr, const RowsStrip& strip, int pitch,
+                                                   int lane) {
   constexpr int NT = Stencil<INTERP>::NT;
-  int key[kStreams], base[kStreams];
-  bool act[kStreams], any_act = false;
-#pragma unroll
-  for (int s = 0; s < kStreams; ++s) {
-    key[s] = inr[s] ? __float_as_int(rec[s].w) : -1;
-    const int rel = (key[s] & 0x7fff) - T[s].ja;
-    act[s] = key[s] >= 0 && (unsigned)rel < (unsigned)T[s].wc;
-    base[s] = (key[s] >> 16) * pitch + rel;
-    any_act = any_act || act[s];
-  }
-  if (!__any_sync(0xffffffffu, any_act)) return;
-  float cc[kStreams][NT * NT];
-  bool lost = false;
-#pragma unroll
-  for (int s = 0; s < kStreams; ++s) {
-    rows_weights<INTERP>(rec[s], act[s], (key[s] & 0x8000) != 0, cc[s]);
-    if (act[s]) T[s].tag[base[s] & (kTagBytes - 1)] = (unsigned char)lane;
-  }
+  const int key = inr ? __float_as_int(rec.w) : -1;
+  const int rel = (key & 0x7fff) - strip.ja;
+  const bool act = key >= 0 && (unsigned)rel < (unsigned)strip.wc;
+  const int base = (key >> 16) * pitch + rel;
+  if (!__any_sync(0xffffffffu, act)) return;
+  float cc[NT * NT];
+  rows_weights<INTERP>(rec, act, (key & 0x8000) != 0, cc);
+  if (act) strip.tag[base & (kTagBytes - 1)] = (unsigned char)lane;
   __syncwarp();
-  bool writer[kStreams], lst[kStreams];
-#pragma unroll
-  for (int s = 0; s < kStreams; ++s) {
-    lst[s] = act[s] && T[s].tag[base[s] & (kTagBytes - 1)] != (unsigned char)lane;
-    lost = lost || lst[s];
-    writer[s] = act[s];
-  }
-  if (__any_sync(0xffffffffu, lost)) {
-#pragma unroll
-    for (int s = 0; s < kStreams; ++s) rows_resolve_pending<NT * NT>(act[s] ? base[s] : -1, lst[s], lane, cc[s], writer[s]);
-  }
-  float* q[kStreams];
-#pragma unroll
-  for (int s = 0; s < kStreams; ++s) q[s] = T[s].ring + (writer[s] ? base[s] : 0);
+  const bool lost = act && strip.tag[base & (kTagBytes - 1)] != (unsigned char)lane;
+  bool writer = act;
+  if (__any_sync(0xffffffffu, lost)) rows_resolve_pending<NT * NT>(act ? base : -1, lost, lane, cc, writer);
+  float* q = strip.ring + (writer ? base : 0);
 #pragma unroll
   for (int a = 0; a < NT; ++a) {
 #pragma unroll
     for (int b = 0; b < NT; ++b) {
-      float v[kStreams];
-#pragma unroll
-      for (int s = 0; s < kStreams; ++s) v[s] = writer[s] ? q[s][a * pitch + b] : 0.0f;
-#pragma unroll
-      for (int s = 0; s < kStreams; ++s)
-        if (writer[s]) q[s][a * pitch + b] = v[s] + cc[s][a * NT + b];
+      if (writer) q[a * pitch + b] += cc[a * NT + b];
       __syncwarp();
     }
   }
@@ -545,7 +503,6 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
           // budget allows (the kernel runs 1024 threads per SM at 64 registers)
           T* gu_row = core ? gu_pl + (long long)(y - S.out0) * W : nullptr;
           T* gv_row = core ? gv_pl + (long long)(y - S.out0) * W : nullptr;
-#if !defined(PSL_DBG_NOPRODUCE) && !defined(PSL_ROWS_NO_PAIRS)
           if (!EXACT && (kStepSub % 2) == 0) {
 #pragma unroll
             for (int j = 0; j < kStepSub; j += 2) {
@@ -567,27 +524,21 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
                 }
               }
             }
-          } else
-#endif
-          {
+          } else {
 #pragma unroll
-          for (int j = 0; j < kStepSub; ++j) {
-            if (xb + 32 * j < W) {                     // uniform: the last step of a row may be short
-              const int x = xb + 32 * j + lane;
-              float ou = 0.0f, ov = 0.0f;
-#ifdef PSL_DBG_NOPRODUCE
-              const float4 rec = make_float4(uu[j], vv[j], gg[j], __int_as_float(rows_key(hbase + rr, min(x, W - 1), false)));
-              ou = uu[j]; ov = vv[j];
-#else
-              const float4 rec = rows_point<EXACT, INTERP, PEER, false>(P, f, pl, mean0, mean1, sp, cp, y, min(x, W - 1), rr, hx,
-                                                                        hbase, ring, core, uu[j], vv[j], gg[j], ll[j], violated, ou, ov);
-#endif
-              if (x < W) {
-                recs[x] = rec;
-                if (core) { stcs_f(gu_row + x, ou); stcs_f(gv_row + x, ov); }
+            for (int j = 0; j < kStepSub; ++j) {
+              if (xb + 32 * j < W) {                   // uniform: the last step of a row may be short
+                const int x = xb + 32 * j + lane;
+                float ou = 0.0f, ov = 0.0f;
+                const float4 rec = rows_point<EXACT, INTERP, PEER, false>(P, f, pl, mean0, mean1, sp, cp, y, min(x, W - 1), rr,
+                                                                          hx, hbase, ring, core, uu[j], vv[j], gg[j], ll[j],
+                                                                          violated, ou, ov);
+                if (x < W) {
+                  recs[x] = rec;
+                  if (core) { stcs_f(gu_row + x, ou); stcs_f(gv_row + x, ov); }
+                }
               }
             }
-          }
           }
           if (last_step) {
             __syncwarp();
@@ -606,28 +557,23 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
 
   if (warp >= cons0 && warp < cons0 + S.nC) {
     // ==================================== consumers ====================================
-    const int cidx = warp - cons0;
+    const int cidx = warp - cons0;                         // strip of this warp
     const int pitch = S.pitch;
-    RowsStrip T[kStreams];
-    int sidx[kStreams];
-#pragma unroll
-    for (int q = 0; q < kStreams; ++q) {
-      sidx[q] = cidx * kStreams + q;                       // strips past the last one are empty (wc = 0)
-      const int ja = min(sidx[q] * S.wc, W);
-      T[q].ja = ja; T[q].wc = min(ja + S.wc, W) - ja;
-      const int slot = min(sidx[q], S.nS - 1);
-      T[q].ring = ring_base + (size_t)slot * S.ring_stride;
-      T[q].tag = smem_raw + S.off_tag + slot * kTagBytes;
+    RowsStrip strip;
+    {
+      const int ja = min(cidx * S.wc, W);                  // a strip past the last column would be empty (wc = 0)
+      strip.ja = ja; strip.wc = min(ja + S.wc, W) - ja;
+      const int slot = min(cidx, S.nS - 1);
+      strip.ring = ring_base + (size_t)slot * S.ring_stride;
+      strip.tag = smem_raw + S.off_tag + slot * kTagBytes;
     }
     int n = 0;
     while (rows_next_seg<INTERP>(P, S, g, g1, sg)) {
       float* gf_pl = P.gfield + (long long)sg.pl * S.outN * W;
       float* guard_pl = S.guard + (long long)sg.pl * S.outN * S.nS * (NT - 1);
-#pragma unroll
-      for (int q = 0; q < kStreams; ++q)
-        if (T[q].wc > 0)
-          for (int k = 4 * lane; k < S.ring_stride; k += 128)
-            *reinterpret_cast<float4*>(T[q].ring + k) = make_float4(0.f, 0.f, 0.f, 0.f);
+      if (strip.wc > 0)
+        for (int k = 4 * lane; k < S.ring_stride; k += 128)
+          *reinterpret_cast<float4*>(strip.ring + k) = make_float4(0.f, 0.f, 0.f, 0.f);
       __syncwarp();
       int head = 0;
       for (int y = sg.y_first; y <= sg.y_last; ++y) {
@@ -637,51 +583,34 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
           const float4* recs = rec_base + (size_t)rs * W;
           const int hx = __ldg(S.hx_tab + y);
           const bool fold_row = (y + OMIN - rr < 0) || (y + OMIN + rr + NT - 1 >= P.H);
-          // Lane l of stream q visits the records start_q + l * k + s, s = 0 .. k-1: the lanes of one step are
-          // k >= len / 32 columns apart, so two of them rarely share a departure cell (consecutive columns clash
-          // about twice per step with white-noise velocities; the records sit in shared memory, any order costs
-          // the same).  k not a multiple of 4: the ring accesses of a step then spread over the banks.
+          // Lane l visits the records start + l * k + s, s = 0 .. k-1: the lanes of one step are k >= len / 32
+          // columns apart, so two of them rarely share a departure cell (consecutive columns clash about twice per
+          // step with white-noise velocities; the records sit in shared memory, any order costs the same).  k not a
+          // multiple of 4: the ring accesses of a step then spread over the banks.
           int len = S.wc + 2 * hx;
           const bool whole = hx >= W || len >= W;
           if (whole) len = W;
           int k = (len + 31) >> 5;
           if ((k & 3) == 0) ++k;
-          int idx[kStreams];
-          bool inr[kStreams];
-          float4 rec[kStreams];
-#pragma unroll
-          for (int q = 0; q < kStreams; ++q) {
-            int start = whole ? 0 : T[q].ja - hx;
-            if (start < 0) start += W;
-            idx[q] = start + lane * k;                   // < 2 W + 32
-            if (idx[q] >= W) idx[q] -= W;
-            if (idx[q] >= W) idx[q] -= W;
-            inr[q] = lane * k < len && T[q].wc > 0;
-            rec[q] = inr[q] ? recs[idx[q]] : make_float4(0.f, 0.f, 0.f, __int_as_float(-1));
-          }
+          int start = whole ? 0 : strip.ja - hx;
+          if (start < 0) start += W;
+          int idx = start + lane * k;                      // < 2 W + 32
+          if (idx >= W) idx -= W;
+          if (idx >= W) idx -= W;
+          bool inr = lane * k < len && strip.wc > 0;
+          float4 rec = inr ? recs[idx] : make_float4(0.f, 0.f, 0.f, __int_as_float(-1));
           for (int s = 0; s < k; ++s) {
-            // fetch the next records before the ring updates of these (the compiler cannot move a shared-memory
+            // fetch the next record before the ring updates of this one (the compiler cannot move a shared-memory
             // load across them)
-            float4 nxt[kStreams];
-            bool inn[kStreams];
-#pragma unroll
-            for (int q = 0; q < kStreams; ++q) {
-              idx[q] = idx[q] + 1 == W ? 0 : idx[q] + 1;
-              inn[q] = (s + 1 < k) && (lane * k + s + 1 < len) && T[q].wc > 0;
-              nxt[q] = recs[idx[q]];                       // always a valid address; `inn` masks the key when it is used
-            }
-#ifndef PSL_DBG_NOCONSUME
-            if (fold_row) {
-#pragma unroll
-              for (int q = 0; q < kStreams; ++q)
-                rows_scatter_fold<INTERP>(W, P.H, rec[q], inr[q], T[q].ring, T[q].tag, pitch, ring, head, y, rr, T[q].ja,
-                                          T[q].wc, lane);
-            } else {
-              rows_scatter_plain<INTERP>(rec, inr, T, pitch, lane);
-            }
-#endif
-#pragma unroll
-            for (int q = 0; q < kStreams; ++q) { rec[q] = nxt[q]; inr[q] = inn[q]; }
+            idx = idx + 1 == W ? 0 : idx + 1;
+            const bool inn = (s + 1 < k) && (lane * k + s + 1 < len) && strip.wc > 0;
+            const float4 nxt = recs[idx];                  // always a valid address; `inn` masks the key when it is used
+            if (fold_row)
+              rows_scatter_fold<INTERP>(W, P.H, rec, inr, strip.ring, strip.tag, pitch, ring, head, y, rr, strip.ja,
+                                        strip.wc, lane);
+            else
+              rows_scatter_plain<INTERP>(rec, inr, strip, pitch, lane);
+            rec = nxt; inr = inn;
           }
           __syncwarp();
           if (lane == 0) mbar_arrive(&rec_free[rs]);
@@ -689,12 +618,10 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
         }
         // retire destination row i = y - rr + OMIN (slot `head`); slots 0 .. NT-2 first take in their alias rows
         const int i = y - rr + OMIN;
-#pragma unroll
-        for (int q = 0; q < kStreams; ++q) {
-          if (T[q].wc <= 0) continue;
-          float* row = T[q].ring + head * pitch;
+        if (strip.wc > 0) {
+          float* row = strip.ring + head * pitch;
           if (head < NT - 1) {
-            float* alias = T[q].ring + (ring + head) * pitch;
+            float* alias = strip.ring + (ring + head) * pitch;
             for (int k = 4 * lane; k < pitch; k += 128) {
               float4 a = *reinterpret_cast<const float4*>(row + k);
               const float4 b = *reinterpret_cast<const float4*>(alias + k);
@@ -705,15 +632,15 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
             __syncwarp();
           }
           if (i >= sg.ra && i < sg.rb) {
-            float* orow = gf_pl + (long long)(i - S.out0) * W + T[q].ja;
-            for (int k = 4 * lane; k < T[q].wc; k += 128)
+            float* orow = gf_pl + (long long)(i - S.out0) * W + strip.ja;
+            for (int k = 4 * lane; k < strip.wc; k += 128)
               __stcs(reinterpret_cast<float4*>(orow + k), *reinterpret_cast<const float4*>(row + k));
             if (lane < NT - 1)
-              guard_pl[((long long)(i - S.out0) * S.nS + sidx[q]) * (NT - 1) + lane] = row[T[q].wc + lane];
+              guard_pl[((long long)(i - S.out0) * S.nS + cidx) * (NT - 1) + lane] = row[strip.wc + lane];
           } else if (S.cut && i < sg.ra && i >= P.own0 && sg.ra > P.own0) {
             // cut mode, rows below the start cut: partial rows of the neighbouring segment (this segment's arrival rows
             // reach across the cut); the whole ring row, guard columns included, is parked for rows_grow_fix_kernel
-            rows_park_row(row, S.grow + ((((size_t)blockIdx.x * 2) * S.GR + (i - (sg.ra - S.GR))) * S.nS + sidx[q]) * pitch,
+            rows_park_row(row, S.grow + ((((size_t)blockIdx.x * 2) * S.GR + (i - (sg.ra - S.GR))) * S.nS + cidx) * pitch,
                           pitch, lane);
           }
           __syncwarp();
@@ -727,19 +654,17 @@ __global__ void __launch_bounds__(kRowsWarps * 32, 1) sl_bwd_rows_kernel(const P
         // above the cut (parked; rows outside the own window belong to a latitude neighbour or do not exist)
         for (int t = 0; t < ring - 1; ++t) {
           const int i = sg.y_last + 1 + t - rr + OMIN;
-#pragma unroll
-          for (int q = 0; q < kStreams; ++q) {
-            if (T[q].wc <= 0) continue;
+          if (strip.wc > 0) {
             // (a segment shorter than the ring still holds rows BELOW its start cut here)
             const bool own = i >= sg.ra && i < sg.rb;
-            float* orow = own ? gf_pl + (long long)(i - S.out0) * W + T[q].ja : nullptr;
-            float* gcol = own ? guard_pl + ((long long)(i - S.out0) * S.nS + sidx[q]) * (NT - 1) : nullptr;
+            float* orow = own ? gf_pl + (long long)(i - S.out0) * W + strip.ja : nullptr;
+            float* gcol = own ? guard_pl + ((long long)(i - S.out0) * S.nS + cidx) * (NT - 1) : nullptr;
             float* park = nullptr;
             if (i >= sg.rb && i < P.own0 + P.ownN)
-              park = S.grow + ((((size_t)blockIdx.x * 2 + 1) * S.GR + (i - sg.rb)) * S.nS + sidx[q]) * pitch;
+              park = S.grow + ((((size_t)blockIdx.x * 2 + 1) * S.GR + (i - sg.rb)) * S.nS + cidx) * pitch;
             else if (i < sg.ra && i >= P.own0 && sg.ra > P.own0)
-              park = S.grow + ((((size_t)blockIdx.x * 2) * S.GR + (i - (sg.ra - S.GR))) * S.nS + sidx[q]) * pitch;
-            rows_flush_row(T[q].ring, head, ring, pitch, T[q].wc, NT - 1, orow, gcol, park, lane);
+              park = S.grow + ((((size_t)blockIdx.x * 2) * S.GR + (i - (sg.ra - S.GR))) * S.nS + cidx) * pitch;
+            rows_flush_row(strip.ring, head, ring, pitch, strip.wc, NT - 1, orow, gcol, park, lane);
           }
           head = head + 1 == ring ? 0 : head + 1;
         }

@@ -27,23 +27,7 @@
 
 namespace psl {
 
-#ifndef PSL_SWEEP_WARPS
-#define PSL_SWEEP_WARPS 4
-#endif
-#if defined(PSL_SWEEP_MINB)
-#define PSL_SWEEP_BOUNDS __launch_bounds__(PSL_SWEEP_WARPS * 32, PSL_SWEEP_MINB)
-#elif defined(PSL_SWEEP_MAXREG)
-#define PSL_SWEEP_BOUNDS __maxnreg__(PSL_SWEEP_MAXREG)
-#else
-// 4 CTAs / SM for the 2x2 stencil (more resident warps measured slower: 2.19 -> 2.23 ms backward at 0.25 deg);
-// 6 CTAs / SM = 80 registers for 4x4, where a fourth row band of resident tasks pays for the few spills
-// (4.54 -> 3.98 ms)
-#define PSL_SWEEP_BOUNDS __launch_bounds__(PSL_SWEEP_WARPS * 32, INTERP == 2 ? 6 : 4)
-#endif
-#ifndef PSL_TOUCH_ON
-#define PSL_TOUCH_ON(NT) ((NT) == 2)      // the 4x4 kernel is register-bound at 80: touches cost it more than they save
-#endif
-constexpr int kSweepWarps = PSL_SWEEP_WARPS;
+constexpr int kSweepWarps = 4;
 constexpr int kMaxBands = 48;
 
 constexpr int kTagRows = 4;                   // clash tags cover (slot mod kTagRows, column)
@@ -77,7 +61,6 @@ struct SweepPlan {
   int out0, outN;                             // rows held by the output tensors (global first row, count)
 };
 
-#define PSL_HAVE_RESOLVE_CLASHES 1
 template <int NT>
 __device__ __forceinline__ void resolve_clashes(int key, int tkey, unsigned char* tag, int lane,
                                                 float (&c)[NT * NT], bool& writer) {
@@ -148,13 +131,11 @@ __device__ __forceinline__ void sweep_compute(const Params& P, const SweepRow<T>
   if (CORE) {
     // every arrival point a task sees in its own columns is checked against the contract
     if (!in_ring || dx < -R.hx || dx > R.hx - NT + 1) violated = true;
-#ifndef PSL_DBG_NOGRADS
     if (R.gu_row) {
       float val, ddx, ddy;
       stencil_eval<INTERP, true, PEER>(P, f, pl, t, mean0, mean1, val, ddx, ddy);
       velocity_grads<EXACT>(P, t, R.sp, R.cp, g * ddx, g * ddy, ou, ov);
     }
-#endif
   }
   const int cidx = (x - ja) + dx + kRingLead;    // ring column of tap 0
   const bool hit = in_ring && (unsigned)(cidx - (kRingLead - NT + 1)) <= (unsigned)(wc + NT - 2);
@@ -186,14 +167,7 @@ template <int NT>
 __device__ __forceinline__ void sweep_scatter(StepOut<NT>& o, float* acc, unsigned char* tag, int ring, int pitch,
                                               int lane) {
   bool writer;
-#ifdef PSL_DBG_NOSCATTER
-  if (o.key != -12345) return;
-#endif
-#ifdef PSL_DBG_NOCLASH
-  writer = o.key >= 0;
-#else
   resolve_clashes<NT>(o.key, (o.slot0 & (kTagRows - 1)) * pitch + o.cidx, tag, lane, o.cc, writer);
-#endif
   if (NT == 2) {
     float* r0 = acc + (writer ? o.key : 0);
     float* r1 = acc + o.off1;
@@ -221,8 +195,11 @@ __device__ __forceinline__ void sweep_scatter(StepOut<NT>& o, float* acc, unsign
   }
 }
 
+// 4 CTAs / SM for the 2x2 stencil (more resident warps measured slower: 2.19 -> 2.23 ms backward at 0.25 deg);
+// 6 CTAs / SM = 80 registers for 4x4, where a fourth row band of resident tasks pays for the few spills
+// (4.54 -> 3.98 ms)
 template <bool EXACT, int INTERP, bool PEER, typename T>
-__global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const SweepPlan S) {
+__global__ void __launch_bounds__(kSweepWarps * 32, INTERP == 2 ? 6 : 4) sl_bwd_sweep_kernel(const Params P, const SweepPlan S) {
   constexpr int NT = Stencil<INTERP>::NT, OMIN = Stencil<INTERP>::OMIN;
   extern __shared__ __align__(16) float smem[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -262,8 +239,9 @@ __global__ void PSL_SWEEP_BOUNDS sl_bwd_sweep_kernel(const Params P, const Sweep
   // row step will need -- u, v, grad_out of the next arrival row and the field row that enters the stencil
   // window with it -- over the columns [ja - 64, ja + 192).  The value is only consumed at the end of the row
   // step, so the load never stalls; it replaces ~3.4k stall cycles per row on first-touch L2 / DRAM latency
-  // (`prefetch.global.L1` did not have that effect).  Measured 2.19 -> 2.07 ms backward at 0.25 deg.
-  constexpr bool kTouch = PSL_TOUCH_ON(NT);
+  // (`prefetch.global.L1` did not have that effect).  Measured 2.19 -> 2.07 ms backward at 0.25 deg.  The 4x4 kernel
+  // is register-bound at 80: touches cost it more than they save.
+  constexpr bool kTouch = NT == 2;
   const int pf_arr = lane >> 3;
   int pf_col = ja - 64 + ((lane & 7) << 5);
   if (pf_col < 0) pf_col += W; else if (pf_col >= W) pf_col -= W;

@@ -107,10 +107,8 @@ def row_costs(H: int, W: int, cfl_cells: float, strip: int = 240, base: float = 
     with (csrc/paradis_sl.cu, launch_rows): a constant for the producers plus the number of 32-record steps a
     consumer scans for the row -- its strip plus the longitudinal reach of the row either side, which grows as
     1 / cos(lat) and becomes the whole circle next to the poles."""
-    import os
     if base is None:      # the forward and the producers: about 2.5 scan steps' worth of time per row at C3
-        base = float(os.environ.get("PARADIS_SL_BAND_BASE", "2.5"))
-    capw = float(os.environ.get("PARADIS_SL_BAND_CAPW", "1.0"))     # weight of the rows that scan the whole circle
+        base = 2.5
     dphi = math.pi / max(H - 1, 1)
     delta = cfl_cells * dphi
     out = []
@@ -122,7 +120,7 @@ def row_costs(H: int, W: int, cfl_cells: float, strip: int = 240, base: float = 
             if sdl < 1.0:
                 cells = min(W, math.asin(sdl) / (2 * math.pi / W) + 4)
         scan = min(W, strip + 2 * cells)
-        out.append(base + math.ceil(scan / 32) * (capw if scan >= W else 1.0))
+        out.append(base + math.ceil(scan / 32))
     return out
 
 
@@ -138,9 +136,8 @@ def make_plan(H: int, W: int, rank: int, world: int, cfl_cells: float, interpola
     that own a polar cap)."""
     halo = halo_rows(cfl_cells, interpolation)
     if balance and world > 1:
-        import os
         # (CTAs + planes) / planes segments per plane, each re-playing ring - 1 = 2 ceil(cfl) + stencil rows - 1 rows
-        warm = float(os.environ.get("PARADIS_SL_BAND_WARM", 3.0 * (2 * math.ceil(cfl_cells) + STENCIL_ROWS[interpolation] - 1)))
+        warm = 3.0 * (2 * math.ceil(cfl_cells) + STENCIL_ROWS[interpolation] - 1)
         try:
             bands = band_rows(H, world, row_costs(H, W, cfl_cells), warm, halo + 1)
         except ValueError:

@@ -10,7 +10,7 @@ import subprocess
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-W0 = 4      # PARADIS_SL_ROWS_W0 default (sl_partition.cuh)
+W0 = 4      # kRowW0 (sl_partition.cuh)
 
 # interp H W planes own0 ownN arr0 arrN cfl cut grid consumers
 SHAPES = [
@@ -42,8 +42,7 @@ def harness(tmp_path_factory):
 
 def run(exe, shapes):
     text = "\n".join(" ".join(str(v) for v in s) for s in shapes) + "\n"
-    env = {k: v for k, v in os.environ.items() if not k.startswith("PARADIS_SL_")}
-    res = subprocess.run([exe], input=text, capture_output=True, text=True, env=env, timeout=120)
+    res = subprocess.run([exe], input=text, capture_output=True, text=True, timeout=120)
     assert res.returncode == 0, res.stderr[-2000:]
     out = [json.loads(line) for line in res.stdout.splitlines() if line.startswith("{")]
     assert len(out) == len(shapes)

@@ -94,8 +94,7 @@ def times():
         R = RawAdvection(geo, B, V, interp, True, "fast", 6.0)
         tf = timeit(lambda: R.forward(f, u, v, DT))
         tb = timeit(lambda: R.backward(g, f, u, v, DT, 3))
-        print(f"TIME C3 {interp} nc={os.environ.get('PARADIS_SL_ROWS_NC','-')} mode={os.environ.get('PARADIS_SL_BWD','0')} "
-              f"lib={os.path.basename(os.environ.get('PARADIS_SL_LIB','default'))}: fwd {tf:.3f} ms "
+        print(f"TIME C3 {interp} lib={os.path.basename(os.environ.get('PARADIS_SL_LIB','default'))}: fwd {tf:.3f} ms "
               f"({16*pts/tf/1e6:.0f} GB/s) bwd {tb:.3f} ms ({28*pts/tb/1e6:.0f} GB/s) step {tf+tb:.3f} ms", flush=True)
     P.check_status()
 
