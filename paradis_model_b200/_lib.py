@@ -1,5 +1,6 @@
 """ctypes binding of the C ABI declared in include/paradis_sl.h (and the bf16 entry points of
-include/paradis_sl_bf16.h, include/paradis_geocyclic.h and include/paradis_sl_tl.h, each in a table of its own).
+include/paradis_sl_bf16.h, include/paradis_geocyclic.h, include/paradis_sl_tl.h and the float64 entry points of
+include/paradis_sl_f64.h, each in a table of its own).
 
 The product has no CPU fallback: if the shared library is missing this module
 raises, it never substitutes another implementation.
@@ -31,6 +32,13 @@ class Geom(C.Structure):
                 ("fld_row0", C.c_int32), ("fld_rows", C.c_int32),
                 ("fld_peer_lo", C.c_void_p), ("fld_peer_hi", C.c_void_p), ("fld_peer_rows", C.c_int32),
                 ("arr_peer_lo", C.c_void_p * 3), ("arr_peer_hi", C.c_void_p * 3), ("arr_peer_rows", C.c_int32)]
+
+
+class GeomF64(C.Structure):
+    """struct paradis_sl_geom_f64 (full mesh, double tables and scalars)"""
+    _fields_ = [("H", C.c_int32), ("W", C.c_int32),
+                ("sin_lat", C.c_void_p), ("cos_lat", C.c_void_p), ("lon", C.c_void_p),
+                ("min_lat", C.c_double), ("d_lat", C.c_double), ("min_lon", C.c_double), ("d_lon", C.c_double)]
 
 
 _lib = None
@@ -99,6 +107,30 @@ _PROTOS_TL = {
 }
 
 
+# include/paradis_sl_f64.h: float64 storage and arithmetic (same ABI version: entry points added)
+_I, _D, _G64 = C.c_int, C.c_double, C.POINTER(GeomF64)
+_PROTOS_F64 = {
+    "paradis_sl_advect_fwd_f64_workspace": (C.c_size_t, [_I, _I]),
+    "paradis_sl_advect_fwd_f64": (_I, [_G64, _P, _P, _P, _P, _I, _I, C.c_int64, C.c_int64, C.c_int64, _D, _I, _I, _I,
+                                       _P, C.c_size_t, _P, _P]),
+    "paradis_sl_advect_bwd_f64_workspace": (C.c_size_t, [_I, _I, _I, _I]),
+    "paradis_sl_advect_bwd_f64": (_I, [_G64, _P, _P, _P, _P, _P, _P, _P, _I, _I, C.c_int64, C.c_int64, C.c_int64,
+                                       C.c_int64, _D, _I, _I, _I, _P, C.c_size_t, _P, _P]),
+    "paradis_sl_advect_jvp_f64_workspace": (C.c_size_t, [_I, _I]),
+    "paradis_sl_advect_jvp_f64": (_I, [_G64, _P, _P, _P, _P, _P, _P, _P, _I, _I, C.c_int64, C.c_int64, C.c_int64,
+                                       C.c_int64, C.c_int64, C.c_int64, _D, _I, _I, _I, _P, C.c_size_t, _P, _P]),
+    "paradis_sl_departure_coords_f64": (_I, [_G64, _P, _P, _P, _I, _I, C.c_int64, C.c_int64, _D, _I, _I, _P]),
+    "paradis_geocyclic_pad_fwd_f64": (_I, [_P, _P, C.c_int64, _I, _I, _I, _P]),
+    "paradis_geocyclic_pad_bwd_f64": (_I, [_P, _P, C.c_int64, _I, _I, _I, _P]),
+    "paradis_geocyclic_dwconv_fwd_f64": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "paradis_geocyclic_dwconv_bwd_input_f64": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
+    "paradis_geocyclic_dwconv_wgrad_f64_workspace": (C.c_size_t, [_I, _I, _I, _I, _I]),
+    "paradis_geocyclic_dwconv_bwd_weight_f64": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _P, C.c_size_t, _P]),
+    "paradis_geocyclic_avgpool5_fwd_f64": (_I, [_P, _P, _I, _I, _I, _I, _I, _P]),
+    "paradis_geocyclic_avgpool5_bwd_f64": (_I, [_P, _P, _I, _I, _I, _I, _I, _P]),
+}
+
+
 def exported_symbols():
     """The functions of include/paradis_sl.h."""
     return list(_PROTOS)
@@ -117,6 +149,11 @@ def exported_symbols_geocyclic():
 def exported_symbols_tl():
     """The functions of include/paradis_sl_tl.h."""
     return list(_PROTOS_TL)
+
+
+def exported_symbols_f64():
+    """The functions of include/paradis_sl_f64.h."""
+    return list(_PROTOS_F64)
 
 
 def lib():
@@ -146,7 +183,7 @@ def lib():
                 pass
         handle = C.CDLL(path)
         for name, (res, args) in (list(_PROTOS.items()) + list(_PROTOS_BF16.items()) + list(_PROTOS_GEO.items())
-                           + list(_PROTOS_TL.items())):
+                           + list(_PROTOS_TL.items()) + list(_PROTOS_F64.items())):
             fn = getattr(handle, name)
             fn.restype, fn.argtypes = res, args
         if handle.paradis_sl_abi_version() != 2 and not os.environ.get("PARADIS_SL_SKIP_ABI_CHECK"):

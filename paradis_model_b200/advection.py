@@ -17,7 +17,7 @@ general path on the device.
 """
 import torch
 
-from .ops import SLGeometry, pack_tables, sl_advect
+from .ops import SLGeometry, pack_tables, pack_tables64, sl_advect
 from .padding import GeoCyclicPadding
 from .projection import resolve_block_factory
 
@@ -66,8 +66,12 @@ class NeuralSemiLagrangian(torch.nn.Module):
         reg("d_lon", self.max_lon - self.min_lon)
         reg("d_lat", self.max_lat - self.min_lat)
         reg("sl_tables", torch.empty(0))
+        reg("sl_tables64", torch.empty(0, dtype=torch.float64))
         self._scalars = [float(self.min_lat.float()), float(self.d_lat.float()),
                          float(self.min_lon.float()), float(self.d_lon.float())]
+        # float64 inputs: the buffers as they are (the reference computes d_lat / d_lon here in the grids' dtype, and
+        # .double() only converts them)
+        self._scalars64 = [float(self.min_lat), float(self.d_lat), float(self.min_lon), float(self.d_lon)]
         self._refresh_tables()
 
     def _refresh_tables(self):
@@ -76,6 +80,8 @@ class NeuralSemiLagrangian(torch.nn.Module):
         lat = self.lat_grid[0, 0, :, 0].float()
         lon = self.lon_grid[0, 0, 0, :].float()
         self.sl_tables = pack_tables(lat, lon)
+        # float64 inputs: the same with torch's fp64 kernels from the grids' own values (the reference after .double())
+        self.sl_tables64 = pack_tables64(self.lat_grid[0, 0, :, 0], self.lon_grid[0, 0, 0, :])
 
     def _apply(self, fn, *args, **kwargs):
         out = super()._apply(fn, *args, **kwargs)
@@ -84,7 +90,7 @@ class NeuralSemiLagrangian(torch.nn.Module):
 
     def geometry(self) -> SLGeometry:
         H, W = self.mesh_size
-        return SLGeometry(self.sl_tables, self._scalars, H, W)
+        return SLGeometry(self.sl_tables, self._scalars, H, W, tables64=self.sl_tables64, scalars64=self._scalars64)
 
     def forward(self, hidden_features: torch.Tensor, u: torch.Tensor, v: torch.Tensor, dt: float) -> torch.Tensor:
         """Compute advection using rotated coordinate system."""

@@ -13,10 +13,12 @@ SOURCES = [os.path.join(_HERE, "csrc", "paradis_sl.cu"), os.path.join(_HERE, "cs
 HEADERS = [os.path.join(_HERE, "csrc", "sl_device.cuh"), os.path.join(_HERE, "csrc", "sl_sweep.cuh"),
            os.path.join(_HERE, "csrc", "sl_partition.cuh"),
            os.path.join(_HERE, "csrc", "sl_rows.cuh"), os.path.join(_HERE, "csrc", "sl_tangent.cuh"),
+           os.path.join(_HERE, "csrc", "sl_f64.cuh"), os.path.join(_HERE, "csrc", "geo_f64.cuh"),
            os.path.join(_HERE, "..", "include", "paradis_sl.h"),
            os.path.join(_HERE, "..", "include", "paradis_sl_tl.h"),
            os.path.join(_HERE, "..", "include", "paradis_sl_bf16.h"),
-           os.path.join(_HERE, "..", "include", "paradis_geocyclic.h")]
+           os.path.join(_HERE, "..", "include", "paradis_geocyclic.h"),
+           os.path.join(_HERE, "..", "include", "paradis_sl_f64.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-shared", "-Xcompiler", "-fPIC"]
 

@@ -439,3 +439,6 @@ extern "C" int paradis_geocyclic_avgpool5_bwd_bf16(const void* gy, void* gx, int
                                                    void* stream) {
   return avgpool5<bf16>(true, (const bf16*)gy, (bf16*)gx, B, C, H, W, stride, stream);
 }
+
+// float64 storage and arithmetic (include/paradis_sl_f64.h)
+#include "geo_f64.cuh"

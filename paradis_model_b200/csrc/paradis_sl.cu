@@ -13,6 +13,7 @@
 //                          covers it (inverse stencils), fixed order, no atomics
 //   geocyclic_pad_{fwd,bwd}_kernel  standalone padding op and its adjoint
 //   sl_tl_kernel           tangent-linear model: d out along (dfield, du, dv), one gather per point (sl_tangent.cuh)
+//   *_f64_kernel           float64 storage and arithmetic, full mesh (sl_f64.cuh)
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -1477,3 +1478,8 @@ extern "C" int paradis_sl_advect_jvp(const paradis_sl_geom* geom, const float* f
   if (pole_fix) pole_rows_fix_kernel<<<planes * 2, kPoleThreads, 0, st>>>(dout, P.ownN, P.own0, P.H, P.W, planes);
   return check_launch("paradis_sl_advect_jvp");
 }
+
+// ---------------------------------------------------------------------------------------------
+// float64 (include/paradis_sl_f64.h)
+// ---------------------------------------------------------------------------------------------
+#include "sl_f64.cuh"

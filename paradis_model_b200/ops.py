@@ -1,10 +1,10 @@
 """torch.library custom ops over the C ABI (include/paradis_sl.h).
 
 Ops (namespace ``paradis``)
-    sl_advect / sl_advect_backward      model/advection.py:129-169, fused
+    sl_advect / sl_advect_backward(_bf16, _f64)   model/advection.py:129-169, fused
     sl_advect_jvp                        its tangent-linear model (forward-mode AD), fused
     geocyclic_pad / geocyclic_pad_backward   model/padding.py:11-39
-    geocyclic_dwconv / geocyclic_dwconv_backward(_bf16)   SepConv's pad + depthwise conv, model/blocks.py:112-114
+    geocyclic_dwconv / geocyclic_dwconv_backward(_bf16, _f64)   SepConv's pad + depthwise conv, model/blocks.py:112-114
     geocyclic_avgpool5 / geocyclic_avgpool5_backward      PhysicalDownsample, model/blocks.py:57-71
 
 Each op has a fake (meta) implementation and an autograd formula, so it works under
@@ -18,7 +18,7 @@ tangent-linear kernel on the full mesh; the GeoCyclic ops: compositions of their
 op is called directly, as before.  vmap / jacfwd over a tangent, forward-over-reverse and tangents on latitude-band
 geometries raise NotImplementedError.
 
-Storage types of sl_advect.  The arithmetic is always fp32 (torch's own autocast policy runs
+Storage types of sl_advect.  The arithmetic is fp32 except for float64 (below) (torch's own autocast policy runs
 grid_sampler / asin / atan2 in fp32) and ``out`` is fp32.  When field, u and v are all bf16 (what
 autocast hands the op: down_projection and velocity_net outputs) on the full mesh, with W % 8 == 0,
 16-byte aligned bases and batch strides in multiples of 8 elements, the kernels read them as bf16 and
@@ -33,6 +33,15 @@ bf16 weight of C * k * k elements is upcast) and so do grad weight / grad bias. 
 fp32 kernels run on ``.float()`` copies with the outputs cast back by ``.to(torch.bfloat16)``.  fp16, fp32 and
 mixed-dtype calls take the fp32 kernels (on fp32 copies where needed).  ``NATIVE_BF16 = False`` forces the upcast path
 for these ops as well.
+
+float64 (include/paradis_sl_f64.h).  If any of field, u, v is float64, sl_advect upcasts the others and computes in
+double with the reference's op order (IEEE double, one rounding per torch op, libdevice's double transcendentals): the
+departure coordinates are bit-identical to the reference's ops run by torch-CUDA in float64, and out, the gradients
+(``paradis::sl_advect_backward_f64``) and the tangent (``paradis::sl_advect_jvp``) are float64.  It uses the
+geometry's float64 tables (``SLGeometry.tables64``); ``math`` does not change the result and ``cfl_cells`` is not used.
+Full mesh only: a latitude-band geometry raises.  The GeoCyclic ops read and write a float64 input as double, with
+weight and bias in double and float64 gradients (``paradis::geocyclic_dwconv_backward_f64``); the padding is exact.
+``departure_coords`` returns double coordinates for a float64 u or v.
 """
 from __future__ import annotations
 
@@ -124,6 +133,17 @@ def pack_tables(lat: Tensor, lon: Tensor) -> Tensor:
     return t
 
 
+def pack_tables64(lat: Tensor, lon: Tensor) -> Tensor:
+    """[sin(lat) | cos(lat) | lon] in float64 (layout of pack_tables): sin/cos run as torch fp64 kernels on the device
+    of ``lat``, what the reference evaluates after ``.double()``."""
+    H, Hp = lat.numel(), _hpad(lat.numel())
+    t = torch.zeros(2 * Hp + lon.numel(), dtype=torch.float64, device=lat.device)
+    t[:H] = torch.sin(lat.double())
+    t[Hp:Hp + H] = torch.cos(lat.double())
+    t[2 * Hp:] = lon.double()
+    return t
+
+
 class SLGeometry:
     """Separable mesh geometry: what model/advection.py:56-72 registers as buffers.
 
@@ -134,13 +154,18 @@ class SLGeometry:
     full mesh by default), optionally followed by [peer_lo_ptr, peer_hi_ptr, peer_rows]: device
     addresses of the latitude neighbours' boundary rows of `field` (NVLink peer memory, see
     include/paradis_sl.h) which the kernels then read in place instead of an assembled halo.
+    ``tables64`` / ``scalars64`` = the same in float64 (``pack_tables64``; the scalars as the module's buffers hold
+    them), used when an input of sl_advect is float64; None where the geometry was built without them.
     """
 
-    def __init__(self, tables: Tensor, scalars: List[float], H: int, W: int, windows=None):
+    def __init__(self, tables: Tensor, scalars: List[float], H: int, W: int, windows=None,
+                 tables64: Optional[Tensor] = None, scalars64: Optional[List[float]] = None):
         self.tables = tables
         self.scalars = [float(s) for s in scalars]
         self.H, self.W = int(H), int(W)
         self.windows = list(windows) if windows is not None else [self.H, self.W, 0, self.H, 0, self.H, 0, self.H]
+        self.tables64 = tables64
+        self.scalars64 = [float(s) for s in scalars64] if scalars64 is not None else None
 
     @staticmethod
     def separable(lat_grid: Tensor, lon_grid: Tensor) -> bool:
@@ -162,10 +187,16 @@ class SLGeometry:
         lat_min, lat_max = lat.min(), lat.max()
         lon_min, lon_max = lon.min(), lon.max()
         scalars = [lat_min.item(), (lat_max - lat_min).item(), lon_min.item(), (lon_max - lon_min).item()]
-        return cls(tables, scalars, H, W)
+        # float64: tables from the grids' own values, scalars computed in the grids' dtype (what the reference
+        # registers at construction; .double() only converts them)
+        lat0, lon0 = lat_grid[:, 0], lon_grid[0, :]
+        scalars64 = [lat0.min().item(), (lat0.max() - lat0.min()).item(), lon0.min().item(),
+                     (lon0.max() - lon0.min()).item()]
+        return cls(tables, scalars, H, W, tables64=pack_tables64(lat0, lon0), scalars64=scalars64)
 
     def to(self, device) -> "SLGeometry":
-        return SLGeometry(self.tables.to(device), self.scalars, self.H, self.W, self.windows)
+        return SLGeometry(self.tables.to(device), self.scalars, self.H, self.W, self.windows,
+                          self.tables64.to(device) if self.tables64 is not None else None, self.scalars64)
 
     def band(self, own: Tuple[int, int], arr: Tuple[int, int], fld: Tuple[int, int], peer=None,
              arr_peer=None) -> "SLGeometry":
@@ -177,7 +208,7 @@ class SLGeometry:
             w += [int(peer[0]), int(peer[1]), int(peer[2])] if peer is not None else [0, 0, 0]
         if arr_peer is not None:
             w += [int(p) for p in arr_peer[0]] + [int(p) for p in arr_peer[1]] + [int(arr_peer[2])]
-        return SLGeometry(self.tables, self.scalars, self.H, self.W, w)
+        return SLGeometry(self.tables, self.scalars, self.H, self.W, w, self.tables64, self.scalars64)
 
 
 def _geom_struct(tables: Tensor, scalars: List[float], windows: List[int]) -> _lib.Geom:
@@ -199,6 +230,31 @@ def _geom_struct(tables: Tensor, scalars: List[float], windows: List[int]) -> _l
             g.arr_peer_hi[k] = int(windows[14 + k]) or None
         g.arr_peer_rows = int(windows[17])
     return g
+
+
+def _geom64_struct(tables: Tensor, scalars: List[float], windows: List[int]) -> _lib.GeomF64:
+    H, W = int(windows[0]), int(windows[1])
+    Hp = _hpad(H)
+    if tables.dtype != torch.float64 or tables.numel() != 2 * Hp + W or not tables.is_contiguous():
+        raise RuntimeError("paradis_sl: float64 inputs need the geometry's float64 tables (pack_tables64(), "
+                           "SLGeometry.tables64)")
+    base = tables.data_ptr()
+    g = _lib.GeomF64()
+    g.H, g.W = H, W
+    g.sin_lat, g.cos_lat, g.lon = base, base + 8 * Hp, base + 16 * Hp
+    g.min_lat, g.d_lat, g.min_lon, g.d_lon = scalars
+    return g
+
+
+def _is_f64(*tensors) -> bool:
+    """The float64 path: any input is float64 (the others are upcast).  Decided from dtypes only."""
+    return any(t is not None and t.dtype == torch.float64 for t in tensors)
+
+
+def _f64_full_mesh(windows: List[int], what: str) -> None:
+    if not _full_mesh(windows):
+        raise RuntimeError(f"{what}: float64 works on the full mesh only; latitude bands (and their peer halos) "
+                           "are fp32 / bf16")
 
 
 def _held_arr_rows(windows: List[int]) -> int:
@@ -238,6 +294,11 @@ def _geo_bf16(*tensors: Tensor) -> bool:
     """Native bf16 storage of the GeoCyclic ops: every large tensor is bf16.  Decided from dtypes only (call time, safe
     in traced code)."""
     return NATIVE_BF16 and all(t.dtype == torch.bfloat16 for t in tensors)
+
+
+def _geo_sfx(t: Tensor) -> str:
+    """Entry-point suffix of the GeoCyclic kernels that read and write t's dtype in place (bf16 or float64)."""
+    return "_f64" if t.dtype == torch.float64 else "_bf16"
 
 
 def _bf16_layout_ok(bf: List[Tensor], f32: List[Tensor]) -> bool:
@@ -300,13 +361,24 @@ def _sl_advect(field: Tensor, u: Tensor, v: Tensor, tables: Tensor, scalars: Lis
                interp: int, pole_fix: bool, math: int, windows: List[int], cfl: float) -> Tensor:
     B, V, H, W, ownN, arrN = _check_inputs(field, u, v, windows)
     L = _lib.lib()
-    if field.dtype == torch.float64 or u.dtype == torch.float64 or v.dtype == torch.float64:
-        raise RuntimeError("paradis::sl_advect computes in fp32 (like the reference under its fp32 / bf16-mixed settings); "
-                           "float64 inputs would silently lose precision -- cast them explicitly")
     poll_status(field.device)
     if tables.device != field.device:
         raise RuntimeError(f"paradis::sl_advect: geometry tables live on {tables.device}, the tensors on {field.device}; "
                            "move the geometry with SLGeometry.to(device)")
+    if _is_f64(field, u, v):
+        _f64_full_mesh(windows, "paradis::sl_advect")
+        field, u, v = [_inner_contig(t.double()) for t in (field, u, v)]
+        out = torch.empty((B, V, ownN, W), dtype=torch.float64, device=field.device)
+        g = _geom64_struct(tables, scalars, windows)
+        ws_bytes = L.paradis_sl_advect_fwd_f64_workspace(B, V)
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=field.device)
+        with torch.cuda.device(field.device):
+            rc = L.paradis_sl_advect_fwd_f64(C.byref(g), _ptr(field), _ptr(u), _ptr(v), _ptr(out), B, V,
+                                             field.stride(0), u.stride(0), v.stride(0), dt, interp, int(pole_fix),
+                                             math, _ptr(ws), ws_bytes, _ptr(_status_word(field.device)),
+                                             _stream(field))
+        _lib.check(rc, "paradis_sl_advect_fwd_f64")
+        return out
     native = _bf16_candidate((field.dtype, u.dtype, v.dtype), windows)
     if native:
         field, u, v = _inner_contig(field), _inner_contig(u), _inner_contig(v)
@@ -331,7 +403,7 @@ def _sl_advect(field: Tensor, u: Tensor, v: Tensor, tables: Tensor, scalars: Lis
 @_sl_advect.register_fake
 def _(field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl):
     B, V = field.shape[:2]
-    return field.new_empty((B, V, windows[3], windows[1]), dtype=torch.float32)
+    return field.new_empty((B, V, windows[3], windows[1]), dtype=torch.float64 if _is_f64(field, u, v) else torch.float32)
 
 
 def _backward_impl(grad_out: Tensor, field: Tensor, u: Tensor, v: Tensor, tables: Tensor, scalars: List[float],
@@ -417,6 +489,48 @@ def _(grad_out, field, u, v, tables, scalars, dt, interp, pole_fix, math, window
     return (full() if need_field else none(), full() if need_uv else none(), full() if need_uv else none())
 
 
+@torch.library.custom_op("paradis::sl_advect_backward_f64", mutates_args=(), device_types="cuda")
+def _sl_advect_backward_f64(grad_out: Tensor, field: Tensor, u: Tensor, v: Tensor, tables: Tensor,
+                            scalars: List[float], dt: float, interp: int, pole_fix: bool, math: int,
+                            windows: List[int], need_field: bool, need_uv: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """Backward of sl_advect in float64 (include/paradis_sl_f64.h): float64 gradients, every input upcast to double.
+    The per-point kernel and the deterministic gather; the fused sweeps are fp32 / bf16 only, so there is no cfl
+    hint."""
+    B, V, H, W, ownN, arrN = _check_inputs(field, u, v, windows)
+    _f64_full_mesh(windows, "paradis::sl_advect_backward_f64")
+    dev = field.device
+    poll_status(dev)
+    if tables.device != dev:
+        raise RuntimeError(f"paradis::sl_advect_backward_f64: geometry tables live on {tables.device}, the tensors on {dev}")
+    grad_out, field, u, v = [_inner_contig(t.double()) for t in (grad_out, field, u, v)]
+    if tuple(grad_out.shape) != tuple(u.shape):
+        raise RuntimeError("paradis::sl_advect_backward_f64: grad_out must have the shape of u and v")
+    L = _lib.lib()
+    full = lambda: torch.empty((B, V, ownN, W), dtype=torch.float64, device=dev)
+    none = lambda: torch.empty(0, dtype=torch.float64, device=dev)
+    gf = full() if need_field else None
+    gu, gv = (full(), full()) if need_uv else (None, None)
+    g = _geom64_struct(tables, scalars, windows)
+    ws_bytes = L.paradis_sl_advect_bwd_f64_workspace(B, V, H, W)
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        rc = L.paradis_sl_advect_bwd_f64(C.byref(g), _ptr(grad_out), _ptr(field), _ptr(u), _ptr(v), _ptr(gf), _ptr(gu),
+                                         _ptr(gv), B, V, grad_out.stride(0), field.stride(0), u.stride(0), v.stride(0),
+                                         dt, interp, int(pole_fix), math, _ptr(ws), ws_bytes, _ptr(_status_word(dev)),
+                                         _stream(field))
+    _lib.check(rc, "paradis_sl_advect_bwd_f64")
+    return (gf if need_field else none(), gu if need_uv else none(), gv if need_uv else none())
+
+
+@_sl_advect_backward_f64.register_fake
+def _(grad_out, field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, need_field, need_uv):
+    B, V = field.shape[:2]
+    shape = (B, V, windows[3], windows[1])
+    full = lambda: field.new_empty(shape, dtype=torch.float64)
+    none = lambda: field.new_empty((0,), dtype=torch.float64)
+    return (full() if need_field else none(), full() if need_uv else none(), full() if need_uv else none())
+
+
 def _sl_setup(ctx, inputs, output):
     field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl = inputs
     ctx.save_for_backward(field, u, v, tables)
@@ -433,11 +547,15 @@ def _sl_backward(ctx, grad_out):
                            "use paradis_model_b200.halo.LatBandAdvection")
     need_field = ctx.needs_input_grad[0]
     need_uv = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
-    # bf16 inputs on the full mesh: bf16 gradients straight from the kernels (no fp32 copies, no casts)
-    bwd = (torch.ops.paradis.sl_advect_backward_bf16 if _bf16_candidate(ctx.dtypes, windows)
-           else torch.ops.paradis.sl_advect_backward)
-    gf, gu, gv = bwd(grad_out, field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl, need_field,
-                     need_uv)
+    if torch.float64 in ctx.dtypes:
+        gf, gu, gv = torch.ops.paradis.sl_advect_backward_f64(grad_out, field, u, v, tables, scalars, dt, interp,
+                                                              pole_fix, math, windows, need_field, need_uv)
+    else:
+        # bf16 inputs on the full mesh: bf16 gradients straight from the kernels (no fp32 copies, no casts)
+        bwd = (torch.ops.paradis.sl_advect_backward_bf16 if _bf16_candidate(ctx.dtypes, windows)
+               else torch.ops.paradis.sl_advect_backward)
+        gf, gu, gv = bwd(grad_out, field, u, v, tables, scalars, dt, interp, pole_fix, math, windows, cfl, need_field,
+                         need_uv)
     gf = gf.to(ctx.dtypes[0]) if need_field else None
     gu = gu.to(ctx.dtypes[1]) if ctx.needs_input_grad[1] else None
     gv = gv.to(ctx.dtypes[2]) if ctx.needs_input_grad[2] else None
@@ -452,38 +570,41 @@ def _sl_advect_jvp(field: Tensor, u: Tensor, v: Tensor, dfield: Optional[Tensor]
                    tables: Tensor, scalars: List[float], dt: float, interp: int, pole_fix: bool, math: int,
                    windows: List[int]) -> Tensor:
     """Tangent-linear model of sl_advect (include/paradis_sl_tl.h): d out along (dfield, du, dv), fp32.  dfield may be
-    None (velocity tangents only).  Full mesh only; every input is read as fp32 (bf16 / fp16 are upcast)."""
+    None (velocity tangents only).  Full mesh only; every input is read as fp32 (bf16 / fp16 are upcast).  If any
+    input is float64, every input is read as double and dout is float64 (include/paradis_sl_f64.h)."""
     B, V, H, W, ownN, arrN = _check_inputs(field, u, v, windows)
     if not _full_mesh(windows):
         raise RuntimeError("paradis::sl_advect_jvp works on the full mesh only")
     for name, t in (("dfield", dfield), ("du", du), ("dv", dv)):
         if t is not None and tuple(t.shape) != tuple(field.shape if name == "dfield" else u.shape):
             raise RuntimeError(f"paradis::sl_advect_jvp: {name} {tuple(t.shape)} does not match its primal")
-    if any(t is not None and t.dtype == torch.float64 for t in (field, u, v, dfield, du, dv)):
-        raise RuntimeError("paradis::sl_advect_jvp computes in fp32; cast float64 inputs explicitly")
     poll_status(field.device)
     if tables.device != field.device:
         raise RuntimeError(f"paradis::sl_advect_jvp: geometry tables live on {tables.device}, the tensors on {field.device}")
-    field, u, v, du, dv = [_inner_contig(t.float()) for t in (field, u, v, du, dv)]
-    dfield = _inner_contig(dfield.float()) if dfield is not None else None
+    f64 = _is_f64(field, u, v, dfield, du, dv)
+    dtype = torch.float64 if f64 else torch.float32
+    field, u, v, du, dv = [_inner_contig(t.to(dtype)) for t in (field, u, v, du, dv)]
+    dfield = _inner_contig(dfield.to(dtype)) if dfield is not None else None
     L = _lib.lib()
-    dout = torch.empty((B, V, ownN, W), dtype=torch.float32, device=field.device)
-    g = _geom_struct(tables, scalars, windows)
-    ws_bytes = L.paradis_sl_advect_jvp_workspace(B, V)
+    dout = torch.empty((B, V, ownN, W), dtype=dtype, device=field.device)
+    g = _geom64_struct(tables, scalars, windows) if f64 else _geom_struct(tables, scalars, windows)
+    name = "paradis_sl_advect_jvp_f64" if f64 else "paradis_sl_advect_jvp"
+    ws_bytes = getattr(L, name + "_workspace")(B, V)
     ws = torch.empty(ws_bytes, dtype=torch.uint8, device=field.device)
     with torch.cuda.device(field.device):
-        rc = L.paradis_sl_advect_jvp(C.byref(g), _ptr(field), _ptr(dfield), _ptr(u), _ptr(v), _ptr(du), _ptr(dv),
-                                     _ptr(dout), B, V, field.stride(0), dfield.stride(0) if dfield is not None else 0,
-                                     u.stride(0), v.stride(0), du.stride(0), dv.stride(0), dt, interp, int(pole_fix),
-                                     math, _ptr(ws), ws_bytes, _ptr(_status_word(field.device)), _stream(field))
-    _lib.check(rc, "paradis_sl_advect_jvp")
+        rc = getattr(L, name)(C.byref(g), _ptr(field), _ptr(dfield), _ptr(u), _ptr(v), _ptr(du), _ptr(dv),
+                              _ptr(dout), B, V, field.stride(0), dfield.stride(0) if dfield is not None else 0,
+                              u.stride(0), v.stride(0), du.stride(0), dv.stride(0), dt, interp, int(pole_fix),
+                              math, _ptr(ws), ws_bytes, _ptr(_status_word(field.device)), _stream(field))
+    _lib.check(rc, name)
     return dout
 
 
 @_sl_advect_jvp.register_fake
 def _(field, u, v, dfield, du, dv, tables, scalars, dt, interp, pole_fix, math, windows):
     B, V = field.shape[:2]
-    return field.new_empty((B, V, windows[3], windows[1]), dtype=torch.float32)
+    dtype = torch.float64 if _is_f64(field, u, v, dfield, du, dv) else torch.float32
+    return field.new_empty((B, V, windows[3], windows[1]), dtype=dtype)
 
 
 class _SLAdvectFn(torch.autograd.Function):
@@ -539,10 +660,21 @@ def sl_advect(field: Tensor, u: Tensor, v: Tensor, geometry: SLGeometry, dt: flo
 
     Forward-mode AD (``torch.func.jvp``, ``torch.autograd.forward_ad``) gives the tangent-linear model on the full
     mesh, in fp32 (``paradis::sl_advect_jvp``).
+
+    float64: if any of field, u, v is float64, the others are upcast and the op computes in double with the reference's
+    op order (``geometry.tables64`` / ``scalars64``); ``out``, the gradients and the tangent are float64.  ``math`` does
+    not change the fp64 result (FAST is an fp32 speed device) and ``cfl_cells`` is not used.  Full mesh only.
     """
     if _ENV_MATH:
         math = _ENV_MATH
-    args = (geometry.tables, geometry.scalars, float(dt), _lib.INTERP[interpolation], bool(pole_fix), _lib.MATH[math],
+    tables, scalars = geometry.tables, geometry.scalars
+    if _is_f64(field, u, v):
+        _f64_full_mesh(geometry.windows, "sl_advect")
+        if geometry.tables64 is None:
+            raise RuntimeError("sl_advect: float64 inputs need a geometry with float64 tables (SLGeometry.from_grids, "
+                               "NeuralSemiLagrangian.geometry())")
+        tables, scalars = geometry.tables64, geometry.scalars64
+    args = (tables, scalars, float(dt), _lib.INTERP[interpolation], bool(pole_fix), _lib.MATH[math],
             geometry.windows, float(cfl_cells))
     if _tangent_path(field, u, v):
         if not _full_mesh(geometry.windows):
@@ -564,10 +696,10 @@ def _geocyclic_pad(x: Tensor, p: int) -> Tensor:
     if not x.is_cuda:
         raise RuntimeError("paradis::geocyclic_pad is a CUDA-only operator (no CPU fallback)")
     B, Cn, H, W = x.shape
-    native = _geo_bf16(x)
+    native = _geo_bf16(x) or _is_f64(x)
     xs = x.contiguous() if native else x.float().contiguous()
     y = torch.empty((B, Cn, H + 2 * p, W + 2 * p), dtype=xs.dtype, device=x.device)
-    name = "paradis_geocyclic_pad_fwd_bf16" if native else "paradis_geocyclic_pad_fwd"
+    name = "paradis_geocyclic_pad_fwd" + _geo_sfx(xs) if native else "paradis_geocyclic_pad_fwd"
     with torch.cuda.device(x.device):
         rc = getattr(_lib.lib(), name)(_ptr(xs), _ptr(y), B * Cn, H, W, p, _stream(x))
     _lib.check(rc, name)
@@ -584,10 +716,10 @@ def _(x, p):
 def _geocyclic_pad_backward(gy: Tensor, p: int) -> Tensor:
     B, Cn, Hp, Wp = gy.shape
     H, W = Hp - 2 * p, Wp - 2 * p
-    native = _geo_bf16(gy)
+    native = _geo_bf16(gy) or _is_f64(gy)
     gs = gy.contiguous() if native else gy.float().contiguous()
     gx = torch.empty((B, Cn, H, W), dtype=gs.dtype, device=gy.device)
-    name = "paradis_geocyclic_pad_bwd_bf16" if native else "paradis_geocyclic_pad_bwd"
+    name = "paradis_geocyclic_pad_bwd" + _geo_sfx(gs) if native else "paradis_geocyclic_pad_bwd"
     with torch.cuda.device(gy.device):
         rc = getattr(_lib.lib(), name)(_ptr(gs), _ptr(gx), B * Cn, H, W, p, _stream(gy))
     _lib.check(rc, name)
@@ -648,6 +780,15 @@ def _geocyclic_dwconv(x: Tensor, weight: Tensor, bias: Optional[Tensor]) -> Tens
     k = weight.shape[-1]
     if tuple(weight.shape) != (Cn, 1, k, k):
         raise RuntimeError("paradis::geocyclic_dwconv expects a depthwise weight [C, 1, k, k]")
+    if _is_f64(x):          # double x: double weight, bias and sums
+        xs, wf = x.contiguous(), weight.double().contiguous()
+        bf = bias.double().contiguous() if bias is not None else None
+        y = torch.empty_like(xs)
+        with torch.cuda.device(x.device):
+            rc = _lib.lib().paradis_geocyclic_dwconv_fwd_f64(_ptr(xs), _ptr(wf), _ptr(bf), _ptr(y), B, Cn, H, W, k,
+                                                             _stream(x))
+        _lib.check(rc, "paradis_geocyclic_dwconv_fwd_f64")
+        return y
     native = _geo_bf16(x)
     xs = x.contiguous() if native else x.float().contiguous()
     wf = weight.float().contiguous()
@@ -666,17 +807,18 @@ def _(x, weight, bias):
 
 
 def _dw_backward_impl(gy: Tensor, x: Tensor, weight: Tensor, need_input: bool, need_weight: bool, need_bias: bool,
-                      native: bool):
-    """Both backward ops.  native: bf16 gy / x read in place and a bf16 grad input; otherwise fp32 copies and an fp32
-    grad input.  grad weight / grad bias are fp32 either way.  Only the requested gradients are computed (a constant
-    filter skips the weight-gradient pass and its workspace)."""
+                      native: bool, f64: bool = False):
+    """All three backward ops.  native: bf16 gy / x read in place and a bf16 grad input; otherwise fp32 copies and an
+    fp32 grad input.  grad weight / grad bias are fp32 either way.  f64: every tensor in double, every gradient double.
+    Only the requested gradients are computed (a constant filter skips the weight-gradient pass and its workspace)."""
     B, Cn, H, W = x.shape
     k = weight.shape[-1]
     L = _lib.lib()
-    gs = gy.contiguous() if native else gy.float().contiguous()
-    wf = weight.float().contiguous()
-    sfx = "_bf16" if native else ""
-    empty = lambda: torch.empty(0, dtype=torch.float32, device=x.device)
+    wdt = torch.float64 if f64 else torch.float32
+    gs = gy.contiguous() if native else gy.to(wdt).contiguous()
+    wf = weight.to(wdt).contiguous()
+    sfx = "_f64" if f64 else "_bf16" if native else ""
+    empty = lambda: torch.empty(0, dtype=wdt, device=x.device)
     gx, gw, gb = empty(), empty(), empty()
     with torch.cuda.device(x.device):
         if need_input:
@@ -685,10 +827,11 @@ def _dw_backward_impl(gy: Tensor, x: Tensor, weight: Tensor, need_input: bool, n
             rc = getattr(L, name)(_ptr(gs), _ptr(wf), _ptr(gx), B, Cn, H, W, k, _stream(x))
             _lib.check(rc, name)
         if need_weight or need_bias:
-            xs = x.contiguous() if native else x.float().contiguous()
+            xs = x.contiguous() if native else x.to(wdt).contiguous()
             gw = torch.empty_like(wf)
-            gb = torch.empty(Cn if need_bias else 0, dtype=torch.float32, device=x.device)
-            ws_bytes = L.paradis_geocyclic_dwconv_wgrad_workspace(B, Cn, H, W, k)
+            gb = torch.empty(Cn if need_bias else 0, dtype=wdt, device=x.device)
+            ws_bytes = getattr(L, "paradis_geocyclic_dwconv_wgrad_f64_workspace" if f64
+                               else "paradis_geocyclic_dwconv_wgrad_workspace")(B, Cn, H, W, k)
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
             name = "paradis_geocyclic_dwconv_bwd_weight" + sfx
             rc = getattr(L, name)(_ptr(xs), _ptr(gs), _ptr(gw), _ptr(gb) if need_bias else _ptr(None),
@@ -731,6 +874,21 @@ def _(gy, x, weight, need_input, need_weight, need_bias):
             x.new_empty((x.shape[1],), dtype=torch.float32) if need_bias else none(torch.float32))
 
 
+@torch.library.custom_op("paradis::geocyclic_dwconv_backward_f64", mutates_args=(), device_types="cuda")
+def _geocyclic_dwconv_backward_f64(gy: Tensor, x: Tensor, weight: Tensor, need_input: bool, need_weight: bool,
+                                   need_bias: bool) -> Tuple[Tensor, Tensor, Tensor]:
+    """Backward for a float64 x: float64 grad input, grad weight and grad bias (include/paradis_sl_f64.h)."""
+    return _dw_backward_impl(gy, x, weight, need_input, need_weight, need_bias, False, f64=True)
+
+
+@_geocyclic_dwconv_backward_f64.register_fake
+def _(gy, x, weight, need_input, need_weight, need_bias):
+    none = lambda: x.new_empty((0,), dtype=torch.float64)
+    return (torch.empty_like(x, dtype=torch.float64) if need_input else none(),
+            torch.empty_like(weight, dtype=torch.float64) if (need_weight or need_bias) else none(),
+            x.new_empty((x.shape[1],), dtype=torch.float64) if need_bias else none())
+
+
 def _dw_setup(ctx, inputs, output):
     x, weight, bias = inputs
     ctx.save_for_backward(x, weight)
@@ -745,9 +903,13 @@ def _dw_backward(ctx, gy):
     need_b = ctx.has_bias and ctx.needs_input_grad[2]
     if not (need_x or need_w or need_b):
         return None, None, None
-    # bf16 x and grad_y: bf16 grad input straight from the kernels (no fp32 copies, no casts)
-    bwd = (torch.ops.paradis.geocyclic_dwconv_backward_bf16 if _geo_bf16(gy) and ctx.dtypes[0] == torch.bfloat16
-           else torch.ops.paradis.geocyclic_dwconv_backward)
+    # bf16 x and grad_y: bf16 grad input straight from the kernels (no fp32 copies, no casts); float64 x: float64
+    if ctx.dtypes[0] == torch.float64:
+        bwd = torch.ops.paradis.geocyclic_dwconv_backward_f64
+    elif _geo_bf16(gy) and ctx.dtypes[0] == torch.bfloat16:
+        bwd = torch.ops.paradis.geocyclic_dwconv_backward_bf16
+    else:
+        bwd = torch.ops.paradis.geocyclic_dwconv_backward
     gx, gw, gb = bwd(gy, x, weight, need_x, need_w, need_b)
     return (gx.to(ctx.dtypes[0]) if need_x else None, gw.to(ctx.dtypes[1]) if need_w else None,
             gb.to(ctx.dtypes[2]) if need_b else None)
@@ -758,7 +920,8 @@ _geocyclic_dwconv.register_autograd(_dw_backward, setup_context=_dw_setup)
 
 class _DwConvFn(torch.autograd.Function):
     """paradis::geocyclic_dwconv with a jvp rule.  The op is bilinear in (x, weight) and affine in bias:
-    d y = dwconv(dx, w) + dwconv(x, dw) + db, each term summed in fp32 and rounded once to y's dtype."""
+    d y = dwconv(dx, w) + dwconv(x, dw) + db, each term summed in fp32 (in float64 for a float64 x) and rounded once
+    to y's dtype."""
 
     @staticmethod
     def forward(x, weight, bias):
@@ -776,13 +939,14 @@ class _DwConvFn(torch.autograd.Function):
     @staticmethod
     def jvp(ctx, dx, dw, db):
         x, weight = ctx.saved_tensors
+        ct = torch.float64 if x.dtype == torch.float64 else torch.float32
         terms = []
         if dx is not None:
-            terms.append(torch.ops.paradis.geocyclic_dwconv(dx, weight, None).float())
+            terms.append(torch.ops.paradis.geocyclic_dwconv(dx.to(x.dtype), weight, None).to(ct))
         if dw is not None:
-            terms.append(torch.ops.paradis.geocyclic_dwconv(x, dw, None).float())
+            terms.append(torch.ops.paradis.geocyclic_dwconv(x, dw, None).to(ct))
         if db is not None and ctx.has_bias:
-            terms.append(db.float().view(1, -1, 1, 1).expand(x.shape))
+            terms.append(db.to(ct).view(1, -1, 1, 1).expand(x.shape))
         dy = terms[0]
         for t in terms[1:]:
             dy = dy + t
@@ -795,10 +959,10 @@ class _DwConvFn(torch.autograd.Function):
 @torch.library.custom_op("paradis::geocyclic_avgpool5", mutates_args=(), device_types="cuda")
 def _geocyclic_avgpool5(x: Tensor, stride: int) -> Tensor:
     B, Cn, H, W = x.shape
-    native = _geo_bf16(x)
+    native = _geo_bf16(x) or _is_f64(x)
     xs = x.contiguous() if native else x.float().contiguous()
     y = torch.empty((B, Cn, (H - 1) // stride + 1, (W - 1) // stride + 1), dtype=xs.dtype, device=x.device)
-    name = "paradis_geocyclic_avgpool5_fwd_bf16" if native else "paradis_geocyclic_avgpool5_fwd"
+    name = "paradis_geocyclic_avgpool5_fwd" + _geo_sfx(xs) if native else "paradis_geocyclic_avgpool5_fwd"
     with torch.cuda.device(x.device):
         rc = getattr(_lib.lib(), name)(_ptr(xs), _ptr(y), B, Cn, H, W, stride, _stream(x))
     _lib.check(rc, name)
@@ -819,10 +983,10 @@ def _geocyclic_avgpool5_backward(gy: Tensor, H: int, W: int, stride: int) -> Ten
     if (Ho, Wo) != ((H - 1) // stride + 1, (W - 1) // stride + 1):
         raise RuntimeError(f"paradis::geocyclic_avgpool5_backward: grad_y {tuple(gy.shape)} does not match an "
                            f"input of {H} x {W} with stride {stride}")
-    native = _geo_bf16(gy)
+    native = _geo_bf16(gy) or _is_f64(gy)
     gs = gy.contiguous() if native else gy.float().contiguous()
     gx = torch.empty((B, Cn, H, W), dtype=gs.dtype, device=gy.device)
-    name = "paradis_geocyclic_avgpool5_bwd_bf16" if native else "paradis_geocyclic_avgpool5_bwd"
+    name = "paradis_geocyclic_avgpool5_bwd" + _geo_sfx(gs) if native else "paradis_geocyclic_avgpool5_bwd"
     with torch.cuda.device(gy.device):
         rc = getattr(_lib.lib(), name)(_ptr(gs), _ptr(gx), B, Cn, H, W, stride, _stream(gy))
     _lib.check(rc, name)
@@ -982,8 +1146,21 @@ class RawAdvection:
 def departure_coords(u: Tensor, v: Tensor, geometry: SLGeometry, dt: float, interpolation="bilinear",
                      math="fast") -> Tensor:
     """Parity instrument: [B, V, 11, H, W] = (ix, iy, sin lat', cos lat', sin lon', cos lon', sin_lat, num, den, lat, lon),
-    the intermediates of model/advection.py:82-94 and the sampler coordinates ATen floors."""
+    the intermediates of model/advection.py:82-94 and the sampler coordinates ATen floors.  float64 for a float64 u or
+    v (the fp64 chain, full mesh; ``math`` does not change it)."""
     L = _lib.lib()
+    if _is_f64(u, v):
+        _f64_full_mesh(geometry.windows, "departure_coords")
+        u, v = _inner_contig(u.double()), _inner_contig(v.double())
+        B, V, R, W = u.shape
+        out = torch.empty((B, V, 11, R, W), dtype=torch.float64, device=u.device)
+        g = _geom64_struct(geometry.tables64, geometry.scalars64, geometry.windows)
+        with torch.cuda.device(u.device):
+            rc = L.paradis_sl_departure_coords_f64(C.byref(g), _ptr(u), _ptr(v), _ptr(out), B, V, u.stride(0),
+                                                   v.stride(0), dt, _lib.INTERP[interpolation], _lib.MATH[math],
+                                                   _stream(u))
+        _lib.check(rc, "paradis_sl_departure_coords_f64")
+        return out
     u, v = _inner_contig(u.float()), _inner_contig(v.float())
     B, V, R, W = u.shape
     out = torch.empty((B, V, 11, geometry.windows[3], W), dtype=torch.float32, device=u.device)
